@@ -195,6 +195,32 @@ WLSQM_API int wlsqm_solver_prepare_hoods(wlsqm_solver_t* s, const double* x, int
 WLSQM_API int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, double* fi, int64_t fi_s0,
                              double* sens, int64_t sens_s0, int64_t sens_s1, int32_t* iters_out);
 
+/* Export of the prepared operators (extension).  The reference offers the linear map from data to fitted DOFs only
+ * as `sens` (impl.pyx:769-779, d fi / d fk, recomputed by every solve), from which its callers assemble Jacobians.
+ * Here each of nops operators is a row of coeffs (host memory, [nops][max no], finite, 1 <= nops <= WLSQM_MAXNO): a
+ * linear combination of DOF slots.  For case i, with j(s) the reduced index of unknown slot s and t(m) the position of
+ * known slot m among the case's knowns (ascending), prepare() stored Op_i (DESIGN.md section 2) and
+ *   W[op][i][k] = sum over unknown s < no_i with coeffs[op][s] != 0, ascending s, of coeffs[op][s] * Op_i[k][j(s)]
+ *                 (FMA from 0; k < nk_i, 0 beyond),
+ *   K[op][i][m] = the same sum over Op_i[nk_i + t(m)][j(s)], plus coeffs[op][m] added last (known m < no_i, 0 elsewhere),
+ * so that sum_s coeffs[s] fi[i][s] = sum_k W[i][k] fk[i][k] + sum_m K[i][m] fi_known[i][m] for an ALGO_BASIC solve.
+ * The map is the same for ALGO_ITERATIVE solvers (prepare does not depend on the algorithm); the corrections of the
+ * refinement loop are not part of it.  Slots >= no_i are ignored; zero coefficients are skipped, never multiplied.
+ * A guest answers with its host's operators and neighbour lists.  Outputs are host or device pointers.
+ *
+ * wlsqm_solver_stencils: W [nops][ncases][max nk], K [nops][ncases][max no] dense (K may be NULL); after any prepare.
+ * wlsqm_solver_operator_nnz / _csr: the global sparse operator over the points of prepare_hoods, which must have been
+ *   the LAST prepare (WLSQM_E_NOTREADY otherwise).  Row i, column p holds the sum of W[i][k] over k < nk_i with
+ *   hoods[i][k] == p, in ascending k.  center = -1: no folding; else 0 <= center, center + ncases <= npoints, and for
+ *   every case with slot 0 (F) known, K[i][0] is added last to column center + i and reported as 0 in K ("the known F
+ *   of case i is f[center + i]").  Pattern: {(i, hoods[i][k]) : k < nk_i} plus the folded diagonal, columns strictly
+ *   ascending, explicit zeros stored; it depends on hoods, knowns and center only and is shared by the nops operators:
+ *   rowptr [ncases + 1] and col [nnz] as int32 (index_bits = 32, nnz < 2^31) or int64, values [nops][nnz]. */
+WLSQM_API int wlsqm_solver_stencils(wlsqm_solver_t* s, int nops, const double* coeffs, double* W, double* K);
+WLSQM_API int wlsqm_solver_operator_nnz(wlsqm_solver_t* s, int64_t center, int64_t* nnz);
+WLSQM_API int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs, int64_t center, int index_bits,
+                              void* rowptr, void* col, double* values, double* K);
+
 /* ExpertSolver.prep_interpolate on the device: index the solver's model origins with a search grid, then
  * interpolate(mode='nearest') may be called with I == NULL, and mode='continuous' is available:
  * weighted average over every model within r, weights (1 - sqrt(d2/r2))^2 (expert.pyx:898-985). */

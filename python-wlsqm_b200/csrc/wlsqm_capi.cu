@@ -4,6 +4,7 @@
 // point needs a CUDA device and fails with WLSQM_E_CUDA otherwise.
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -225,6 +226,8 @@ struct wlsqm_solver {
     DevBuf st_xk, st_fk, st_fi, st_sens, st_x, st_I, st_out;
     DevBuf hoods_dev, hood_x, hood_f, hood_fk;   // prepare_hoods / solve_hoods: neighbour lists and gathered data
     long long hood_points = 0;
+    bool hoods_current = false;                  // the LAST prepare was prepare_hoods: hoods_dev belongs to the operators
+    DevBuf opx_coef;                             // operator export: device copy of the coefficient rows
     int* hood_err = nullptr;                     // device flag: a used hood index fell outside [0, npoints)
     // fused result gather: global solution arrays of the GPUs of the job (peer memory), see wlsqm_solver_set_gather
     int ngather = 0;
@@ -243,7 +246,8 @@ namespace {
 
 long long staging_bytes(const wlsqm_solver* s) {
     return (long long)(s->xk_keep.cap + s->st_xk.cap + s->st_fk.cap + s->st_fi.cap + s->st_sens.cap + s->st_x.cap +
-                       s->st_I.cap + s->st_out.cap + s->hoods_dev.cap + s->hood_x.cap + s->hood_f.cap + s->hood_fk.cap);
+                       s->st_I.cap + s->st_out.cap + s->hoods_dev.cap + s->hood_x.cap + s->hood_f.cap + s->hood_fk.cap +
+                       s->opx_coef.cap);
 }
 
 int use_device(const wlsqm_solver* s) {
@@ -732,7 +736,7 @@ int wlsqm_solver_destroy(wlsqm_solver_t* s) {
     }
     dev_free(s->fi_case); dev_free(s->iters_dev); s->st_xk.release(); s->st_fk.release(); s->st_fi.release(); s->st_sens.release();
     s->st_x.release(); s->st_I.release(); s->st_out.release();
-    s->hoods_dev.release(); s->hood_x.release(); s->hood_f.release(); s->hood_fk.release();
+    s->hoods_dev.release(); s->hood_x.release(); s->hood_f.release(); s->hood_fk.release(); s->opx_coef.release();
     dev_free(s->hood_err);
     if (s->models_grid) { wlsqm_grid_destroy(s->models_grid); s->models_grid = nullptr; }
     if (s->own_stream && s->stream) cudaStreamDestroy(s->stream);
@@ -906,6 +910,7 @@ int wlsqm_solver_prepare(wlsqm_solver_t* s, const double* xi, int64_t xi_s0, con
     if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
     if (s->lender) return wlsqm_solver_prepare_guest(s);
     s->ready = false;
+    s->hoods_current = false;   // (prepare_hoods sets it again once its own prepare has succeeded)
     if (s->models_grid) { wlsqm_grid_destroy(s->models_grid); s->models_grid = nullptr; }   // the origins may move
     if (s->ncases == 0) { s->ready = true; return WLSQM_OK; }
     if (!xi || !xk) return fail(WLSQM_E_VALUE, "xi and xk must not be NULL");
@@ -1367,7 +1372,14 @@ int wlsqm_gather_hoods(const double* src, int64_t src_s0, int w, int64_t nsrc, c
 int wlsqm_solver_prepare_hoods(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t npoints, const int32_t* hoods,
                                int64_t hoods_s0, const double* xi, int64_t xi_s0) {
     if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
-    if (s->ncases == 0) return wlsqm_solver_prepare(s, x, x_s0, x, 0, 0);
+    s->hoods_current = false;   // until the new neighbour lists and the operators built from them are both in place
+    if (s->ncases == 0) {
+        const int rc0 = wlsqm_solver_prepare(s, x, x_s0, x, 0, 0);
+        if (rc0) return rc0;
+        s->hood_points = npoints;
+        s->hoods_current = true;
+        return WLSQM_OK;
+    }
     if (!x || !hoods) return fail(WLSQM_E_VALUE, "x and hoods must not be NULL");
     if (!xi && npoints < s->ncases) return fail(WLSQM_E_VALUE, "without xi, x must hold one point per case");
     int rc = use_device(s);
@@ -1416,6 +1428,7 @@ int wlsqm_solver_prepare_hoods(wlsqm_solver_t* s, const double* x, int64_t x_s0,
     }
     s->st_xk.release();      // (ALGO_ITERATIVE keeps its own copy of the geometry)
     s->hood_x.release();
+    s->hoods_current = true;
     return WLSQM_OK;
 }
 
@@ -1453,6 +1466,212 @@ int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, d
         s->uni.nk, nullptr);
     CU(cudaGetLastError());
     return wlsqm_solver_solve(s, (const double*)s->hood_fk.p, kp, 1, fi, fi_s0, sens, sens_s0, sens_s1, iters_out);
+}
+
+// ---- export of the prepared operators (wlsqm_operator.cu) -------------------------------------------------------
+// A guest answers with its host's operators and neighbour lists: everything below reads the lender's state.
+static int opx_check(wlsqm_solver_t* s, int nops, const double* coeffs, bool hoods) {
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (!r->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called first");
+    if (hoods && !r->hoods_current)
+        return fail(WLSQM_E_NOTREADY, "the global operator needs the neighbour lists of prepare_hoods() as the last prepare");
+    if (nops < 1 || nops > WLSQM_MAXNO) return fail(WLSQM_E_VALUE, "nops must be 1..%d, got %d", WLSQM_MAXNO, nops);
+    if (!coeffs) return fail(WLSQM_E_VALUE, "coeffs must not be NULL");
+    for (long long t = 0; t < (long long)nops * s->maxno; ++t)
+        if (!std::isfinite(coeffs[t])) return fail(WLSQM_E_VALUE, "coefficients must be finite (entry %lld)", t);
+    return use_device(s);
+}
+
+static int opx_center(const wlsqm_solver* s, int64_t center) {
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (center != -1 && (center < 0 || center + s->ncases > r->hood_points))
+        return fail(WLSQM_E_VALUE, "center must be -1 (no folding) or 0 <= center, center + ncases <= npoints = %lld; got %lld",
+                    (long long)r->hood_points, (long long)center);
+    return WLSQM_OK;
+}
+
+// W [nops][ncases][maxnk], K [nops][ncases][maxno] (or NULL), kf [nops][ncases] (or NULL): device pointers
+static int opx_stencils(wlsqm_solver_t* s, int nops, const double* coeffs, double* W, double* K, double* kf) {
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (s->lender) CU(order_streams(r->stream, s->stream));   // the host's prepare may still be in flight
+    const int maxno = s->maxno;
+    int rc = s->opx_coef.reserve((size_t)nops * maxno * 8);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(s->opx_coef.p, coeffs, (size_t)nops * maxno * 8, cudaMemcpyHostToDevice, s->stream));
+    StencilParams P{};
+    P.meta = r->dmeta; P.uni = r->uni; P.geom_uniform = r->geom_uniform ? 1 : 0; P.op_stride = r->op_stride;
+    P.ncases = s->ncases; P.op = r->op; P.coef = (const double*)s->opx_coef.p;
+    P.nops = nops; P.maxnk = s->maxnk; P.maxno = maxno; P.W = W; P.K = K; P.kf = kf;
+    // the ring of solve_kernel: two stages of the largest block, 16 warps per SM for blocks of 3 KB and more
+    P.stage_doubles = std::max(2, even(s->maxnq * s->maxnr));
+    P.ring_off = (nops * maxno + nops + 15) & ~15;
+    const size_t stage_bytes = (size_t)P.stage_doubles * 8;
+    int S = 2, warps = stage_bytes >= 3072 ? 16 : 32;
+    size_t smem = 0;
+    for (;;) {
+        smem = (size_t)P.ring_off * 8 + (size_t)warps * S * (stage_bytes + 8);
+        if (smem <= SMEM_PER_CTA) break;
+        if (warps > 4) --warps;
+        else if (S > 1) --S;
+        else if (warps > 1) --warps;
+        else return fail(WLSQM_E_VALUE, "operator block too large for shared memory (%zu bytes)", stage_bytes);
+    }
+    P.stages = S;
+    P.bar_off_bytes = P.ring_off * 8 + warps * S * P.stage_doubles * 8;
+    int ctas = (int)(SMEM_PER_SM / (smem + 1024));
+    ctas = std::max(1, std::min(ctas, std::max(1, (stage_bytes >= 3072 ? 16 : 32) / warps)));
+    const long long need = (s->ncases + warps - 1) / warps;
+    const int blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    CU(launch_stencils(P, blocks, warps * 32, smem, s->stream));
+    return WLSQM_OK;
+}
+
+// a device view of an output: the caller's pointer, or a staging buffer copied back by opx_copy_out
+static int opx_out(void* p, size_t bytes, DevBuf& stage, void** dev) {
+    *dev = p;
+    if (!p || is_device_ptr(p)) return WLSQM_OK;
+    int rc = stage.reserve(bytes);
+    if (rc) return rc;
+    *dev = stage.p;
+    return WLSQM_OK;
+}
+static int opx_copy_out(void* p, const void* dev, size_t bytes, cudaStream_t st) {
+    if (p && p != dev && bytes) CU(cudaMemcpyAsync(p, dev, bytes, cudaMemcpyDeviceToHost, st));
+    return WLSQM_OK;
+}
+
+// count pass + scan: rp [ncases + 1] (device), nnz on the host
+static int opx_pattern(wlsqm_solver_t* s, int64_t center, DevBuf& cnt, DevBuf& rp, CsrParams& P, long long* nnz) {
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (s->lender) CU(order_streams(r->stream, s->stream));
+    const long long n = s->ncases;
+    if (n >= (1LL << 31) - 1) return fail(WLSQM_E_VALUE, "the global operator supports up to 2^31 - 2 rows");
+    if ((size_t)CSR_BYTES_PER_NK * r->maxnk > CSR_SMEM_MAX)
+        return fail(WLSQM_E_VALUE, "the global operator supports up to %zu neighbours per case, got %d",
+                    CSR_SMEM_MAX / CSR_BYTES_PER_NK, r->maxnk);
+    int rc = cnt.reserve((size_t)(n + 1) * 8);
+    if (!rc) rc = rp.reserve((size_t)(n + 1) * 8);
+    if (rc) return rc;
+    P.meta = r->dmeta; P.uni = r->uni; P.ncases = n;
+    P.hoods = (const int32_t*)r->hoods_dev.p; P.hoods_s0 = r->maxnk; P.maxnk = r->maxnk;
+    P.center = center;
+    P.cnt = (long long*)cnt.p;
+    CU(cudaMemsetAsync((long long*)cnt.p + n, 0, 8, s->stream));
+    CU(launch_csr_count(P, s->stream));
+    size_t tb = 0;
+    CU(csr_scan((long long*)cnt.p, (long long*)rp.p, n + 1, nullptr, &tb, s->stream));
+    DevBuf tmp;
+    rc = tmp.reserve(tb + 16);
+    if (rc) return rc;
+    tb += 16;
+    long long total = 0;
+    cudaError_t e = csr_scan((long long*)cnt.p, (long long*)rp.p, n + 1, tmp.p, &tb, s->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&total, (long long*)rp.p + n, 8, cudaMemcpyDeviceToHost, s->stream);
+    const cudaError_t e2 = cudaStreamSynchronize(s->stream);
+    tmp.release();
+    if (e == cudaSuccess) e = e2;
+    if (e != cudaSuccess) return fail(WLSQM_E_CUDA, "operator pattern: %s", cudaGetErrorString(e));
+    P.rp = (const long long*)rp.p;
+    P.nnz = total;
+    *nnz = total;
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_stencils(wlsqm_solver_t* s, int nops, const double* coeffs, double* W, double* K) {
+    int rc = opx_check(s, nops, coeffs, false);
+    if (rc) return rc;
+    if (!W) return fail(WLSQM_E_VALUE, "W must not be NULL");
+    if (s->ncases == 0) return WLSQM_OK;
+    const size_t wb = (size_t)nops * s->ncases * s->maxnk * 8, kb = (size_t)nops * s->ncases * s->maxno * 8;
+    DevBuf sw, sk;
+    void *Wd, *Kd;
+    rc = opx_out(W, wb, sw, &Wd);
+    if (!rc) rc = opx_out(K, kb, sk, &Kd);
+    if (!rc) rc = opx_stencils(s, nops, coeffs, (double*)Wd, (double*)Kd, nullptr);
+    if (!rc) rc = opx_copy_out(W, Wd, wb, s->stream);
+    if (!rc && K) rc = opx_copy_out(K, Kd, kb, s->stream);
+    if (sw.p || sk.p) {
+        const cudaError_t e = cudaStreamSynchronize(s->stream);
+        sw.release(); sk.release();
+        if (!rc && e != cudaSuccess) return fail(WLSQM_E_CUDA, "stencils: %s", cudaGetErrorString(e));
+    }
+    return rc;
+}
+
+int wlsqm_solver_operator_nnz(wlsqm_solver_t* s, int64_t center, int64_t* nnz) {
+    if (!nnz) return fail(WLSQM_E_VALUE, "nnz must not be NULL");
+    *nnz = 0;
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (!r->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called first");
+    if (!r->hoods_current)
+        return fail(WLSQM_E_NOTREADY, "the global operator needs the neighbour lists of prepare_hoods() as the last prepare");
+    int rc = opx_center(s, center);
+    if (rc) return rc;
+    if (s->ncases == 0) return WLSQM_OK;
+    rc = use_device(s);
+    if (rc) return rc;
+    DevBuf cnt, rp;
+    CsrParams P{};
+    long long total = 0;
+    rc = opx_pattern(s, center, cnt, rp, P, &total);
+    cudaStreamSynchronize(s->stream);
+    cnt.release(); rp.release();
+    if (rc) return rc;
+    *nnz = total;
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs, int64_t center, int index_bits, void* rowptr,
+                              void* col, double* values, double* K) {
+    int rc = opx_check(s, nops, coeffs, true);
+    if (rc) return rc;
+    rc = opx_center(s, center);
+    if (rc) return rc;
+    if (index_bits != 32 && index_bits != 64) return fail(WLSQM_E_VALUE, "index_bits must be 32 or 64, got %d", index_bits);
+    if (!rowptr) return fail(WLSQM_E_VALUE, "rowptr must not be NULL");
+    const long long n = s->ncases;
+    const size_t ib = index_bits / 8;
+    if (n == 0) {
+        const long long z = 0;
+        if (is_device_ptr(rowptr)) CU(cudaMemcpy(rowptr, &z, ib, cudaMemcpyHostToDevice));
+        else memcpy(rowptr, &z, ib);
+        return WLSQM_OK;
+    }
+    DevBuf cnt, rp, wtmp, kf, s_rp, s_col, s_val, s_k;
+    struct Release {     // every scratch block goes back once the stream is idle
+        wlsqm_solver_t* s; DevBuf* b[8];
+        ~Release() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release{s, {&cnt, &rp, &wtmp, &kf, &s_rp, &s_col, &s_val, &s_k}};
+    CsrParams P{};
+    long long nnz = 0;
+    rc = opx_pattern(s, center, cnt, rp, P, &nnz);
+    if (rc) return rc;
+    if (index_bits == 32 && nnz >= (1LL << 31))
+        return fail(WLSQM_E_VALUE, "nnz = %lld does not fit 32-bit indices; use index_bits = 64", nnz);
+    if (nnz > 0 && (!col || !values)) return fail(WLSQM_E_VALUE, "col and values must not be NULL");
+    rc = wtmp.reserve((size_t)nops * n * std::max(s->maxnk, 1) * 8);
+    if (!rc && center >= 0) rc = kf.reserve((size_t)nops * n * 8);
+    if (rc) return rc;
+    const size_t rb = (size_t)(n + 1) * ib, cb = (size_t)nnz * ib, vb = (size_t)nops * nnz * 8, kb = (size_t)nops * n * s->maxno * 8;
+    void *rpd, *cd, *vd, *kd;
+    rc = opx_out(rowptr, rb, s_rp, &rpd);
+    if (!rc) rc = opx_out(nnz ? col : nullptr, cb, s_col, &cd);
+    if (!rc) rc = opx_out(nnz ? values : nullptr, vb, s_val, &vd);
+    if (!rc) rc = opx_out(K, kb, s_k, &kd);
+    if (!rc) rc = opx_stencils(s, nops, coeffs, (double*)wtmp.p, (double*)kd, center >= 0 ? (double*)kf.p : nullptr);
+    if (rc) return rc;
+    P.W = (const double*)wtmp.p; P.kf = (const double*)kf.p; P.nops = nops;
+    P.rowptr = rpd; P.col = cd; P.values = (double*)vd;
+    CU(launch_csr_fill(P, index_bits, s->stream));
+    rc = opx_copy_out(rowptr, rpd, rb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(col, cd, cb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(values, vd, vb, s->stream);
+    if (!rc && K) rc = opx_copy_out(K, kd, kb, s->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(s->stream));
+    return WLSQM_OK;
 }
 
 int wlsqm_solver_index_models(wlsqm_solver_t* s) {

@@ -82,6 +82,61 @@ struct SolveParams {
     int gather_full;                                 // rows are whole 128 B lines (gather_s0 a multiple of 16, <= 32): the padding is stored too
 };
 
+// operator export (wlsqm_operator.cu): contraction of the operator blocks with coefficient rows, CSR assembly
+struct StencilParams {
+    const CaseMeta* meta;
+    CaseMeta uni;
+    int geom_uniform;                                // every case has the sizes of `uni`; only meta[c].knowns is read
+    long long op_stride;
+    long long ncases;
+    const double* op;
+    const double* coef;                              // [nops][maxno] (device copy of the caller's coefficients)
+    int nops, maxnk, maxno;
+    double* W;                                       // [nops][ncases][maxnk]
+    double* K;                                       // [nops][ncases][maxno] or nullptr
+    double* kf;                                      // centre folding: [nops][ncases] known-F weight (K[.][.][0] := 0), or nullptr
+    int stages, stage_doubles, ring_off, bar_off_bytes;   // per-warp ring of operator blocks (doubles / bytes)
+};
+
+// CSR assembly stages a row's used hood indices (int) and a flag byte per index in shared memory: max nk is bounded by
+// CSR_SMEM_MAX / CSR_BYTES_PER_NK (46 489), above what prepare accepts (both prepare kernels stage >= 8 bytes per neighbour)
+constexpr int CSR_BYTES_PER_NK = 5;
+constexpr size_t CSR_SMEM_MAX = 227 * 1024;
+struct CsrParams {
+    const CaseMeta* meta;
+    CaseMeta uni;
+    long long ncases;
+    const int32_t* hoods; int hoods_s0;              // [ncases][hoods_s0], only the first nk_i of row i are read
+    long long center;                                // column of case 0's own point, or -1 (no folding)
+    int maxnk;
+    long long* cnt;                                  // count pass: distinct columns of row i
+    const long long* rp;                             // fill pass: exclusive scan of cnt, [ncases + 1]
+    const double* W; const double* kf; int nops;     // fill pass: stencil weights, folded known-F weights
+    void* rowptr; void* col; double* values;         // outputs, int32 or int64 indices; values [nops][nnz]
+    long long nnz;
+};
+
+#ifdef __CUDACC__
+// Record of case c.  UNI: every case has the sizes of `uni` (only the knowns pattern may vary per case, read from meta
+// when given) and the blocks are op_stride apart; otherwise the per-case record.
+template <bool UNI>
+__device__ __forceinline__ CaseMeta case_meta(const CaseMeta* meta, const CaseMeta& uni, long long op_stride, long long c) {
+    CaseMeta m;
+    if (UNI) {
+        m = uni;
+        m.op_off = c * op_stride;
+        if (meta) m.knowns = meta[c].knowns;
+    } else {
+        m = meta[c];
+    }
+    return m;
+}
+// bytes of a case's operator block as one bulk copy (a multiple of 16; blocks start 16 B aligned)
+__device__ __forceinline__ uint32_t op_block_bytes(const CaseMeta& m) {
+    return ((uint32_t)((m.nk + m.nkn) * (int)m.nr) * 8u + 15u) & ~15u;
+}
+#endif
+
 struct InterpParams {
     int dim;
     long long nx;
@@ -114,6 +169,10 @@ cudaError_t launch_solve_pack(const SolveParams& P, int blocks, int threads, siz
 cudaError_t launch_scatter_fi(const CaseMeta* meta, const CaseMeta& uni, long long ncases, const double* fi_case,
                               int fi_case_ld, double* fi_out, long long fi_out_s0, cudaStream_t st);
 cudaError_t launch_interpolate(const InterpParams& P, cudaStream_t st);
+cudaError_t launch_stencils(const StencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
+cudaError_t launch_csr_count(const CsrParams& P, cudaStream_t st);
+cudaError_t csr_scan(long long* cnt, long long* rp, long long n1, void* tmp, size_t* tmp_bytes, cudaStream_t st);
+cudaError_t launch_csr_fill(const CsrParams& P, int index_bits, cudaStream_t st);
 struct GridView;
 cudaError_t launch_interpolate_continuous(const InterpParams& P, const GridView& g, double r, cudaStream_t st);
 cudaError_t launch_getrf(int n, long long nlhs, double* A, int* ipiv, cudaStream_t st);

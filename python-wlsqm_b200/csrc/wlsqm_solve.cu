@@ -182,17 +182,7 @@ solve_kernel(SolveParams P) {
     const long long GW = (long long)gridDim.x * nwarps;
     const long long n_my = gw < P.ncases ? (P.ncases - gw + GW - 1) / GW : 0;
 
-    auto get_meta = [&](long long c) {
-        CaseMeta m;
-        if (UNI) {
-            m = P.uni;
-            m.op_off = c * P.op_stride;
-            if (P.meta) m.knowns = P.meta[c].knowns;   // same sizes everywhere, only the knowns pattern varies
-        } else {
-            m = P.meta[c];
-        }
-        return m;
-    };
+    auto get_meta = [&](long long c) { return case_meta<UNI>(P.meta, P.uni, P.op_stride, c); };
     // bulk copies need 16 B alignment and sizes: the host says whether the arrays qualify (f_tma, xk_tma: 16 B aligned
     // base, unit stride, EVEN row pitch); otherwise the lanes gather with plain loads.  A row with an odd element count is
     // copied with one element more -- the pitch is even, so that element exists, and nothing reads it (fext[nk] is either
@@ -203,7 +193,7 @@ solve_kernel(SolveParams P) {
     auto issue = [&](int s, long long c) {   // lane 0 only: arm the stage's barrier and start its copies
         const CaseMeta m = get_meta(c);
         const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
-        const uint32_t b_op = ((uint32_t)((m.nk + m.nkn) * (int)m.nr) * 8u + 15u) & ~15u;
+        const uint32_t b_op = op_block_bytes(m);
         const uint32_t b_f = f_by_tma(m) ? (((uint32_t)m.nk + 1u) & ~1u) * 8u : 0u;
         const uint32_t b_x = xk_by_tma(m) ? (((uint32_t)(m.nk * DIM) + 1u) & ~1u) * 8u : 0u;
         mbar_expect_tx_u32(bar, b_op + b_f + b_x);

@@ -24,6 +24,7 @@ from libc.stdint cimport int32_t, int64_t, uintptr_t
 
 from .fitter import defs
 from . import _lib
+from .fitter import opexport as _opexport
 
 cdef extern from "wlsqm_b200.h" nogil:
     ctypedef struct wlsqm_solver_t:
@@ -58,6 +59,10 @@ cdef extern from "wlsqm_b200.h" nogil:
                                    int64_t hoods_s0, const double* xi, int64_t xi_s0)
     int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, double* fi, int64_t fi_s0, double* sens,
                                  int64_t sens_s0, int64_t sens_s1, int32_t* iters_out)
+    int wlsqm_solver_stencils(wlsqm_solver_t* s, int nops, const double* coeffs, double* W, double* K)
+    int wlsqm_solver_operator_nnz(wlsqm_solver_t* s, int64_t center, int64_t* nnz)
+    int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs, int64_t center, int index_bits,
+                                  void* rowptr, void* col, double* values, double* K)
     int wlsqm_solver_index_models(wlsqm_solver_t* s)
     int wlsqm_solver_nearest_models(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, int64_t* I_out)
     int wlsqm_solver_interpolate_continuous(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r, int diff,
@@ -561,6 +566,7 @@ class ExpertSolver:
         with nogil:
             rc = wlsqm_solver_prepare(h, axi.p, axi.s0, axk.p, axk.s0, axk.s1)
         _check(rc)
+        self._cuda_out = bool(axk.cuda)
         self.ready = True
 
     def conds(self):
@@ -610,7 +616,24 @@ class ExpertSolver:
         self.xi = xi if xi is not None else x[:self.ncases]
         self.xk, self.tree = None, None
         self._hood_points = npts
+        self._cuda_out = bool(ha.is_cuda)
         self.ready = True
+
+    # -- export of the prepared operators (extension; wlsqm_b200/fitter/opexport.py) ------------------------------------
+    def stencils(self, coeffs):
+        """(W, K): the prepared operators contracted with coefficient rows -- W (nops, ncases, max nk) weights on fk,
+        K (nops, ncases, max no) weights on the known values, so that sum_s c[s] fi[i, s] = W[i] . fk[i] + K[i] . fi[i]
+        for an ALGO_BASIC solve.  coeffs: an int slot, a (max no,) row or a (nops, max no) array (the nops axis is dropped
+        for the first two).  The d fi / d fk of the reference's sens (impl.pyx:769-779); an ALGO_ITERATIVE solver exports
+        the same operator (the refinement corrections are not part of it)."""
+        return _opexport.stencils(self, coeffs)
+
+    def operator(self, coeffs, center=None):
+        """(D, K): the global sparse operator (ncases, npoints) over the points of prepare_hoods (torch CSR on the
+        device for CUDA hoods, scipy csr_array otherwise; a list for 2-D coeffs) and the known-value weights.
+        center: index in x of case 0's own point -- the weight on a known F of case i then goes to column center + i.
+        See wlsqm_b200.fitter.opexport.operator."""
+        return _opexport.operator(self, coeffs, center)
 
     def solve_hoods(self, f, fi, sens=None):
         """``solve(f[hoods], fi, sens)`` with the gather done on the device (extension; needs prepare_hoods).

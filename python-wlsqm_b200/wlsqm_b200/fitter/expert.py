@@ -19,7 +19,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import defs
+from . import defs, opexport
 from .. import _lib
 
 __all__ = ["number_of_dofs", "ExpertSolver"]
@@ -219,6 +219,7 @@ class ExpertSolver:
         if self.host is None:
             self.xk, self.xi, self.tree = xk, xi, None
         _lib.check(_lib.lib().wlsqm_solver_prepare(self._handle, xi_a.ptr, xi_s0, xk_a.ptr, xk_s0, xk_s1))
+        self._cuda_out = bool(xk_a.is_cuda)
         self.ready = True
 
     def conds(self):
@@ -259,7 +260,24 @@ class ExpertSolver:
         self.xi = xi if xi is not None else x[:self.ncases]
         self.xk, self.tree = None, None
         self._hood_points = npts
+        self._cuda_out = bool(ha.is_cuda)
         self.ready = True
+
+    # -- export of the prepared operators (extension; opexport.py) --------------------------------------------------------
+    def stencils(self, coeffs):
+        """(W, K): the prepared operators contracted with coefficient rows -- W (nops, ncases, max nk) weights on fk,
+        K (nops, ncases, max no) weights on the known values, so that sum_s c[s] fi[i, s] = W[i] . fk[i] + K[i] . fi[i]
+        for an ALGO_BASIC solve.  coeffs: an int slot, a (max no,) row or a (nops, max no) array (the nops axis is dropped
+        for the first two).  The d fi / d fk of the reference's sens (impl.pyx:769-779); an ALGO_ITERATIVE solver exports
+        the same operator (the refinement corrections are not part of it)."""
+        return opexport.stencils(self, coeffs)
+
+    def operator(self, coeffs, center=None):
+        """(D, K): the global sparse operator (ncases, npoints) over the points of prepare_hoods (torch CSR on the
+        device for CUDA hoods, scipy csr_array otherwise; a list for 2-D coeffs) and the known-value weights.
+        center: index in x of case 0's own point -- the weight on a known F of case i then goes to column center + i.
+        See wlsqm_b200.fitter.opexport.operator."""
+        return opexport.operator(self, coeffs, center)
 
     def solve_hoods(self, f, fi, sens=None):
         """``solve(f[hoods], fi, sens)`` with the gather done on the device (extension; needs prepare_hoods).

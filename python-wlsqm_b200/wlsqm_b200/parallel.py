@@ -21,7 +21,7 @@ import os
 import numpy as np
 
 from .fitter.expert import ExpertSolver
-from .fitter import defs
+from .fitter import defs, opexport
 from . import _lib
 
 __all__ = ["shard_range", "shard_ranges", "balanced_shards", "all_gather_rows", "ShardedExpertSolver"]
@@ -167,6 +167,23 @@ class ShardedExpertSolver:
         if f_is_local:
             f = all_gather_rows(f, self.ranges, group=group)
         return self.solver.solve_hoods(f, self._rows(fi, local), self._rows(sens, local))
+
+    def operator(self, coeffs, fold_center=False):
+        """This rank's row block ``[lo, hi)`` of the global sparse operator (``ExpertSolver.operator``) after
+        ``prepare_hoods``, with global column indices: stacking the blocks of all ranks gives the unsharded matrix.
+        ``coeffs`` are rows over the GLOBAL batch's max no; K comes back with that width.  ``fold_center``: the
+        origins of this rank's cases are ``x[lo:hi]``, so the known-F weight of case lo + i goes to column lo + i."""
+        c, squeeze = opexport.coefficient_rows(coeffs, self.maxno)
+        c = c[:, :self.solver._maxno]       # slots beyond this rank's largest model are ignored by all its cases
+        D, K = self.solver.operator(c[0] if squeeze else c, center=self.lo if fold_center else None)
+        pad = self.maxno - K.shape[-1]
+        if pad:
+            if _lib._is_torch_tensor(K):
+                import torch
+                K = torch.nn.functional.pad(K, (0, pad))
+            else:
+                K = np.pad(K, [(0, 0)] * (K.ndim - 1) + [(0, pad)])
+        return D, K
 
     def gather(self, local_rows, out=None, group=None):
         """collective all-gather of a per-rank result (e.g. the local fi tensor) into the global array"""

@@ -221,6 +221,37 @@ WLSQM_API int wlsqm_solver_operator_nnz(wlsqm_solver_t* s, int64_t center, int64
 WLSQM_API int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs, int64_t center, int index_bits,
                               void* rowptr, void* col, double* values, double* K);
 
+/* Interpolation operators (extension): the linear map from the data to interpolate(x, mode='nearest', diff) at
+ * arbitrary query points, d^D f(xq) = sum_s T_D(s, xq - xi[m]) fi[m][s] with m = I[q] (expert.pyx:687-781).
+ * For query q with model m = I[q] and offset h = xq - xi[m], taken per axis:
+ *   - per-axis steps are those of steps_of in wlsqm_common.cuh: st = (h, 0.5*h, (1.0/3.0)*h, 0.25*h), each rounded once;
+ *   - per-axis Taylor terms: t[0] = 1, t[n] = t[n-1] * st[n-1], with separately rounded multiplies;
+ *   - for a slot s with exponents (a, b, c) and a derivative slot D = (p, r, u):
+ *       T_D(s) = (tx[a-p] * ty[b-r]) * tz[c-u] if a >= p, b >= r and c >= u;  T_D(s) = 0 otherwise.
+ * Coefficient rows keep the convention above ([nops][max no]).  Operator o at query q has the coefficient row
+ *   c_q[o][s] = sum over D ascending with coeffs[o][D] != 0 of coeffs[o][D] * T_D(s),
+ * each product and each sum rounded separately, with no FMA (__dmul_rn / __dadd_rn: nvcc cannot contract them).
+ * Then W, K and the CSR row of query q are EXACTLY the definitions of wlsqm_solver_stencils / _operator_csr for case m
+ * with c_q in place of coeffs: the same ascending-slot FMA chain from 0, zero coefficients skipped, c_q[m] added last for
+ * known slots, duplicate neighbours merged in ascending k, and with center the known-F weight added last to column
+ * center + I[q].  At h = 0, c_q = coeffs: a query at a model origin reproduces that model's stencils / operator row.
+ * I[q] outside [0, ncases) (ncases is the search's "none found" for a NaN query): W row 0, K row NaN, empty CSR row,
+ * so that W . fk + K . fi is NaN, as interpolate returns NaN for such a query.
+ * The operator is the ALGO_BASIC one for every solver (the refinement corrections of ALGO_ITERATIVE are not part of it);
+ * it does not read the solver's solution copy (valid after keep_solution(0)).  A guest answers with its host's operators
+ * and neighbour lists.  x [nx][dim] (row pitch x_s0) and I (int64 [nx]) may be host or device memory; outputs too.
+ *
+ * wlsqm_solver_interp_stencils: W [nops][nx][max nk], K [nops][nx][max no] (K may be NULL); valid after ANY prepare.
+ * wlsqm_solver_interp_operator_nnz / _csr: rows = queries in caller order, columns = points of prepare_hoods, which
+ *   must have been the LAST prepare (WLSQM_E_NOTREADY otherwise); center as for wlsqm_solver_operator_csr; nx = 0 gives
+ *   rowptr = [0]. */
+WLSQM_API int wlsqm_solver_interp_stencils(wlsqm_solver_t* s, const double* x, int64_t x_s0, const int64_t* I, int64_t nx,
+                                           int nops, const double* coeffs, double* W, double* K);
+WLSQM_API int wlsqm_solver_interp_operator_nnz(wlsqm_solver_t* s, const int64_t* I, int64_t nx, int64_t center, int64_t* nnz);
+WLSQM_API int wlsqm_solver_interp_operator_csr(wlsqm_solver_t* s, const double* x, int64_t x_s0, const int64_t* I, int64_t nx,
+                                               int nops, const double* coeffs, int64_t center, int index_bits, void* rowptr,
+                                               void* col, double* values, double* K);
+
 /* ExpertSolver.prep_interpolate on the device: index the solver's model origins with a search grid, then
  * interpolate(mode='nearest') may be called with I == NULL, and mode='continuous' is available:
  * weighted average over every model within r, weights (1 - sqrt(d2/r2))^2 (expert.pyx:898-985). */

@@ -228,6 +228,7 @@ struct wlsqm_solver {
     long long hood_points = 0;
     bool hoods_current = false;                  // the LAST prepare was prepare_hoods: hoods_dev belongs to the operators
     DevBuf opx_coef;                             // operator export: device copy of the coefficient rows
+    DevBuf opx_runs, opx_tmp;                    // interpolation operators: runs of the sorted queries, cub scratch
     int* hood_err = nullptr;                     // device flag: a used hood index fell outside [0, npoints)
     // fused result gather: global solution arrays of the GPUs of the job (peer memory), see wlsqm_solver_set_gather
     int ngather = 0;
@@ -247,7 +248,7 @@ namespace {
 long long staging_bytes(const wlsqm_solver* s) {
     return (long long)(s->xk_keep.cap + s->st_xk.cap + s->st_fk.cap + s->st_fi.cap + s->st_sens.cap + s->st_x.cap +
                        s->st_I.cap + s->st_out.cap + s->hoods_dev.cap + s->hood_x.cap + s->hood_f.cap + s->hood_fk.cap +
-                       s->opx_coef.cap);
+                       s->opx_coef.cap + s->opx_runs.cap + s->opx_tmp.cap);
 }
 
 int use_device(const wlsqm_solver* s) {
@@ -737,6 +738,7 @@ int wlsqm_solver_destroy(wlsqm_solver_t* s) {
     dev_free(s->fi_case); dev_free(s->iters_dev); s->st_xk.release(); s->st_fk.release(); s->st_fi.release(); s->st_sens.release();
     s->st_x.release(); s->st_I.release(); s->st_out.release();
     s->hoods_dev.release(); s->hood_x.release(); s->hood_f.release(); s->hood_fk.release(); s->opx_coef.release();
+    s->opx_runs.release(); s->opx_tmp.release();
     dev_free(s->hood_err);
     if (s->models_grid) { wlsqm_grid_destroy(s->models_grid); s->models_grid = nullptr; }
     if (s->own_stream && s->stream) cudaStreamDestroy(s->stream);
@@ -1541,11 +1543,12 @@ static int opx_copy_out(void* p, const void* dev, size_t bytes, cudaStream_t st)
     return WLSQM_OK;
 }
 
-// count pass + scan: rp [ncases + 1] (device), nnz on the host
-static int opx_pattern(wlsqm_solver_t* s, int64_t center, DevBuf& cnt, DevBuf& rp, CsrParams& P, long long* nnz) {
+// count pass + scan: rp [n + 1] (device), nnz on the host.  Rows are the cases (row_case == nullptr, n == ncases) or
+// queries with their case index (device int64 [n], the interpolation operators)
+static int opx_pattern(wlsqm_solver_t* s, int64_t center, long long n, const long long* row_case, DevBuf& cnt, DevBuf& rp,
+                       CsrParams& P, long long* nnz) {
     const wlsqm_solver* r = s->lender ? s->lender : s;
     if (s->lender) CU(order_streams(r->stream, s->stream));
-    const long long n = s->ncases;
     if (n >= (1LL << 31) - 1) return fail(WLSQM_E_VALUE, "the global operator supports up to 2^31 - 2 rows");
     if ((size_t)CSR_BYTES_PER_NK * r->maxnk > CSR_SMEM_MAX)
         return fail(WLSQM_E_VALUE, "the global operator supports up to %zu neighbours per case, got %d",
@@ -1553,7 +1556,7 @@ static int opx_pattern(wlsqm_solver_t* s, int64_t center, DevBuf& cnt, DevBuf& r
     int rc = cnt.reserve((size_t)(n + 1) * 8);
     if (!rc) rc = rp.reserve((size_t)(n + 1) * 8);
     if (rc) return rc;
-    P.meta = r->dmeta; P.uni = r->uni; P.ncases = n;
+    P.meta = r->dmeta; P.uni = r->uni; P.ncases = n; P.row_case = row_case; P.nmodels = s->ncases;
     P.hoods = (const int32_t*)r->hoods_dev.p; P.hoods_s0 = r->maxnk; P.maxnk = r->maxnk;
     P.center = center;
     P.cnt = (long long*)cnt.p;
@@ -1615,7 +1618,7 @@ int wlsqm_solver_operator_nnz(wlsqm_solver_t* s, int64_t center, int64_t* nnz) {
     DevBuf cnt, rp;
     CsrParams P{};
     long long total = 0;
-    rc = opx_pattern(s, center, cnt, rp, P, &total);
+    rc = opx_pattern(s, center, s->ncases, nullptr, cnt, rp, P, &total);
     cudaStreamSynchronize(s->stream);
     cnt.release(); rp.release();
     if (rc) return rc;
@@ -1646,7 +1649,7 @@ int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs,
     } release{s, {&cnt, &rp, &wtmp, &kf, &s_rp, &s_col, &s_val, &s_k}};
     CsrParams P{};
     long long nnz = 0;
-    rc = opx_pattern(s, center, cnt, rp, P, &nnz);
+    rc = opx_pattern(s, center, n, nullptr, cnt, rp, P, &nnz);
     if (rc) return rc;
     if (index_bits == 32 && nnz >= (1LL << 31))
         return fail(WLSQM_E_VALUE, "nnz = %lld does not fit 32-bit indices; use index_bits = 64", nnz);
@@ -1661,6 +1664,199 @@ int wlsqm_solver_operator_csr(wlsqm_solver_t* s, int nops, const double* coeffs,
     if (!rc) rc = opx_out(nnz ? values : nullptr, vb, s_val, &vd);
     if (!rc) rc = opx_out(K, kb, s_k, &kd);
     if (!rc) rc = opx_stencils(s, nops, coeffs, (double*)wtmp.p, (double*)kd, center >= 0 ? (double*)kf.p : nullptr);
+    if (rc) return rc;
+    P.W = (const double*)wtmp.p; P.kf = (const double*)kf.p; P.nops = nops;
+    P.rowptr = rpd; P.col = cd; P.values = (double*)vd;
+    CU(launch_csr_fill(P, index_bits, s->stream));
+    rc = opx_copy_out(rowptr, rpd, rb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(col, cd, cb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(values, vd, vb, s->stream);
+    if (!rc && K) rc = opx_copy_out(K, kd, kb, s->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(s->stream));
+    return WLSQM_OK;
+}
+
+// ---- interpolation operators: rows at query points (wlsqm_operator.cu) ----------------------------------------
+// a device view of the case indices I [nx] (int64): the caller's array, or the solver's staging copy
+static int opx_index(wlsqm_solver_t* s, const int64_t* I, long long nx, const long long** Id) {
+    if (!I) return fail(WLSQM_E_VALUE, "I must not be NULL");
+    if (nx >= (1LL << 31) - 1) return fail(WLSQM_E_VALUE, "the interpolation operators support up to 2^31 - 2 queries");
+    if (is_device_ptr(I)) { *Id = (const long long*)I; return WLSQM_OK; }
+    int rc = s->st_I.reserve((size_t)nx * 8);
+    if (!rc) rc = stage_in(s->device, (double*)s->st_I.p, reinterpret_cast<const double*>(I), nx, 1, 1, s->stream);   // (8-byte items)
+    if (rc) return rc;
+    *Id = (const long long*)s->st_I.p;
+    return WLSQM_OK;
+}
+// ... and of the query points x [nx][dim] (row pitch x_s0)
+static int opx_points(wlsqm_solver_t* s, const double* x, int64_t x_s0, long long nx, const double** xd, long long* xs) {
+    if (!x) return fail(WLSQM_E_VALUE, "x must not be NULL");
+    if (is_device_ptr(x)) { *xd = x; *xs = x_s0; return WLSQM_OK; }
+    int rc = s->st_x.reserve((size_t)nx * s->dim * 8);
+    if (!rc) rc = stage_in(s->device, (double*)s->st_x.p, x, nx, s->dim, x_s0, s->stream);
+    if (rc) return rc;
+    *xd = (const double*)s->st_x.p; *xs = s->dim;
+    return WLSQM_OK;
+}
+
+// W [nops][nx][maxnk], K [nops][nx][maxno] (or NULL), kf [nops][nx] (or NULL) of the queries: device pointers
+static int opx_interp(wlsqm_solver_t* s, const double* xd, long long xs, const long long* Id, long long nx, int nops,
+                      const double* coeffs, double* W, double* K, double* kf) {
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (s->lender) CU(order_streams(r->stream, s->stream));   // the host's prepare may still be in flight
+    const int maxno = s->maxno;
+    // runs of equal I among the queries
+    int rc = s->opx_runs.reserve(((size_t)7 * nx + 1) * sizeof(int));
+    if (rc) return rc;
+    int* rb = (int*)s->opx_runs.p;
+    InterpRuns R{rb, rb + nx, rb + 2 * nx, rb + 3 * nx, rb + 4 * nx, rb + 5 * nx, rb + 6 * nx, rb + 7 * nx};
+    size_t tb = 0;
+    CU(interp_runs(Id, nx, s->ncases, R, nullptr, &tb, s->stream));
+    rc = s->opx_tmp.reserve(tb + 16);
+    if (rc) return rc;
+    tb = s->opx_tmp.cap;
+    CU(interp_runs(Id, nx, s->ncases, R, s->opx_tmp.p, &tb, s->stream));
+    rc = s->opx_coef.reserve((size_t)nops * maxno * 8);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(s->opx_coef.p, coeffs, (size_t)nops * maxno * 8, cudaMemcpyHostToDevice, s->stream));
+    InterpStencilParams P{};
+    P.meta = r->dmeta; P.uni = r->uni; P.geom_uniform = r->geom_uniform ? 1 : 0; P.op_stride = r->op_stride;
+    P.nmodels = s->ncases; P.op = r->op; P.xi = r->xi_dev; P.x = xd; P.x_s0 = xs; P.dim = s->dim; P.nx = nx;
+    P.run_case = R.run_case; P.run_len = R.run_len; P.run_off = R.run_off; P.nruns = R.nruns; P.perm = R.perm;
+    P.coef = (const double*)s->opx_coef.p; P.nops = nops; P.maxnk = s->maxnk; P.maxno = maxno;
+    P.W = W; P.K = K; P.kf = kf;
+    // the ring of stencil_kernel, plus per warp the coefficient rows of one query (all nops operators, or fewer per pass
+    // when shared memory is short) and its Taylor terms
+    P.stage_doubles = std::max(2, even(s->maxnq * s->maxnr));
+    P.ring_off = (nops * maxno + nops + (maxno + 3) / 4 + 15) & ~15;
+    const size_t stage_bytes = (size_t)P.stage_doubles * 8;
+    int S = 2, warps = stage_bytes >= 3072 ? 16 : 32, opc = nops, cqd = 0;
+    size_t smem = 0;
+    for (;;) {
+        cqd = even(opc * maxno + opc + 15);
+        smem = (size_t)P.ring_off * 8 + (size_t)warps * S * (stage_bytes + 8) + (size_t)warps * cqd * 8;
+        if (smem <= SMEM_PER_CTA) break;
+        if (warps > 8) --warps;
+        else if (opc > 1) opc = (opc + 1) / 2;
+        else if (warps > 4) --warps;
+        else if (S > 1) --S;
+        else if (warps > 1) --warps;
+        else return fail(WLSQM_E_VALUE, "operator block too large for shared memory (%zu bytes)", stage_bytes);
+    }
+    P.stages = S; P.opc = opc; P.cq_doubles = cqd;
+    P.cq_off = P.ring_off + warps * S * P.stage_doubles;
+    P.bar_off_bytes = (P.cq_off + warps * cqd) * 8;
+    int ctas = (int)(SMEM_PER_SM / (smem + 1024));
+    ctas = std::max(1, std::min(ctas, std::max(1, (stage_bytes >= 3072 ? 16 : 32) / warps)));
+    const long long need = (nx + warps - 1) / warps;      // (there are at most nx runs)
+    const int blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    CU(launch_interp_stencils(P, blocks, warps * 32, smem, s->stream));
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_interp_stencils(wlsqm_solver_t* s, const double* x, int64_t x_s0, const int64_t* I, int64_t nx, int nops,
+                                 const double* coeffs, double* W, double* K) {
+    int rc = opx_check(s, nops, coeffs, false);
+    if (rc) return rc;
+    if (nx < 0) return fail(WLSQM_E_VALUE, "nx must be >= 0, got %lld", (long long)nx);
+    if (nx == 0) return WLSQM_OK;
+    if (!W) return fail(WLSQM_E_VALUE, "W must not be NULL");
+    const double* xd;
+    long long xs;
+    const long long* Id;
+    rc = opx_index(s, I, nx, &Id);
+    if (!rc) rc = opx_points(s, x, x_s0, nx, &xd, &xs);
+    if (rc) return rc;
+    const size_t wb = (size_t)nops * nx * s->maxnk * 8, kb = (size_t)nops * nx * s->maxno * 8;
+    DevBuf sw, sk;
+    void *Wd, *Kd;
+    rc = opx_out(W, wb, sw, &Wd);
+    if (!rc) rc = opx_out(K, kb, sk, &Kd);
+    if (!rc) rc = opx_interp(s, xd, xs, Id, nx, nops, coeffs, (double*)Wd, (double*)Kd, nullptr);
+    if (!rc) rc = opx_copy_out(W, Wd, wb, s->stream);
+    if (!rc && K) rc = opx_copy_out(K, Kd, kb, s->stream);
+    if (sw.p || sk.p || xd != x || (const void*)Id != (const void*)I) {
+        const cudaError_t e = cudaStreamSynchronize(s->stream);
+        sw.release(); sk.release();
+        if (!rc && e != cudaSuccess) return fail(WLSQM_E_CUDA, "interp_stencils: %s", cudaGetErrorString(e));
+    }
+    return rc;
+}
+
+int wlsqm_solver_interp_operator_nnz(wlsqm_solver_t* s, const int64_t* I, int64_t nx, int64_t center, int64_t* nnz) {
+    if (!nnz) return fail(WLSQM_E_VALUE, "nnz must not be NULL");
+    *nnz = 0;
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (!r->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called first");
+    if (!r->hoods_current)
+        return fail(WLSQM_E_NOTREADY, "the global operator needs the neighbour lists of prepare_hoods() as the last prepare");
+    int rc = opx_center(s, center);
+    if (rc) return rc;
+    if (nx < 0) return fail(WLSQM_E_VALUE, "nx must be >= 0, got %lld", (long long)nx);
+    if (nx == 0) return WLSQM_OK;
+    rc = use_device(s);
+    if (rc) return rc;
+    const long long* Id;
+    rc = opx_index(s, I, nx, &Id);
+    if (rc) return rc;
+    DevBuf cnt, rp;
+    CsrParams P{};
+    long long total = 0;
+    rc = opx_pattern(s, center, nx, Id, cnt, rp, P, &total);
+    cudaStreamSynchronize(s->stream);
+    cnt.release(); rp.release();
+    if (rc) return rc;
+    *nnz = total;
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_interp_operator_csr(wlsqm_solver_t* s, const double* x, int64_t x_s0, const int64_t* I, int64_t nx, int nops,
+                                     const double* coeffs, int64_t center, int index_bits, void* rowptr, void* col,
+                                     double* values, double* K) {
+    int rc = opx_check(s, nops, coeffs, true);
+    if (rc) return rc;
+    rc = opx_center(s, center);
+    if (rc) return rc;
+    if (index_bits != 32 && index_bits != 64) return fail(WLSQM_E_VALUE, "index_bits must be 32 or 64, got %d", index_bits);
+    if (!rowptr) return fail(WLSQM_E_VALUE, "rowptr must not be NULL");
+    if (nx < 0) return fail(WLSQM_E_VALUE, "nx must be >= 0, got %lld", (long long)nx);
+    const size_t ib = index_bits / 8;
+    if (nx == 0) {
+        const long long z = 0;
+        if (is_device_ptr(rowptr)) CU(cudaMemcpy(rowptr, &z, ib, cudaMemcpyHostToDevice));
+        else memcpy(rowptr, &z, ib);
+        return WLSQM_OK;
+    }
+    const double* xd;
+    long long xs;
+    const long long* Id;
+    rc = opx_index(s, I, nx, &Id);
+    if (!rc) rc = opx_points(s, x, x_s0, nx, &xd, &xs);
+    if (rc) return rc;
+    DevBuf cnt, rp, wtmp, kf, s_rp, s_col, s_val, s_k;
+    struct Release {     // every scratch block goes back once the stream is idle
+        wlsqm_solver_t* s; DevBuf* b[8];
+        ~Release() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release{s, {&cnt, &rp, &wtmp, &kf, &s_rp, &s_col, &s_val, &s_k}};
+    CsrParams P{};
+    long long nnz = 0;
+    rc = opx_pattern(s, center, nx, Id, cnt, rp, P, &nnz);
+    if (rc) return rc;
+    if (index_bits == 32 && nnz >= (1LL << 31))
+        return fail(WLSQM_E_VALUE, "nnz = %lld does not fit 32-bit indices; use index_bits = 64", nnz);
+    if (nnz > 0 && (!col || !values)) return fail(WLSQM_E_VALUE, "col and values must not be NULL");
+    rc = wtmp.reserve((size_t)nops * nx * std::max(s->maxnk, 1) * 8);
+    if (!rc && center >= 0) rc = kf.reserve((size_t)nops * nx * 8);
+    if (rc) return rc;
+    const size_t rb = (size_t)(nx + 1) * ib, cb = (size_t)nnz * ib, vb = (size_t)nops * nnz * 8, kb = (size_t)nops * nx * s->maxno * 8;
+    void *rpd, *cd, *vd, *kd;
+    rc = opx_out(rowptr, rb, s_rp, &rpd);
+    if (!rc) rc = opx_out(nnz ? col : nullptr, cb, s_col, &cd);
+    if (!rc) rc = opx_out(nnz ? values : nullptr, vb, s_val, &vd);
+    if (!rc) rc = opx_out(K, kb, s_k, &kd);
+    if (!rc) rc = opx_interp(s, xd, xs, Id, nx, nops, coeffs, (double*)wtmp.p, (double*)kd, center >= 0 ? (double*)kf.p : nullptr);
     if (rc) return rc;
     P.W = (const double*)wtmp.p; P.kf = (const double*)kf.p; P.nops = nops;
     P.rowptr = rpd; P.col = cd; P.values = (double*)vd;

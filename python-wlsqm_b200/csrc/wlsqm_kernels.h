@@ -105,8 +105,10 @@ constexpr size_t CSR_SMEM_MAX = 227 * 1024;
 struct CsrParams {
     const CaseMeta* meta;
     CaseMeta uni;
-    long long ncases;
-    const int32_t* hoods; int hoods_s0;              // [ncases][hoods_s0], only the first nk_i of row i are read
+    long long ncases;                                // rows: the cases, or the queries when row_case is given
+    const long long* row_case;                       // case of each row (interpolation operators), or nullptr: row i is case i;
+    long long nmodels;                               //   a case outside [0, nmodels) gives an empty row
+    const int32_t* hoods; int hoods_s0;              // [cases][hoods_s0], only the first nk_c of case c are read
     long long center;                                // column of case 0's own point, or -1 (no folding)
     int maxnk;
     long long* cnt;                                  // count pass: distinct columns of row i
@@ -114,6 +116,36 @@ struct CsrParams {
     const double* W; const double* kf; int nops;     // fill pass: stencil weights, folded known-F weights
     void* rowptr; void* col; double* values;         // outputs, int32 or int64 indices; values [nops][nnz]
     long long nnz;
+};
+
+// interpolation operators (wlsqm_operator.cu): per query q, the coefficient rows c_q = (Taylor terms at x[q] - xi[I[q]])
+// applied to coef, contracted with the block of case I[q].  The queries are sorted stably by I; one warp per run of
+// equal I reads that case's block once.  Runs of index nmodels hold the queries whose I is outside [0, nmodels).
+struct InterpRuns {
+    int* keys; int* keys_sorted;                     // [nx] clamped I, sorted
+    int* qidx; int* perm;                            // [nx] 0..nx-1, and the query of each sorted position
+    int* run_case; int* run_len; int* run_off;       // [nx] per run (the first *nruns are valid)
+    int* nruns;                                      // [1]
+};
+struct InterpStencilParams {
+    const CaseMeta* meta;
+    CaseMeta uni;
+    int geom_uniform;
+    long long op_stride;
+    long long nmodels;
+    const double* op;
+    const double* xi;                                // [nmodels][dim] model origins
+    const double* x; long long x_s0;                 // queries
+    int dim;
+    long long nx;
+    const int* run_case; const int* run_len; const int* run_off; const int* nruns; const int* perm;
+    const double* coef;                              // [nops][maxno]
+    int nops, maxnk, maxno;
+    int opc;                                         // operators formed per pass over a query (per-warp shared space)
+    double* W;                                       // [nops][nx][maxnk]
+    double* K;                                       // [nops][nx][maxno] or nullptr
+    double* kf;                                      // [nops][nx] known-F weight for centre folding, or nullptr
+    int stages, stage_doubles, ring_off, cq_off, cq_doubles, bar_off_bytes;
 };
 
 #ifdef __CUDACC__
@@ -173,6 +205,9 @@ cudaError_t launch_stencils(const StencilParams& P, int blocks, int threads, siz
 cudaError_t launch_csr_count(const CsrParams& P, cudaStream_t st);
 cudaError_t csr_scan(long long* cnt, long long* rp, long long n1, void* tmp, size_t* tmp_bytes, cudaStream_t st);
 cudaError_t launch_csr_fill(const CsrParams& P, int index_bits, cudaStream_t st);
+cudaError_t interp_runs(const long long* I, long long nx, long long nmodels, const InterpRuns& R, void* tmp, size_t* tmp_bytes,
+                        cudaStream_t st);
+cudaError_t launch_interp_stencils(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
 struct GridView;
 cudaError_t launch_interpolate_continuous(const InterpParams& P, const GridView& g, double r, cudaStream_t st);
 cudaError_t launch_getrf(int n, long long nlhs, double* A, int* ipiv, cudaStream_t st);

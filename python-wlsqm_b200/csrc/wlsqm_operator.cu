@@ -17,6 +17,12 @@
 // operators from that one read; the coefficients live in shared memory.  Bound by the HBM read of the blocks.
 // csr_kernel<false>: distinct columns per row (count); cub exclusive scan; csr_kernel<true>: columns in ascending
 // order, merged values (fill).  A warp per row; the row's used hood indices are staged in shared memory.
+//
+// Interpolation operators (include/wlsqm_b200.h, DESIGN.md §4 K6): the rows at query points q with model I[q] are the
+// node rows of that model contracted with c_q = (Taylor terms at x[q] - xi[I[q]]) applied to the coefficients.  The
+// queries are sorted stably by I (cub radix sort of 32-bit keys, run-length encoding, scan); interp_stencil_kernel
+// takes one run per warp, streams the model's block once through the ring of stencil_kernel and writes each query's
+// rows at the query's own position through the same contract_case.  csr_kernel<., ., true> maps row q to case I[q].
 #include <cub/cub.cuh>
 #include "wlsqm_common.cuh"
 #include "wlsqm_kernels.h"
@@ -25,6 +31,52 @@ namespace wlsqm {
 
 constexpr int OPX_MAX_THREADS = 1024;
 constexpr int CSR_MAX_WARPS = 8;
+
+// sum over the unknown slots with a nonzero coefficient, ascending, of c[s] * row[j(s)] (FMA chain from 0)
+__device__ __forceinline__ double contract(const double* co, unsigned long long bits, unsigned long long knowns, const double* row) {
+    double acc = 0.0;
+    for (; bits; bits &= bits - 1) {
+        const int s = __ffsll((long long)bits) - 1;
+        const int j = s - __popcll(knowns & ((1ull << s) - 1));
+        acc = fma(co[s], row[j], acc);
+    }
+    return acc;
+}
+
+// The rows of one case (one warp) for nops coefficient rows cs (stride maxno, nonzero slots nzm): W[o][row][k] (lane = k),
+// K[o][row][s] and the known-F weight kf[o][row] (lane = known slot s, its row of the block is nk + its position among
+// the knowns).  Operator o of W / K / kf lies o * nrows rows after the pointer given.  stencil_kernel and
+// interp_stencil_kernel both write their rows here, so that the two definitions cannot drift apart.
+__device__ __forceinline__ void contract_case(const double* op, const CaseMeta& m, const double* cs, const unsigned long long* nzm,
+                                              int nops, int maxno, int maxnk, long long nrows, long long row, double* W,
+                                              double* K, double* kf, int lane) {
+    const int nk = m.nk, no = m.no, nr = m.nr;
+    const unsigned long long knowns = (unsigned long long)m.knowns;
+    const unsigned long long unk = ~knowns & ((1ull << no) - 1);     // no <= 35
+    for (int k = lane; k < maxnk; k += 32) {
+        const double* r = op + k * nr;
+        double* w = W + row * maxnk + k;
+        for (int o = 0; o < nops; ++o) {
+            const double v = k < nk ? contract(cs + o * maxno, nzm[o] & unk, knowns, r) : 0.0;
+            w[(long long)o * nrows * maxnk] = v;
+        }
+    }
+    if (K || kf) {
+        for (int s = lane; s < maxno; s += 32) {
+            const bool kn = s < no && ((knowns >> s) & 1ull);
+            const double* r = op + (nk + __popcll(knowns & ((1ull << s) - 1))) * nr;
+            for (int o = 0; o < nops; ++o) {
+                double v = 0.0;
+                if (kn) v = contract(cs + o * maxno, nzm[o] & unk, knowns, r) + cs[o * maxno + s];
+                if (kf && s == 0) {
+                    kf[(long long)o * nrows + row] = v;   // folded into the fold column of the CSR row
+                    v = 0.0;
+                }
+                if (K) K[((long long)o * nrows + row) * maxno + s] = v;
+            }
+        }
+    }
+}
 
 template <bool UNI>
 __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) stencil_kernel(StencilParams P) {
@@ -78,47 +130,9 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) stencil_kernel(StencilPara
             issue(sn, c + (long long)(S - 1) * GW);
         }
         const CaseMeta m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
-        const int nk = m.nk, no = m.no, nr = m.nr;
-        const unsigned long long knowns = (unsigned long long)m.knowns;
-        const unsigned long long unk = ~knowns & ((1ull << no) - 1);     // no <= 35
         const double* op = ring + (size_t)stage * P.stage_doubles;
         mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
-
-        // sum over the unknown slots with a nonzero coefficient, ascending, of c[s] * row[j(s)]
-        auto contract = [&](const double* co, unsigned long long bits, const double* row) {
-            double acc = 0.0;
-            for (; bits; bits &= bits - 1) {
-                const int s = __ffsll((long long)bits) - 1;
-                const int j = s - __popcll(knowns & ((1ull << s) - 1));
-                acc = fma(co[s], row[j], acc);
-            }
-            return acc;
-        };
-        // neighbour rows: lane = k
-        for (int k = lane; k < P.maxnk; k += 32) {
-            const double* row = op + k * nr;
-            double* w = P.W + c * P.maxnk + k;
-            for (int o = 0; o < nops; ++o) {
-                const double v = k < nk ? contract(cs + o * maxno, nzm[o] & unk, row) : 0.0;
-                w[(long long)o * P.ncases * P.maxnk] = v;
-            }
-        }
-        // known slots: lane = slot m, its row is nk + (its position among the knowns)
-        if (P.K || P.kf) {
-            for (int s = lane; s < maxno; s += 32) {
-                const bool kn = s < no && ((knowns >> s) & 1ull);
-                const double* row = op + (nk + __popcll(knowns & ((1ull << s) - 1))) * nr;
-                for (int o = 0; o < nops; ++o) {
-                    double v = 0.0;
-                    if (kn) v = contract(cs + o * maxno, nzm[o] & unk, row) + cs[o * maxno + s];
-                    if (P.kf && s == 0) {
-                        P.kf[(long long)o * P.ncases + c] = v;   // folded into column center + c of the CSR row
-                        v = 0.0;
-                    }
-                    if (P.K) P.K[((long long)o * P.ncases + c) * maxno + s] = v;
-                }
-            }
-        }
+        contract_case(op, m, cs, nzm, nops, maxno, P.maxnk, P.ncases, c, P.W, P.K, P.kf, lane);
         __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
         if (++stage == S) { stage = 0; phase ^= 1u; }
     }
@@ -139,11 +153,221 @@ cudaError_t launch_stencils(const StencilParams& P, int blocks, int threads, siz
     return cudaGetLastError();
 }
 
+// ---- interpolation operators -----------------------------------------------------------------------------------
+// slot exponents (a | b << 4 | c << 8) per dimension, for runtime slot indices
+struct SlotExpTable { unsigned short e[3][WLSQM_MAXNO]; };
+constexpr SlotExpTable make_slot_exp_table() {
+    SlotExpTable t{};
+    for (int s = 0; s < WLSQM_MAXNO; ++s) {
+        const SlotExp e1 = slot_exp_1d(s), e2 = slot_exp_2d(s), e3 = slot_exp_3d(s);
+        t.e[0][s] = (unsigned short)(e1.a | (e1.b << 4) | (e1.c << 8));
+        t.e[1][s] = (unsigned short)(e2.a | (e2.b << 4) | (e2.c << 8));
+        t.e[2][s] = (unsigned short)(e3.a | (e3.b << 4) | (e3.c << 8));
+    }
+    return t;
+}
+__constant__ SlotExpTable c_slot_exp = make_slot_exp_table();
+
+// One warp per run of queries with the same case m: the case's block is streamed once (the ring of stencil_kernel),
+// then for each query q of the run the lanes form the coefficient rows
+//   c_q[o][s] = sum_{D ascending, coef[o][D] != 0} coef[o][D] * T_D(s),  T_D(s) = (tx[a-p] * ty[b-r]) * tz[c-u]
+// (each product and sum rounded on its own: __dmul_rn / __dadd_rn cannot be contracted), with t[n] = t[n-1] * st[n-1]
+// the Taylor terms of the offset h = x[q] - xi[m] per axis (st = steps_of(h)), and contract them with the block
+// (contract_case) into row q.  A term with T_D(s) = 0 is not added: the sum starts at +0 and never becomes -0, so
+// adding +-0 changes nothing.  Runs of the index nmodels (I outside [0, nmodels)): W row 0, K row NaN.
+template <bool UNI>
+__global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(InterpStencilParams P) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    const int nwarps = blockDim.x >> 5;
+    const int nops = P.nops, maxno = P.maxno, opc = P.opc, dim = P.dim;
+    double* cs = reinterpret_cast<double*>(smem_raw);                                      // [nops][maxno]
+    unsigned long long* nzm = reinterpret_cast<unsigned long long*>(cs + nops * maxno);     // [nops] nonzero slots
+    unsigned short* ex = reinterpret_cast<unsigned short*>(nzm + nops);                     // [maxno] slot exponents
+    for (int t = threadIdx.x; t < nops * maxno; t += blockDim.x) cs[t] = P.coef[t];
+    for (int t = threadIdx.x; t < maxno; t += blockDim.x) ex[t] = c_slot_exp.e[dim - 1][t];
+    __syncthreads();
+    for (int o = warp; o < nops; o += nwarps) {
+        const double* co = cs + o * maxno;
+        const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
+        const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
+        if (lane == 0) nzm[o] = ((unsigned long long)hi << 32) | lo;
+    }
+    __syncthreads();
+
+    // the warp's coefficient rows of one query: cq [opc][maxno], their nonzero slots qnz [opc], Taylor terms tt [3][5]
+    double* cq = reinterpret_cast<double*>(smem_raw) + P.cq_off + (size_t)warp * P.cq_doubles;
+    unsigned long long* qnz = reinterpret_cast<unsigned long long*>(cq + opc * maxno);
+    double* tt = reinterpret_cast<double*>(qnz + opc);
+
+    const int S = P.stages;
+    double* ring = reinterpret_cast<double*>(smem_raw) + P.ring_off + (size_t)warp * S * P.stage_doubles;
+    const uint32_t ring_u32 = smem_u32(ring);
+    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
+    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
+    const long long nruns = *P.nruns;
+    const long long gw = (long long)blockIdx.x * nwarps + warp;
+    const long long GW = (long long)gridDim.x * nwarps;
+    const long long n_my = gw < nruns ? (nruns - gw + GW - 1) / GW : 0;
+
+    auto issue = [&](int s, long long r) {   // lane 0 only
+        const long long c = P.run_case[r];
+        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
+        uint32_t b = 0;
+        CaseMeta m{};
+        if (c < P.nmodels) {
+            m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
+            b = op_block_bytes(m);
+        }
+        mbar_expect_tx_u32(bar, b);
+        if (b) tma_load_1d_u32(st, P.op + m.op_off, b, bar);
+    };
+    if (lane == 0) {
+        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
+        fence_mbar_init();
+        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
+    }
+    __syncwarp();
+
+    int stage = 0;
+    uint32_t phase = 0;
+    long long r = gw;
+    for (long long i = 0; i < n_my; ++i, r += GW) {
+        if (lane == 0 && i + S - 1 < n_my) {
+            int sn = stage + S - 1;
+            if (sn >= S) sn -= S;
+            issue(sn, r + (long long)(S - 1) * GW);
+        }
+        const long long c = P.run_case[r];
+        const int q0 = P.run_off[r], nq = P.run_len[r];
+        const double* op = ring + (size_t)stage * P.stage_doubles;
+        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        if (c >= P.nmodels) {
+            // no model: W row 0, K row NaN (interpolate's NaN for such a query), nothing folded
+            for (int t = 0; t < nq; ++t) {
+                const long long q = P.perm[q0 + t];
+                for (int o = 0; o < nops; ++o) {
+                    for (int k = lane; k < P.maxnk; k += 32) P.W[((long long)o * P.nx + q) * P.maxnk + k] = 0.0;
+                    if (P.K)
+                        for (int s = lane; s < maxno; s += 32)
+                            P.K[((long long)o * P.nx + q) * maxno + s] = __longlong_as_double(0x7ff8000000000000LL);
+                    if (P.kf && lane == 0) P.kf[(long long)o * P.nx + q] = 0.0;
+                }
+            }
+        } else {
+            const CaseMeta m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
+            for (int t = 0; t < nq; ++t) {
+                const long long q = P.perm[q0 + t];
+                if (lane < 3) {     // Taylor terms of axis `lane` (h = 0 beyond the dimension: 1, 0, 0, 0, 0)
+                    const double h = lane < dim ? P.x[q * P.x_s0 + lane] - P.xi[c * dim + lane] : 0.0;
+                    const Steps st = steps_of(h);
+                    double tv = 1.0;
+                    tt[lane * 5] = tv;
+#pragma unroll
+                    for (int n = 1; n < 5; ++n) {
+                        tv = __dmul_rn(tv, st.s[n - 1]);
+                        tt[lane * 5 + n] = tv;
+                    }
+                }
+                __syncwarp();
+                for (int o0 = 0; o0 < nops; o0 += opc) {
+                    const int oc = min(opc, nops - o0);
+                    for (int idx = lane; idx < oc * maxno; idx += 32) {
+                        const int o = idx / maxno, s = idx - o * maxno;
+                        const int es = ex[s], a = es & 15, b = (es >> 4) & 15, cz = es >> 8;
+                        const double* co = cs + (o0 + o) * maxno;
+                        double acc = 0.0;
+                        for (unsigned long long bits = nzm[o0 + o]; bits; bits &= bits - 1) {
+                            const int D = __ffsll((long long)bits) - 1;
+                            const int ed = ex[D], p = ed & 15, pr = (ed >> 4) & 15, pu = ed >> 8;
+                            if (a >= p && b >= pr && cz >= pu) {
+                                const double T = __dmul_rn(__dmul_rn(tt[a - p], tt[5 + b - pr]), tt[10 + cz - pu]);
+                                acc = __dadd_rn(acc, __dmul_rn(co[D], T));
+                            }
+                        }
+                        cq[idx] = acc;
+                    }
+                    __syncwarp();
+                    for (int o = 0; o < oc; ++o) {
+                        const double* co = cq + o * maxno;
+                        const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
+                        const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
+                        if (lane == 0) qnz[o] = ((unsigned long long)hi << 32) | lo;
+                    }
+                    __syncwarp();
+                    contract_case(op, m, cq, qnz, oc, maxno, P.maxnk, P.nx, q, P.W + (long long)o0 * P.nx * P.maxnk,
+                                  P.K ? P.K + (long long)o0 * P.nx * maxno : nullptr, P.kf ? P.kf + (long long)o0 * P.nx : nullptr,
+                                  lane);
+                    __syncwarp();   // cq / qnz / tt are rewritten for the next pass or query
+                }
+            }
+        }
+        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
+        if (++stage == S) { stage = 0; phase ^= 1u; }
+    }
+}
+
+cudaError_t launch_interp_stencils(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st) {
+    const bool uni = P.meta == nullptr || P.geom_uniform;
+    cudaError_t e;
+    if (uni) {
+        e = cudaFuncSetAttribute(interp_stencil_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        interp_stencil_kernel<true><<<blocks, threads, smem, st>>>(P);
+    } else {
+        e = cudaFuncSetAttribute(interp_stencil_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        interp_stencil_kernel<false><<<blocks, threads, smem, st>>>(P);
+    }
+    return cudaGetLastError();
+}
+
+// keys[q] = I[q] when it is a case index, else nmodels; qidx[q] = q
+__global__ void interp_keys_kernel(const long long* __restrict__ I, long long nx, long long nmodels, int* __restrict__ keys,
+                                   int* __restrict__ qidx) {
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < nx; q += (long long)gridDim.x * blockDim.x) {
+        const long long m = I[q];
+        keys[q] = (int)(m >= 0 && m < nmodels ? m : nmodels);
+        qidx[q] = (int)q;
+    }
+}
+
+// The runs of equal case index among the queries: a stable radix sort of (key, q) on the bits that keys <= nmodels use,
+// then run-length encoding and an exclusive scan of the run lengths.  tmp == nullptr: *tmp_bytes := the scratch needed.
+cudaError_t interp_runs(const long long* I, long long nx, long long nmodels, const InterpRuns& R, void* tmp, size_t* tmp_bytes,
+                        cudaStream_t st) {
+    int end_bit = 1;
+    while (end_bit < 32 && (1LL << end_bit) <= nmodels) ++end_bit;
+    const int n = (int)nx;
+    if (!tmp) {
+        size_t a = 0, b = 0, c = 0;
+        cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, a, R.keys, R.keys_sorted, R.qidx, R.perm, n, 0, end_bit, st);
+        if (e == cudaSuccess) e = cub::DeviceRunLengthEncode::Encode(nullptr, b, R.keys_sorted, R.run_case, R.run_len, R.nruns, n, st);
+        if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(nullptr, c, R.run_len, R.run_off, n, st);
+        *tmp_bytes = std::max(a, std::max(b, c));
+        return e;
+    }
+    const unsigned blocks = (unsigned)std::max<long long>(1, std::min<long long>((nx + 255) / 256, 148LL * 32));
+    interp_keys_kernel<<<blocks, 256, 0, st>>>(I, nx, nmodels, R.keys, R.qidx);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemsetAsync(R.run_len, 0, (size_t)nx * sizeof(int), st);
+    size_t tb = *tmp_bytes;
+    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(tmp, tb, R.keys, R.keys_sorted, R.qidx, R.perm, n, 0, end_bit, st);
+    tb = *tmp_bytes;
+    if (e == cudaSuccess) e = cub::DeviceRunLengthEncode::Encode(tmp, tb, R.keys_sorted, R.run_case, R.run_len, R.nruns, n, st);
+    tb = *tmp_bytes;
+    if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(tmp, tb, R.run_len, R.run_off, n, st);
+    return e;
+}
+
 // One warp per CSR row.  FILL = false: the number of distinct columns of row i -> cnt[i].  FILL = true: columns in
 // ascending order at rp[i] ..., each with its W entries summed in ascending k, the folded known-F weight added last.
 // A column's rank is the number of distinct columns below it, so no sort is needed: an O(nk^2) comparison per row
 // against the indices staged in shared memory (broadcast reads).
-template <bool FILL, typename IDX>
+// MAP (P.row_case given): row i belongs to case c = row_case[i] -- the neighbour list, record and fold column
+// center + c are the case's, W / kf / the output the row's; a case outside [0, nmodels) gives an empty row.
+template <bool FILL, typename IDX, bool MAP>
 __global__ void __launch_bounds__(CSR_MAX_WARPS * 32) csr_kernel(CsrParams P) {
     extern __shared__ int csr_smem[];
     const int lane = threadIdx.x & 31;
@@ -155,13 +379,20 @@ __global__ void __launch_bounds__(CSR_MAX_WARPS * 32) csr_kernel(CsrParams P) {
                                                               // bit 0: first occurrence, bit 1: occurs again later
     const long long GW = (long long)gridDim.x * nwarps;
     for (long long i = (long long)blockIdx.x * nwarps + warp; i < P.ncases; i += GW) {
-        const CaseMeta m = P.meta ? P.meta[i] : P.uni;
-        const int nk = m.nk;
-        const int32_t* hr = P.hoods + i * P.hoods_s0;
+        long long c = i;
+        bool live = true;
+        if (MAP) {
+            c = P.row_case[i];
+            live = c >= 0 && c < P.nmodels;
+            if (!live) c = 0;
+        }
+        const CaseMeta m = P.meta ? P.meta[c] : P.uni;
+        const int nk = live ? m.nk : 0;
+        const int32_t* hr = P.hoods + c * P.hoods_s0;
         for (int k = lane; k < nk; k += 32) hs[k] = hr[k];
         __syncwarp();
-        const bool fold = P.center >= 0 && (m.knowns & 1LL);
-        const long long fc = P.center + i;
+        const bool fold = live && P.center >= 0 && (m.knowns & 1LL);
+        const long long fc = P.center + c;
         int cnt = 0;
         bool fc_in = false;
         for (int k = lane; k - lane < nk; k += 32) {
@@ -236,14 +467,18 @@ static cudaError_t launch_csr(Kernel kernel, const CsrParams& P, cudaStream_t st
     return cudaGetLastError();
 }
 
-cudaError_t launch_csr_count(const CsrParams& P, cudaStream_t st) { return launch_csr(csr_kernel<false, int>, P, st); }
+cudaError_t launch_csr_count(const CsrParams& P, cudaStream_t st) {
+    return P.row_case ? launch_csr(csr_kernel<false, int, true>, P, st) : launch_csr(csr_kernel<false, int, false>, P, st);
+}
 
 cudaError_t csr_scan(long long* cnt, long long* rp, long long n1, void* tmp, size_t* tmp_bytes, cudaStream_t st) {
     return cub::DeviceScan::ExclusiveSum(tmp, *tmp_bytes, cnt, rp, (int)n1, st);
 }
 
 cudaError_t launch_csr_fill(const CsrParams& P, int index_bits, cudaStream_t st) {
-    return index_bits == 32 ? launch_csr(csr_kernel<true, int32_t>, P, st) : launch_csr(csr_kernel<true, long long>, P, st);
+    if (P.row_case)
+        return index_bits == 32 ? launch_csr(csr_kernel<true, int32_t, true>, P, st) : launch_csr(csr_kernel<true, long long, true>, P, st);
+    return index_bits == 32 ? launch_csr(csr_kernel<true, int32_t, false>, P, st) : launch_csr(csr_kernel<true, long long, false>, P, st);
 }
 
 }  // namespace wlsqm

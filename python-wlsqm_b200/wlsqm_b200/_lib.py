@@ -66,6 +66,9 @@ SIGNATURES = {
     "wlsqm_solver_stencils": (_int, [_vp, _int, _vp, _vp, _vp]),
     "wlsqm_solver_operator_nnz": (_int, [_vp, _i64, _vp]),
     "wlsqm_solver_operator_csr": (_int, [_vp, _int, _vp, _i64, _int, _vp, _vp, _vp, _vp]),
+    "wlsqm_solver_interp_stencils": (_int, [_vp, _vp, _i64, _vp, _i64, _int, _vp, _vp, _vp]),
+    "wlsqm_solver_interp_operator_nnz": (_int, [_vp, _vp, _i64, _i64, _vp]),
+    "wlsqm_solver_interp_operator_csr": (_int, [_vp, _vp, _i64, _vp, _i64, _int, _vp, _i64, _int, _vp, _vp, _vp, _vp]),
     "wlsqm_solver_index_models": (_int, [_vp]),
     "wlsqm_solver_nearest_models": (_int, [_vp, _vp, _i64, _i64, _vp]),
     "wlsqm_solver_interpolate_continuous": (_int, [_vp, _vp, _i64, _i64, C.c_double, _int, _vp]),

@@ -740,6 +740,43 @@ class ExpertSolver:
             xi_rank2 = xi if self.dimension >= 2 else np.atleast_2d(xi).T
             self.tree = scipy.spatial.cKDTree(data=xi_rank2)
 
+    def _nearest_models(self, x, uintptr_t xp, int64_t x_s0, Py_ssize_t nx, bint x_cuda, I):
+        """(I_use, I_out): the model of every query in mode='nearest' -- I itself when given, else the nearest origin
+        by self.tree (the device grid for CUDA queries or search='gpu', I then stays where x lives; cKDTree otherwise).
+        interpolate() and the interpolation operators (fitter/opexport.py) resolve their models here."""
+        cdef uintptr_t ip
+        if I is not None:
+            return I, I
+        if isinstance(self.tree, _DeviceModelIndex) or x_cuda:
+            # nearest model by the device-side grid (extension); I stays where x lives
+            if x_cuda:
+                I_out = _torch.empty((nx,), dtype=_torch.int64, device=x.device)
+                ip = I_out.data_ptr()
+            else:
+                I_out = np.empty((nx,), dtype=np.int_)
+                ip = I_out.ctypes.data
+            _lib.announce_stream(self.device)
+            _check(wlsqm_solver_nearest_models(_h(self), <const double*>xp, x_s0, nx, <int64_t*>ip))
+            return I_out, I_out
+        xh = np.asarray(x)
+        xq = xh if self.dimension >= 2 else np.atleast_2d(xh).T
+        _d, I_h = self.tree.query(xq, k=1)
+        I_out = np.ascontiguousarray(I_h, dtype=np.int_)
+        return I_out, I_out
+
+    # -- interpolation operators (extension; wlsqm_b200/fitter/opexport.py) -------------------------------------------
+    def interp_stencils(self, x, coeffs=0, I=None):
+        """(W, K, I_out): the map from the data to interpolate(x, mode='nearest') as per-query weights -- W (nops, nx,
+        max nk) on fk[I[q]], K (nops, nx, max no) on the known values of model I[q], for the coefficient rows coeffs over
+        the derivative slots (an int slot, a (max no,) row or a (nops, max no) array).  I=None: the nearest models, found
+        as interpolate() finds them.  See wlsqm_b200.fitter.opexport.interp_stencils."""
+        return _opexport.interp_stencils(self, x, coeffs, I)
+
+    def interp_operator(self, x, coeffs=0, I=None, center=None):
+        """(E, K, I_out): the same map as a sparse matrix (nx, npoints) over the points of prepare_hoods, like operator().
+        See wlsqm_b200.fitter.opexport.interp_operator."""
+        return _opexport.interp_operator(self, x, coeffs, I, center)
+
     def interpolate(self, x, mode='nearest', r=None, diff=0, I=None):
         """Interpolate the global patched model or one derivative of it (``expert.pyx:687-781``).
 
@@ -779,26 +816,7 @@ class ExpertSolver:
         if mode == 'continuous':
             return self._interpolate_continuous(x, <uintptr_t>ax.p, x_s0, nx, ax.cuda, float(r), cdiff), np.asanyarray(None)
 
-        if I is None and (isinstance(self.tree, _DeviceModelIndex) or ax.cuda):
-            # nearest model by the device-side grid (extension); I stays where x lives
-            if ax.cuda:
-                I_out = _torch.empty((nx,), dtype=_torch.int64, device=x.device)
-                ip = I_out.data_ptr()
-            else:
-                I_out = np.empty((nx,), dtype=np.int_)
-                ip = I_out.ctypes.data
-            _lib.announce_stream(self.device)
-            _check(wlsqm_solver_nearest_models(h, ax.p, x_s0, nx, <int64_t*>ip))
-            I_use = I_out
-        elif I is None:
-            xh = np.asarray(x)
-            xq = xh if dim >= 2 else np.atleast_2d(xh).T
-            _d, I_h = self.tree.query(xq, k=1)
-            I_out = np.ascontiguousarray(I_h, dtype=np.int_)
-            I_use = I_out
-        else:
-            I_use = I
-            I_out = I
+        I_use, I_out = self._nearest_models(x, <uintptr_t>ax.p, x_s0, nx, ax.cuda, I)
         i_cuda = _is_tensor(I_use) and I_use.is_cuda
         if i_cuda:
             if I_use.dtype != _torch.int64 or I_use.dim() != 1 or (nx > 1 and I_use.stride(0) != 1):

@@ -372,6 +372,42 @@ class ExpertSolver:
             xi_rank2 = xi if self.dimension >= 2 else np.atleast_2d(xi).T
             self.tree = scipy.spatial.cKDTree(data=xi_rank2)
 
+    def _nearest_models(self, x, xp, x_s0, nx, x_cuda, I):
+        """(I_use, I_out): the model of every query in mode='nearest' -- I itself when given, else the nearest origin
+        by self.tree (the device grid for CUDA queries or search='gpu', I then stays where x lives; cKDTree otherwise).
+        interpolate() and the interpolation operators (opexport.py) resolve their models here."""
+        if I is not None:
+            return I, I
+        if isinstance(self.tree, _DeviceModelIndex) or x_cuda:
+            # nearest model by the device-side grid (extension); I stays where x lives
+            if x_cuda:
+                import torch
+                I_out = torch.empty((nx,), dtype=torch.int64, device=x.device)
+                ip = int(I_out.data_ptr())
+            else:
+                I_out = np.empty((nx,), dtype=np.int_)
+                ip = I_out.ctypes.data
+            _lib.check(_lib.lib().wlsqm_solver_nearest_models(self._handle, xp, x_s0, nx, ip))
+            return I_out, I_out
+        xh = np.asarray(x)
+        xq = xh if self.dimension >= 2 else np.atleast_2d(xh).T
+        _d, I_h = self.tree.query(xq, k=1)
+        I_out = np.ascontiguousarray(I_h, dtype=np.int_)
+        return I_out, I_out
+
+    # -- interpolation operators (extension; opexport.py) -----------------------------------------------------------------
+    def interp_stencils(self, x, coeffs=0, I=None):
+        """(W, K, I_out): the map from the data to interpolate(x, mode='nearest') as per-query weights -- W (nops, nx,
+        max nk) on fk[I[q]], K (nops, nx, max no) on the known values of model I[q], for the coefficient rows coeffs over
+        the derivative slots (an int slot, a (max no,) row or a (nops, max no) array).  I=None: the nearest models, found
+        as interpolate() finds them.  See wlsqm_b200.fitter.opexport.interp_stencils."""
+        return opexport.interp_stencils(self, x, coeffs, I)
+
+    def interp_operator(self, x, coeffs=0, I=None, center=None):
+        """(E, K, I_out): the same map as a sparse matrix (nx, npoints) over the points of prepare_hoods, like operator().
+        See wlsqm_b200.fitter.opexport.interp_operator."""
+        return opexport.interp_operator(self, x, coeffs, I, center)
+
     def interpolate(self, x, mode='nearest', r=None, diff=0, I=None):
         """Interpolate the global patched model or one derivative of it (``expert.pyx:687-781``).
 
@@ -401,26 +437,7 @@ class ExpertSolver:
         if mode == 'continuous':
             return self._interpolate_continuous(x_a, x_s0, float(r), cdiff), np.asanyarray(None)
 
-        if I is None and (isinstance(self.tree, _DeviceModelIndex) or x_a.is_cuda):
-            # nearest model by the device-side grid (extension); I stays where x lives
-            if x_a.is_cuda:
-                import torch
-                I_out = torch.empty((nx,), dtype=torch.int64, device=x.device)
-                ip = int(I_out.data_ptr())
-            else:
-                I_out = np.empty((nx,), dtype=np.int_)
-                ip = I_out.ctypes.data
-            _lib.check(_lib.lib().wlsqm_solver_nearest_models(self._handle, x_a.ptr, x_s0, nx, ip))
-            I_use = I_out
-        elif I is None:
-            xh = np.asarray(x)
-            xq = xh if dim >= 2 else np.atleast_2d(xh).T
-            _d, I_h = self.tree.query(xq, k=1)
-            I_out = np.ascontiguousarray(I_h, dtype=np.int_)
-            I_use = I_out
-        else:
-            I_use = I
-            I_out = I
+        I_use, I_out = self._nearest_models(x, x_a.ptr, x_s0, nx, x_a.is_cuda, I)
         I_a = _lib.as_arr(I_use, np.int64, 1, "I")
         if not I_a.is_cuda and I_a.strides[0] != 1 and nx > 1:
             raise ValueError("I: ndarray is not C-contiguous")

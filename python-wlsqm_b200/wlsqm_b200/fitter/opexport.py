@@ -6,6 +6,12 @@ map that ``prepare`` stored is contracted on the device with caller-given coeffi
 ``c[i2_X2] = c[i2_Y2] = 1``) and, for ``prepare_hoods`` solvers, assembled into a CSR matrix over the point cloud.
 Definitions: ``include/wlsqm_b200.h`` (``wlsqm_solver_stencils`` / ``wlsqm_solver_operator_csr``).
 
+The interpolation operators do the same at arbitrary query points: the map from the data to
+``interpolate(x, mode='nearest', diff)`` (``expert.pyx:687-781``), whose row for query q is the operator of its model
+I[q] contracted with the Taylor terms of the offset x[q] - xi[I[q]] (``wlsqm_solver_interp_stencils`` /
+``wlsqm_solver_interp_operator_csr``).  For fixed queries one CSR product replaces a solve followed by an interpolate;
+mesh-to-mesh transfer, boundary conditions at points that are not fit origins and observation operators are such maps.
+
 Both bindings of ``ExpertSolver`` (the Cython shim and the ctypes twin) call these functions.
 """
 from __future__ import annotations
@@ -119,3 +125,99 @@ def operator(solver, coeffs, center=None):
         import scipy.sparse as sp
         mats = [sp.csr_array((values[o], col, rowptr), shape=(n, npoints)) for o in range(nops)]
     return (mats[0], K[0]) if squeeze else (mats, K)
+
+
+def _queries(solver, x, I):
+    """-> (x Arr, row stride, nx, int64 index array for the C ABI, I_out): the query points and their models, resolved
+    as ``interpolate(x, mode='nearest', I=I)`` resolves them (``solver._nearest_models``)."""
+    dim = solver.dimension
+    x_a = _lib.as_arr(x, np.float64, 2 if dim >= 2 else 1, "x", last_contig=dim >= 2)
+    nx = x_a.shape[0]
+    if dim >= 2 and x_a.shape[1] < dim:
+        raise ValueError("x must have %d coordinates on its last axis" % dim)
+    x_s0 = x_a.strides[0] if nx > 1 or dim >= 2 else dim
+    if not x_a.is_cuda and dim == 1 and nx > 1 and x_s0 != 1:
+        x_a = _lib.as_arr(np.ascontiguousarray(x_a.np), np.float64, 1, "x", last_contig=False)
+        x_s0 = 1
+    if I is None and solver.tree is None:
+        raise RuntimeError("Points xi have not been indexed; prep_interpolate() must be called before the nearest models "
+                           "can be found (or pass I)")
+    if I is not None and len(I) != nx:
+        raise ValueError("When 'I' is specified, 'I' must have the same length as x; got len(I) = %d, len(x) = %d."
+                         % (len(I), nx))
+    solver._use_stream()
+    I_use, I_out = solver._nearest_models(x, x_a.ptr, x_s0, nx, x_a.is_cuda, I)
+    if _lib._is_torch_tensor(I_use) and I_use.is_cuda:
+        import torch
+        if I_use.dtype != torch.int64 or I_use.dim() != 1 or (nx > 1 and I_use.stride(0) != 1):
+            raise ValueError("I: a contiguous int64 tensor of shape (nx,) is required")
+        I_c = I_use
+    else:
+        if _lib._is_torch_tensor(I_use):
+            I_use = I_use.detach().cpu().numpy()
+        I_c = np.ascontiguousarray(I_use, dtype=np.int64)
+        if I_c.ndim != 1:
+            raise ValueError("I must be one-dimensional")
+    if not (x_a.is_cuda and _lib._is_torch_tensor(I_out)):
+        I_out = np.asanyarray(I_out)
+    return x_a, x_s0, nx, I_c, I_out
+
+
+def interp_stencils(solver, x, coeffs=0, I=None):
+    """(W, K, I_out): the interpolation operators at the query points x as per-query weights.
+
+    W (nops, nx, max nk) weights on the data of model I[q]'s neighbours, K (nops, nx, max no) on its known values, so
+    that for an ALGO_BASIC solve  sum_D coeffs[D] d^D f(x[q]) = W[q] . fk[I[q]] + K[q] . fi[I[q]]  with d^D f the value
+    interpolate(x, mode='nearest', diff=D) returns.  The nops axis is dropped for an int slot or a 1-D row.  I=None: the
+    nearest models, found as interpolate() finds them (I_out returns them); a query without a model (I outside
+    [0, ncases)) has W row 0 and K row NaN.  CUDA tensors when the solver was prepared from CUDA tensors."""
+    c, squeeze = coefficient_rows(coeffs, solver._maxno)
+    x_a, x_s0, nx, I_c, I_out = _queries(solver, x, I)
+    root = _root(solver)
+    cuda = getattr(root, "_cuda_out", False)
+    nops = c.shape[0]
+    W = _empty((nops, nx, solver._maxnk), np.float64, cuda, solver.device)
+    K = _empty((nops, nx, solver._maxno), np.float64, cuda, solver.device)
+    _lib.check(_lib.lib().wlsqm_solver_interp_stencils(solver._handle, x_a.ptr, x_s0, _ptr(I_c), nx, nops, c.ctypes.data,
+                                                       _ptr(W), _ptr(K)))
+    return (W[0], K[0], I_out) if squeeze else (W, K, I_out)
+
+
+def interp_operator(solver, x, coeffs=0, I=None, center=None):
+    """(E, K, I_out): the interpolation operators as a sparse matrix over the points of ``prepare_hoods``.
+
+    E (nx, npoints), rows in the order of x: a ``torch.sparse_csr_tensor`` or a ``scipy.sparse.csr_array`` by the rule
+    of ``operator()`` (a list of nops matrices sharing one index pair for 2-D coeffs), so that
+    sum_D coeffs[D] d^D f(x[q]) = (E @ f)[q] + K[q] . fi[I[q]].  ``center``: index in x of case 0's own point; the weight
+    on a known F of model I[q] then moves into column center + I[q] and is 0 in K.  A query without a model has an
+    empty row and a NaN K row."""
+    c, squeeze = coefficient_rows(coeffs, solver._maxno)
+    if center is None:
+        center = -1
+    else:
+        center = int(center)
+        if center < 0:
+            raise ValueError("center must be >= 0, got %d" % center)
+    x_a, x_s0, nx, I_c, I_out = _queries(solver, x, I)
+    root = _root(solver)
+    L = _lib.lib()
+    nnz = C.c_int64(0)
+    _lib.check(L.wlsqm_solver_interp_operator_nnz(solver._handle, _ptr(I_c), nx, center, C.byref(nnz)))
+    nnz = int(nnz.value)
+    cuda = getattr(root, "_cuda_out", False)
+    nops, npoints = c.shape[0], int(getattr(root, "_hood_points", 0))
+    bits = 32 if nnz < 2 ** 31 else 64
+    it = np.int32 if bits == 32 else np.int64
+    rowptr = _empty((nx + 1,), it, cuda, solver.device)
+    col = _empty((nnz,), it, cuda, solver.device)
+    values = _empty((nops, nnz), np.float64, cuda, solver.device)
+    K = _empty((nops, nx, solver._maxno), np.float64, cuda, solver.device)
+    _lib.check(L.wlsqm_solver_interp_operator_csr(solver._handle, x_a.ptr, x_s0, _ptr(I_c), nx, nops, c.ctypes.data,
+                                                  center, bits, _ptr(rowptr), _ptr(col), _ptr(values), _ptr(K)))
+    if cuda:
+        import torch
+        mats = [torch.sparse_csr_tensor(rowptr, col, values[o], size=(nx, npoints)) for o in range(nops)]
+    else:
+        import scipy.sparse as sp
+        mats = [sp.csr_array((values[o], col, rowptr), shape=(nx, npoints)) for o in range(nops)]
+    return (mats[0], K[0], I_out) if squeeze else (mats, K, I_out)

@@ -195,6 +195,33 @@ WLSQM_API int wlsqm_solver_prepare_hoods(wlsqm_solver_t* s, const double* x, int
 WLSQM_API int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, double* fi, int64_t fi_s0,
                              double* sens, int64_t sens_s0, int64_t sens_s1, int32_t* iters_out);
 
+/* Several fields on one geometry in one pass (extension): the operator blocks are streamed once per pass for all fields
+ * of the pass instead of once per field (the reference solves each field with its own solve, or with a guest solver).
+ * fk [nf][ncases][>= max nk] (strides fk_sf, fk_s0, fk_s1, device arrays fully strided as in wlsqm_solver_solve);
+ * fi [nf][ncases][>= max no] in/out (field stride fi_sf, row stride fi_s0, contiguous last axis).  For every field j the
+ * unknown slots of fi[j] receive BIT FOR BIT what wlsqm_solver_solve(fk[j], fi[j]) writes on the same solver (same
+ * algorithm, kernel path and summation order, ALGO_ITERATIVE refinement with its exact-equality exit per field); known
+ * slots and slots >= no_i are not written.  *iters_out (may be NULL) is the maximum of the per-field solve return values;
+ * wlsqm_solver_iterations afterwards gives the per-case maximum over the fields.
+ *   - The solver's own solution copy is not written: interpolate / get_fi fail with WLSQM_E_NOTREADY until the next
+ *     wlsqm_solver_solve (as after keep_solution(0)).
+ *   - sens is not produced (it does not depend on the data: take it from one solve or from wlsqm_solver_stencils); a
+ *     do_sens solver is accepted.
+ *   - WLSQM_E_VALUE: device fk overlapping device fi; an fi layout whose (field, case, slot) map is not injective -- accepted
+ *     are fields-outer (fi_sf >= (ncases-1)*fi_s0 + max no, fi_s0 >= max no) and fields-inner (fi_sf >= max no,
+ *     fi_s0 >= (nf-1)*fi_sf + max no) with non-negative strides; an active fused gather (wlsqm_solver_set_gather).
+ *   - nf = 0 or ncases = 0: no-op, returns 0.  Cases with nr == 0 or nq == 0 behave as in wlsqm_solver_solve.
+ *   - Host fk / fi are staged whole (so a host fk aliasing the host fi reads the values from before the call); device
+ *     arrays are used in place, asynchronously on the solver's stream.  A guest answers with its host's operators.
+ *   - The fields of a pass share the shared-memory ring of the single-field launch shape; nf above what it holds runs
+ *     several passes, each streaming the operators again.
+ * wlsqm_solver_solve_hoods_fields: the same with the data per point, f [nf][>= npoints] (strides f_sf, f_s0, any), each
+ * field equal bit for bit to wlsqm_solver_solve_hoods(f[j], fi[j]); needs prepare_hoods (WLSQM_E_NOTREADY otherwise). */
+WLSQM_API int wlsqm_solver_solve_fields(wlsqm_solver_t* s, int64_t nf, const double* fk, int64_t fk_sf, int64_t fk_s0,
+                                        int64_t fk_s1, double* fi, int64_t fi_sf, int64_t fi_s0, int32_t* iters_out);
+WLSQM_API int wlsqm_solver_solve_hoods_fields(wlsqm_solver_t* s, int64_t nf, const double* f, int64_t f_sf, int64_t f_s0,
+                                              double* fi, int64_t fi_sf, int64_t fi_s0, int32_t* iters_out);
+
 /* Export of the prepared operators (extension).  The reference offers the linear map from data to fitted DOFs only
  * as `sens` (impl.pyx:769-779, d fi / d fk, recomputed by every solve), from which its callers assemble Jacobians.
  * Here each of nops operators is a row of coeffs (host memory, [nops][max no], finite, 1 <= nops <= WLSQM_MAXNO): a

@@ -154,13 +154,15 @@ struct DevBuf {
     }
 };
 
-// dst[i][k][0..w) = src[idx[i][k]][0..w).  Only the first nk_i neighbours of case i are read (nk_i from the per-case
-// records, else nk_uni; negative: all k columns): the padding of a ragged hood array (cKDTree and wlsqm_grid_knn both
-// report missing neighbours as the index n) is never dereferenced and its slots are zero-filled.  An index outside
-// [0, nsrc) among the USED slots -- where the reference's x[hoods] raises IndexError -- gives NaN and raises *err.
+// dst[f][i][k][0..w) = src[f][idx[i][k]][0..w) for the nf fields f (src field stride src_sf, dst field stride dst_sf).
+// Only the first nk_i neighbours of case i are read (nk_i from the per-case records, else nk_uni; negative: all k
+// columns): the padding of a ragged hood array (cKDTree and wlsqm_grid_knn both report missing neighbours as the index
+// n) is never dereferenced and its slots are zero-filled.  An index outside [0, nsrc) among the USED slots -- where the
+// reference's x[hoods] raises IndexError -- gives NaN and raises *err.
 __global__ void gather_hoods_kernel(const double* __restrict__ src, long long src_s0, int w, const int32_t* __restrict__ idx,
                                     long long idx_s0, long long n, int k, double* __restrict__ dst, long long nsrc,
-                                    const CaseMeta* __restrict__ meta, int nk_uni, int* __restrict__ err) {
+                                    const CaseMeta* __restrict__ meta, int nk_uni, int* __restrict__ err, int nf = 1,
+                                    long long src_sf = 0, long long dst_sf = 0) {
     const long long per = (long long)k * w;
     for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t < n * per;
          t += (long long)gridDim.x * blockDim.x) {
@@ -168,16 +170,17 @@ __global__ void gather_hoods_kernel(const double* __restrict__ src, long long sr
         const int r = (int)(t - i * per);
         const int kk = r / w, d = r - kk * w;
         const int nki = meta ? meta[i].nk : (nk_uni >= 0 ? nk_uni : k);
-        double v = 0.0;
         if (kk < nki) {
             const long long j = idx[i * idx_s0 + kk];
-            if (j >= 0 && j < nsrc) v = src[j * src_s0 + d];
-            else {
-                v = __longlong_as_double(0x7ff8000000000000LL);
+            if (j >= 0 && j < nsrc) {
+                for (int f = 0; f < nf; ++f) dst[t + f * dst_sf] = src[f * src_sf + j * src_s0 + d];
+            } else {
+                for (int f = 0; f < nf; ++f) dst[t + f * dst_sf] = __longlong_as_double(0x7ff8000000000000LL);
                 if (err) *err = 1;
             }
+        } else {
+            for (int f = 0; f < nf; ++f) dst[t + f * dst_sf] = 0.0;
         }
-        dst[t] = v;
     }
 }
 
@@ -459,6 +462,44 @@ int config_solve_pack(const wlsqm_solver* s, SolveParams& P, LaunchCfg& L, long 
     ctas = std::max(1, std::min(ctas, std::max(1, env_int("WLSQM_SOLVE_MAXWARPS_SM", 32) / warps)));
     const long long packs = (ncases_launch + cpw - 1) / cpw;
     long long need = (packs + warps - 1) / warps;
+    L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    return WLSQM_OK;
+}
+
+// Field-batched solve: the launch shape of the single-field solve (ring depth, fext / known-value slot sizes, warps per
+// CTA -- at most SOLVE_FIELDS_THREADS: 128 registers for the accumulators of 8 fields, or the refinement of a field) with
+// every stage widened by one data slot per further field.  F.nf is lowered to the fields that the shared memory of that
+// shape holds (at least 1: the single-field shape fits).  F.P.fk / fk strides and F.fk_sf must be set (bulk-copy
+// eligibility).
+int config_solve_fields(const wlsqm_solver* s, FieldsParams& F, LaunchCfg& L, long long ncases_launch, bool pack) {
+    SolveParams& P = F.P;
+    const int rc = pack ? config_solve_pack(s, P, L, ncases_launch) : config_solve(s, P, L, ncases_launch);
+    if (rc) return rc;
+    const bool iter = s->algorithm == WLSQM_ALGO_ITERATIVE;
+    const int warps = std::min(L.threads / 32, SOLVE_FIELDS_THREADS / 32);
+    const int S = P.stages;
+    const int op_d = P.off_f, f_d = P.off_xk - P.off_f, x_d = P.stage_doubles - P.off_xk;
+    const int tail = pack ? 0 : 36 + (iter ? std::max(2, even(s->maxnk)) : 0);     // fis + rs per warp (solve_kernel)
+    auto stage_of = [&](int nfp) { return pack ? op_d + nfp * (f_d + x_d) : op_d + nfp * f_d + x_d; };
+    auto warp_of = [&](int nfp) { return (S * stage_of(nfp) + tail + 15) & ~15; };
+    int nfp = std::max(1, F.nf);
+    while (nfp > 1 && (size_t)warps * ((size_t)warp_of(nfp) * 8 + (size_t)S * 8) > SMEM_PER_CTA) --nfp;
+    F.nf = nfp;
+    F.f_doubles = f_d;
+    F.k_doubles = pack ? x_d : 0;
+    P.stage_doubles = stage_of(nfp);
+    P.off_xk = op_d + nfp * f_d;
+    P.off_fi = S * P.stage_doubles;
+    P.off_r = P.off_fi + 36;
+    P.warp_doubles = warp_of(nfp);
+    if (nfp > 1 && (F.fk_sf % 2)) P.f_tma = 0;     // every field's rows must start 16 B aligned
+    P.bar_off_bytes = warps * P.warp_doubles * 8;
+    L.threads = warps * 32;
+    L.smem = (size_t)P.bar_off_bytes + (size_t)warps * S * 8;
+    int ctas = (int)(SMEM_PER_SM / (L.smem + 1024));
+    ctas = std::max(1, std::min(ctas, std::max(1, 16 / warps)));
+    const long long units = pack ? (ncases_launch + (32 >> P.pack_lw) - 1) / (32 >> P.pack_lw) : ncases_launch;
+    const long long need = (units + warps - 1) / warps;
     L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
     return WLSQM_OK;
 }
@@ -1468,6 +1509,171 @@ int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, d
         s->uni.nk, nullptr);
     CU(cudaGetLastError());
     return wlsqm_solver_solve(s, (const double*)s->hood_fk.p, kp, 1, fi, fi_s0, sens, sens_s0, sens_s1, iters_out);
+}
+
+// Several fields on one geometry (wlsqm_solve.cu, FieldsParams): fk given per case, or (hoods) per point through the
+// neighbour lists of prepare_hoods (hf [nf][npoints], strides f_sf / f_s0).
+static int solve_fields_core(wlsqm_solver_t* s, int64_t nf, bool hoods, const double* fk, int64_t fk_sf, int64_t fk_s0,
+                             int64_t fk_s1, const double* hf, int64_t f_sf, int64_t f_s0, double* fi, int64_t fi_sf, int64_t fi_s0,
+                             int32_t* iters_out) {
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    if (iters_out) *iters_out = 0;
+    if (!s->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called before solve()");
+    if (nf < 0) return fail(WLSQM_E_VALUE, "nf must be >= 0, got %lld", (long long)nf);
+    if (s->ngather > 0) return fail(WLSQM_E_VALUE, "the field solves do not support the fused result gather (wlsqm_solver_set_gather)");
+    const long long n = s->ncases;
+    if (nf == 0 || n == 0) return WLSQM_OK;
+    if (hoods && !s->hoods_dev.p) return fail(WLSQM_E_NOTREADY, "solve_hoods_fields() needs the neighbour lists of prepare_hoods()");
+    if ((hoods ? !hf : !fk) || !fi) return fail(WLSQM_E_VALUE, "fk (f) and fi must not be NULL");
+    const int maxno = s->maxno, maxnk = s->maxnk;
+    // the (field, case, slot) -> element map of fi must be injective: fields-outer or fields-inner rows
+    const bool fi_outer = (nf == 1 || fi_sf >= (n - 1) * fi_s0 + maxno) && (n == 1 || fi_s0 >= maxno);
+    const bool fi_inner = (nf == 1 || fi_sf >= maxno) && (n == 1 || fi_s0 >= (nf - 1) * fi_sf + maxno);
+    if (fi_sf < 0 || fi_s0 < 0 || !(fi_outer || fi_inner))
+        return fail(WLSQM_E_VALUE, "fi layout (field stride %lld, row stride %lld) maps two (field, case, slot) entries to one "
+                    "element; use fields-outer (fi_sf >= (ncases-1)*fi_s0 + max no) or fields-inner (fi_sf >= max no, "
+                    "fi_s0 >= (nf-1)*fi_sf + max no) rows", (long long)fi_sf, (long long)fi_s0);
+    int rc = use_device(s);
+    if (rc) return rc;
+    cudaStream_t st = s->stream;
+    const bool iter = s->algorithm == WLSQM_ALGO_ITERATIVE;
+    const bool fk_dev = hoods ? true : is_device_ptr(fk) != 0, fi_dev = is_device_ptr(fi) != 0;
+    if (!hoods && fk_dev && fi_dev) {
+        // address span [lo, hi] of each strided array (element offsets)
+        auto span = [](long long a, long long sa, long long b, long long sb, long long c, long long sc, long long& lo, long long& hi) {
+            lo = hi = 0;
+            for (long long t : {(a - 1) * sa, (b - 1) * sb, (c - 1) * sc}) (t < 0 ? lo : hi) += t;
+        };
+        long long klo, khi, ilo, ihi;
+        span(nf, fk_sf, n, fk_s0, maxnk, fk_s1, klo, khi);
+        span(nf, fi_sf, n, fi_s0, maxno, 1, ilo, ihi);
+        if (ranges_overlap(fk + klo, (khi - klo + 1) * 8, fi + ilo, (ihi - ilo + 1) * 8))
+            return fail(WLSQM_E_VALUE, "device fk overlaps device fi: the field solves write fi while other fields still read fk");
+    }
+
+    // ---- host arrays: staged whole (one dense device mirror per argument) -----------------------------------------------
+    if (!hoods && !fk_dev) {
+        if (fk_s1 != 1 && maxnk > 1) return fail(WLSQM_E_VALUE, "host fk must have unit stride on its last axis");
+        rc = s->st_fk.reserve((size_t)nf * n * maxnk * 8);
+        if (rc) return rc;
+        for (long long j = 0; j < nf; ++j) {
+            rc = to_dense((double*)s->st_fk.p + j * n * maxnk, fk + j * fk_sf, n, maxnk, fk_s0, st);
+            if (rc) return rc;
+        }
+        fk = (const double*)s->st_fk.p; fk_sf = n * maxnk; fk_s0 = maxnk; fk_s1 = 1;
+    }
+    if (hoods && !is_device_ptr(hf)) {
+        const long long np = s->hood_points;
+        rc = s->hood_f.reserve((size_t)nf * np * 8);
+        if (rc) return rc;
+        for (long long j = 0; j < nf; ++j) {
+            rc = to_dense((double*)s->hood_f.p + j * np, hf + j * f_sf, np, 1, f_s0, st);
+            if (rc) return rc;
+        }
+        hf = (const double*)s->hood_f.p; f_sf = np; f_s0 = 1;
+    }
+    double* fi_use = fi;
+    long long fi_sf_use = fi_sf, fi_s0_use = fi_s0;
+    if (!fi_dev) {
+        rc = s->st_fi.reserve((size_t)nf * n * maxno * 8);
+        if (rc) return rc;
+        for (long long j = 0; j < nf; ++j) {
+            rc = to_dense((double*)s->st_fi.p + j * n * maxno, fi + j * fi_sf, n, maxno, fi_s0, st);
+            if (rc) return rc;
+        }
+        fi_use = (double*)s->st_fi.p; fi_sf_use = n * maxno; fi_s0_use = maxno;
+    }
+
+    FieldsParams F{};
+    SolveParams& P = F.P;
+    P.meta = s->dmeta; P.uni = s->uni; P.op_stride = s->op_stride; P.ncases = n; P.op = s->op;
+    P.geom_uniform = s->geom_uniform ? 1 : 0;
+    P.algorithm = s->algorithm; P.max_iter = s->max_iter;
+    P.xi = s->xi_dev; P.xi_s0 = s->dim;
+    P.xk = (const double*)s->xk_keep.p; P.xk_s0 = (long long)maxnk * s->dim; P.xk_s1 = s->dim;
+    if (iter) {
+        CU(cudaMemsetAsync(s->iters_dev, 0, ((size_t)n + 1) * 4, st));   // per-case counts: maxima over the passes
+        P.iters_max = s->iters_dev;
+        P.iters_case = s->iters_dev + 1;
+    }
+    // gathered hood data: (fields of a pass, ncases, kp) with an EVEN row pitch kp, so that every row qualifies for bulk copies
+    const long long kp = ((long long)maxnk + 1) & ~1ll;
+    auto set_fk = [&](long long p0) {
+        if (hoods) { P.fk = (const double*)s->hood_fk.p; P.fk_s0 = kp; P.fk_s1 = 1; F.fk_sf = n * kp; }
+        else { P.fk = fk + p0 * fk_sf; P.fk_s0 = fk_s0; P.fk_s1 = fk_s1; F.fk_sf = fk_sf; }
+    };
+    const bool pack = pack_eligible(s);
+    LaunchCfg L;
+    // fields per pass: what one launch shape holds, spread evenly over the passes
+    set_fk(0);
+    F.nf = (int)std::min<int64_t>(nf, 1 << 20);
+    rc = config_solve_fields(s, F, L, n, pack);
+    if (rc) return rc;
+    const long long passes = (nf + F.nf - 1) / F.nf, per_pass = (nf + passes - 1) / passes;
+    if (hoods) {
+        rc = s->hood_fk.reserve((size_t)per_pass * n * kp * 8);
+        if (rc) return rc;
+    }
+    for (long long p0 = 0; p0 < nf; p0 += per_pass) {
+        const int nfp = (int)std::min(per_pass, nf - p0);
+        if (hoods) {
+            const long long total = n * kp;
+            gather_hoods_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)s->sm_count * 32), 256, 0, st>>>(
+                hf + p0 * f_sf, f_s0, 1, (const int32_t*)s->hoods_dev.p, maxnk, n, (int)kp, (double*)s->hood_fk.p,
+                s->hood_points, s->dmeta, s->uni.nk, nullptr, nfp, f_sf, n * kp);
+            CU(cudaGetLastError());
+        }
+        set_fk(p0);
+        F.fi = fi_use + p0 * fi_sf_use; F.fi_sf = fi_sf_use; F.fi_s0 = fi_s0_use;
+        P.case_lo = 0; P.ncases = n;
+        F.nf = nfp;
+        rc = config_solve_fields(s, F, L, n, pack);
+        if (rc) return rc;
+        if (F.nf != nfp) return fail(WLSQM_E_VALUE, "internal: %d fields per pass do not fit the launch shape", nfp);
+        if (pack) {
+            CU(launch_solve_pack_fields(F, L.blocks, L.threads, L.smem, st));
+            continue;
+        }
+        // the last case's fk rows with an odd element count: plain loads, as in wlsqm_solver_solve (every field's row
+        // of that case may end its array)
+        if (P.f_tma && s->last_nk_odd) {
+            if (n > 1) {
+                P.ncases = n - 1;
+                rc = config_solve_fields(s, F, L, n - 1, false);
+                if (rc) return rc;
+                CU(launch_solve_fields(s->dim, F, L.blocks, L.threads, L.smem, st));
+            }
+            P.case_lo = n - 1;
+            P.ncases = n;
+            rc = config_solve_fields(s, F, L, 1, false);
+            if (rc) return rc;
+            P.f_tma = 0;
+        }
+        CU(launch_solve_fields(s->dim, F, L.blocks, L.threads, L.smem, st));
+    }
+    // the solver's own solution copy is not written: interpolate / get_fi refuse until the next solve()
+    s->fi_case_valid = false;
+    if (!fi_dev) {
+        for (long long j = 0; j < nf; ++j) {
+            rc = from_dense(fi + j * fi_sf, fi_s0, (const double*)s->st_fi.p + j * n * maxno, maxno, n, maxno, st);
+            if (rc) return rc;
+        }
+    }
+    int32_t it = 0;
+    if (iter) CU(cudaMemcpyAsync(&it, s->iters_dev, 4, cudaMemcpyDeviceToHost, st));
+    if (iter || !fi_dev || !fk_dev) CU(cudaStreamSynchronize(st));
+    if (iters_out) *iters_out = it;
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_solve_fields(wlsqm_solver_t* s, int64_t nf, const double* fk, int64_t fk_sf, int64_t fk_s0, int64_t fk_s1,
+                              double* fi, int64_t fi_sf, int64_t fi_s0, int32_t* iters_out) {
+    return solve_fields_core(s, nf, false, fk, fk_sf, fk_s0, fk_s1, nullptr, 0, 0, fi, fi_sf, fi_s0, iters_out);
+}
+
+int wlsqm_solver_solve_hoods_fields(wlsqm_solver_t* s, int64_t nf, const double* f, int64_t f_sf, int64_t f_s0, double* fi,
+                                    int64_t fi_sf, int64_t fi_s0, int32_t* iters_out) {
+    return solve_fields_core(s, nf, true, nullptr, 0, 0, 0, f, f_sf, f_s0, fi, fi_sf, fi_s0, iters_out);
 }
 
 // ---- export of the prepared operators (wlsqm_operator.cu) -------------------------------------------------------

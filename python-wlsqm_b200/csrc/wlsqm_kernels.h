@@ -82,6 +82,21 @@ struct SolveParams {
     int gather_full;                                 // rows are whole 128 B lines (gather_s0 a multiple of 16, <= 32): the padding is stored too
 };
 
+// Field-batched solve (wlsqm_solve.cu): the nf fields of a pass share each streamed operator block.  Field f reads its
+// data at P.fk + f * fk_sf (strides P.fk_s0 / P.fk_s1) and its known values from fi + f * fi_sf (row stride fi_s0), and
+// writes its unknown slots there.  A stage of P's ring is [operator | fext of field 0 | ... | fext of field nf-1 | xk]:
+// the fext slots are f_doubles apart from P.off_f on, xk is at P.off_xk (packed variant: [CPW operator blocks | CPW fk
+// rows of each field, f_doubles apart | CPW x nkn known values of each field, k_doubles apart from P.off_xk]).
+// P.fi_in / fi_out / fi_case / sens / gather are not used; P.iters_case[c] is raised to the maximum over the fields.
+constexpr int SOLVE_FIELDS_THREADS = 512;     // field kernels: 128 registers hold the accumulators of 8 fields
+constexpr int SOLVE_FIELDS_BLOCK = 8;         // fields fed by one shared-memory read of an operator element
+struct FieldsParams {
+    SolveParams P;
+    int nf, f_doubles, k_doubles;
+    long long fk_sf;
+    double* fi; long long fi_s0, fi_sf;
+};
+
 // operator export (wlsqm_operator.cu): contraction of the operator blocks with coefficient rows, CSR assembly
 struct StencilParams {
     const CaseMeta* meta;
@@ -198,6 +213,8 @@ cudaError_t launch_prepare_reg(int dim, int maxorder, const PrepRegParams& P, in
                                cudaStream_t st);
 cudaError_t launch_solve(int dim, const SolveParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
 cudaError_t launch_solve_pack(const SolveParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
+cudaError_t launch_solve_fields(int dim, const FieldsParams& F, int blocks, int threads, size_t smem, cudaStream_t st);
+cudaError_t launch_solve_pack_fields(const FieldsParams& F, int blocks, int threads, size_t smem, cudaStream_t st);
 cudaError_t launch_scatter_fi(const CaseMeta* meta, const CaseMeta& uni, long long ncases, const double* fi_case,
                               int fi_case_ld, double* fi_out, long long fi_out_s0, cudaStream_t st);
 cudaError_t launch_interpolate(const InterpParams& P, cudaStream_t st);

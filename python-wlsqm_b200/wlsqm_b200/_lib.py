@@ -63,6 +63,8 @@ SIGNATURES = {
     "wlsqm_gather_hoods": (_int, [_vp, _i64, _int, _i64, _vp, _i64, _i64, _int, _vp, _int, _vp]),
     "wlsqm_solver_prepare_hoods": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _i64]),
     "wlsqm_solver_solve_hoods": (_int, [_vp, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32p]),
+    "wlsqm_solver_solve_fields": (_int, [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _i64, _i64, _i32p]),
+    "wlsqm_solver_solve_hoods_fields": (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _i64, _i64, _i32p]),
     "wlsqm_solver_stencils": (_int, [_vp, _int, _vp, _vp, _vp]),
     "wlsqm_solver_operator_nnz": (_int, [_vp, _i64, _vp]),
     "wlsqm_solver_operator_csr": (_int, [_vp, _int, _vp, _i64, _int, _vp, _vp, _vp, _vp]),

@@ -25,6 +25,7 @@ from libc.stdint cimport int32_t, int64_t, uintptr_t
 from .fitter import defs
 from . import _lib
 from .fitter import opexport as _opexport
+from .fitter import fields as _fields
 
 cdef extern from "wlsqm_b200.h" nogil:
     ctypedef struct wlsqm_solver_t:
@@ -700,6 +701,21 @@ class ExpertSolver:
             rc = wlsqm_solver_solve(h, afk.p, afk.s0, afk.s1, afi.p, afi.s0, sens_p, sn0, sn1, &it)
         _check(rc)
         return it
+
+    def solve_fields(self, fk, fi):
+        """Fit nf fields on the prepared geometry in one pass over the stored operators (extension).
+
+        fk (nf, >= ncases, >= max nk); fi (nf, >= ncases, >= max no) in/out, fields-outer or fields-inner rows (e.g.
+        ``fi_all.transpose(1, 0, 2)`` of an (ncases, nf, no) array).  Field j's unknown slots are bit for bit what
+        ``solve(fk[j], fi[j])`` writes; returns the maximum of those solves' return values, and iterations() gives the
+        per-case maximum.  The solver's own solution copy is not written (interpolate() raises until the next solve());
+        sens is not produced.  See wlsqm_b200.fitter.fields."""
+        return _fields.solve_fields(self, fk, fi)
+
+    def solve_hoods_fields(self, f, fi):
+        """solve_fields with the data per point (extension; needs prepare_hoods): f (nf, >= npoints), any strides --
+        ``f_all.T`` of an (npoints, nf) array is fine.  Field j equals ``solve_hoods(f[j], fi[j])`` bit for bit."""
+        return _fields.solve_hoods_fields(self, f, fi)
 
     def iterations(self):
         """Per-case refinement iteration counts of the last solve (extension; zeros for ALGO_BASIC)."""

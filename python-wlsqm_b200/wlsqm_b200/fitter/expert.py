@@ -19,7 +19,7 @@ import ctypes as C
 
 import numpy as np
 
-from . import defs, opexport
+from . import defs, fields, opexport
 from .. import _lib
 
 __all__ = ["number_of_dofs", "ExpertSolver"]
@@ -333,6 +333,21 @@ class ExpertSolver:
         _lib.check(_lib.lib().wlsqm_solver_solve(self._handle, fk_a.ptr, fk_a.strides[0], fk_a.strides[1],
                                                  fi_a.ptr, fi_a.strides[0], sens_p, s0, s1, C.byref(it)))
         return int(it.value)
+
+    def solve_fields(self, fk, fi):
+        """Fit nf fields on the prepared geometry in one pass over the stored operators (extension).
+
+        fk (nf, >= ncases, >= max nk); fi (nf, >= ncases, >= max no) in/out, fields-outer or fields-inner rows (e.g.
+        ``fi_all.transpose(1, 0, 2)`` of an (ncases, nf, no) array).  Field j's unknown slots are bit for bit what
+        ``solve(fk[j], fi[j])`` writes; returns the maximum of those solves' return values, and iterations() gives the
+        per-case maximum.  The solver's own solution copy is not written (interpolate() raises until the next solve());
+        sens is not produced.  See wlsqm_b200.fitter.fields."""
+        return fields.solve_fields(self, fk, fi)
+
+    def solve_hoods_fields(self, f, fi):
+        """solve_fields with the data per point (extension; needs prepare_hoods): f (nf, >= npoints), any strides --
+        ``f_all.T`` of an (npoints, nf) array is fine.  Field j equals ``solve_hoods(f[j], fi[j])`` bit for bit."""
+        return fields.solve_hoods_fields(self, f, fi)
 
     def iterations(self):
         """Per-case refinement iteration counts of the last solve (extension; zeros for ALGO_BASIC)."""

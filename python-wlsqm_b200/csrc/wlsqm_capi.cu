@@ -259,8 +259,70 @@ int use_device(const wlsqm_solver* s) {
     return WLSQM_OK;
 }
 
+// dst[f][i][0..k*w) = the first nk_i neighbours of case i in the solver's neighbour lists (prepare_hoods), w values each,
+// from src[f] (points of the last prepare_hoods), for the nf fields f; on the solver's stream
+cudaError_t gather_hoods(const wlsqm_solver* s, const double* src, long long src_s0, int w, int k, double* dst, int* err,
+                         int nf = 1, long long src_sf = 0, long long dst_sf = 0) {
+    const long long total = s->ncases * k * w;
+    gather_hoods_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)s->sm_count * 32), 256, 0, s->stream>>>(
+        src, src_s0, w, (const int32_t*)s->hoods_dev.p, s->maxnk, s->ncases, k, dst, s->hood_points, s->dmeta, s->uni.nk, err,
+        nf, src_sf, dst_sf);
+    return cudaGetLastError();
+}
+
+// the fields of a solve launch that come from the solver: records, operators, algorithm, the geometry the refinement
+// reads, and (ALGO_ITERATIVE) its iteration counters, which the caller clears
+void solve_params(const wlsqm_solver* s, SolveParams& P) {
+    P.meta = s->dmeta; P.uni = s->uni; P.op_stride = s->op_stride; P.ncases = s->ncases; P.op = s->op;
+    P.geom_uniform = s->geom_uniform ? 1 : 0;
+    P.algorithm = s->algorithm; P.max_iter = s->max_iter;
+    P.xi = s->xi_dev; P.xi_s0 = s->dim;
+    P.xk = (const double*)s->xk_keep.p; P.xk_s0 = (long long)s->maxnk * s->dim; P.xk_s1 = s->dim;
+    if (s->algorithm == WLSQM_ALGO_ITERATIVE) {
+        P.iters_max = s->iters_dev;
+        P.iters_case = s->iters_dev + 1;
+    }
+}
+
+// One solve launch over the cases [P.case_lo, P.ncases): config(rows) sets the launch shape for `rows` cases, launch()
+// starts the kernel.  Rows of fk with an odd element count are fetched by bulk copies of one element more (inside the
+// even row pitch, wlsqm_solve.cu), but the storage of a caller's strided device array may end with the last element of
+// its last row: with `odd_last` (the launch ends with the last case, whose nk is odd) and bulk copies of fk, that one
+// case runs in a launch of its own with plain loads.
+template <class Config, class Launch>
+int launch_solve_split(SolveParams& P, bool odd_last, Config config, Launch launch) {
+    const long long c0 = P.case_lo, c1 = P.ncases;
+    int rc = config(c1 - c0);
+    if (rc) return rc;
+    if (odd_last && P.f_tma) {
+        if (c1 - c0 > 1) {
+            P.ncases = c1 - 1;
+            rc = config(c1 - c0 - 1);
+            if (rc) return rc;
+            CU(launch());
+        }
+        P.case_lo = c1 - 1;
+        P.ncases = c1;
+        rc = config(1);
+        if (rc) return rc;
+        P.f_tma = 0;
+    }
+    CU(launch());
+    return WLSQM_OK;
+}
+
 // ---- launch configuration ------------------------------------------------------------------------
 struct LaunchCfg { int blocks, threads; size_t smem; };
+
+// Grid of a kernel whose CTAs of `warps` warps and `smem` bytes each take units in turn: as many CTAs per SM as shared
+// memory holds (1 KB of it reserved per CTA), at most max_warps_sm / warps of them (at least one), and no more CTAs
+// than the units fill.
+int grid_blocks(const wlsqm_solver* s, size_t smem, int warps, int max_warps_sm, long long units) {
+    int ctas = (int)(SMEM_PER_SM / (smem + 1024));
+    ctas = std::max(1, std::min(ctas, std::max(1, max_warps_sm / warps)));
+    const long long need = (units + warps - 1) / warps;
+    return (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+}
 
 int config_prepare(const wlsqm_solver* s, PrepareParams& P, LaunchCfg& L) {
     const int nk = std::max(s->maxnk, 1), no = s->maxno, nr = std::max(s->maxnr, 1), nq = std::max(s->maxnq, 1);
@@ -281,10 +343,7 @@ int config_prepare(const wlsqm_solver* s, PrepareParams& P, LaunchCfg& L) {
     while (warps > 1 && warps * per_warp > SMEM_PER_CTA) --warps;
     L.threads = warps * 32;
     L.smem = warps * per_warp;
-    int ctas = (int)(SMEM_PER_SM / (L.smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, 48 / warps)));
-    long long need = (s->ncases + warps - 1) / warps;
-    L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    L.blocks = grid_blocks(s, L.smem, warps, 48, s->ncases);
     return WLSQM_OK;
 }
 
@@ -411,10 +470,9 @@ int config_solve(const wlsqm_solver* s, SolveParams& P, LaunchCfg& L, long long 
     P.bar_off_bytes = warps * wd * 8;
     L.threads = warps * 32;
     L.smem = (size_t)P.bar_off_bytes + (size_t)warps * S * 8;
-    int ctas = (int)(SMEM_PER_SM / (L.smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, env_int("WLSQM_SOLVE_MAXWARPS_SM", iter_small ? 24 : ((stage_bytes >= 3072 && !small_mean) ? 16 : 32)) / warps)));
-    long long need = (ncases_launch + warps - 1) / warps;
-    L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    L.blocks = grid_blocks(s, L.smem, warps,
+                           env_int("WLSQM_SOLVE_MAXWARPS_SM", iter_small ? 24 : ((stage_bytes >= 3072 && !small_mean) ? 16 : 32)),
+                           ncases_launch);
     return WLSQM_OK;
 }
 
@@ -458,11 +516,7 @@ int config_solve_pack(const wlsqm_solver* s, SolveParams& P, LaunchCfg& L, long 
     P.bar_off_bytes = warps * wd * 8;
     L.threads = warps * 32;
     L.smem = (size_t)P.bar_off_bytes + (size_t)warps * S * 8;
-    int ctas = (int)(SMEM_PER_SM / (L.smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, env_int("WLSQM_SOLVE_MAXWARPS_SM", 32) / warps)));
-    const long long packs = (ncases_launch + cpw - 1) / cpw;
-    long long need = (packs + warps - 1) / warps;
-    L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    L.blocks = grid_blocks(s, L.smem, warps, env_int("WLSQM_SOLVE_MAXWARPS_SM", 32), (ncases_launch + cpw - 1) / cpw);
     return WLSQM_OK;
 }
 
@@ -496,11 +550,8 @@ int config_solve_fields(const wlsqm_solver* s, FieldsParams& F, LaunchCfg& L, lo
     P.bar_off_bytes = warps * P.warp_doubles * 8;
     L.threads = warps * 32;
     L.smem = (size_t)P.bar_off_bytes + (size_t)warps * S * 8;
-    int ctas = (int)(SMEM_PER_SM / (L.smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, 16 / warps)));
     const long long units = pack ? (ncases_launch + (32 >> P.pack_lw) - 1) / (32 >> P.pack_lw) : ncases_launch;
-    const long long need = (units + warps - 1) / warps;
-    L.blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    L.blocks = grid_blocks(s, L.smem, warps, 16, units);
     return WLSQM_OK;
 }
 
@@ -1051,17 +1102,9 @@ int wlsqm_solver_solve(wlsqm_solver_t* s, const double* fk, int64_t fk_s0, int64
     cudaStream_t st = s->stream;
 
     SolveParams P{};
-    P.meta = s->dmeta; P.uni = s->uni; P.op_stride = s->op_stride; P.ncases = n; P.op = s->op;
-    P.geom_uniform = s->geom_uniform ? 1 : 0;
-    P.algorithm = s->algorithm; P.max_iter = s->max_iter;
+    solve_params(s, P);
+    if (iter) CU(cudaMemsetAsync(s->iters_dev, 0, 4, st));
     P.fi_case = s->fi_case; P.fi_case_ld = s->maxno;
-    P.xi = s->xi_dev; P.xi_s0 = s->dim;
-    P.xk = (const double*)s->xk_keep.p; P.xk_s0 = (long long)s->maxnk * s->dim; P.xk_s1 = s->dim;
-    if (iter) {
-        CU(cudaMemsetAsync(s->iters_dev, 0, 4, st));
-        P.iters_max = s->iters_dev;
-        P.iters_case = s->iters_dev + 1;
-    }
     P.ngather = s->ngather;
     for (int p = 0; p < s->ngather; ++p) P.gather[p] = s->gather[p];
     P.gather_row0 = s->gather_row0; P.gather_s0 = s->gather_s0;
@@ -1216,30 +1259,13 @@ int wlsqm_solver_solve(wlsqm_solver_t* s, const double* fk, int64_t fk_s0, int64
         P.case_lo = c0;
         P.ncases = c1;
         if (pack_eligible(s)) {
-            rc = config_solve_pack(s, P, L, rows);
-            if (rc) return rc;
-            CU(launch_solve_pack(P, L.blocks, L.threads, L.smem, st));
+            rc = launch_solve_split(P, false, [&](long long r) { return config_solve_pack(s, P, L, r); },
+                                    [&] { return launch_solve_pack(P, L.blocks, L.threads, L.smem, st); });
         } else {
-            rc = config_solve(s, P, L, rows);
-            if (rc) return rc;
-            // Rows of fk with an odd element count are fetched by bulk copies of one element more (inside the even row
-            // pitch, wlsqm_solve.cu).  The storage of a CALLER's strided device array may end with the last element of
-            // its last row: that one case runs in a launch of its own with plain loads.
-            if (fk_dev && P.f_tma && s->last_nk_odd && c1 == n) {
-                if (rows > 1) {
-                    P.ncases = c1 - 1;
-                    rc = config_solve(s, P, L, rows - 1);
-                    if (rc) return rc;
-                    CU(launch_solve(s->dim, P, L.blocks, L.threads, L.smem, st));
-                }
-                P.case_lo = c1 - 1;
-                P.ncases = c1;
-                rc = config_solve(s, P, L, 1);
-                if (rc) return rc;
-                P.f_tma = 0;
-            }
-            CU(launch_solve(s->dim, P, L.blocks, L.threads, L.smem, st));
+            rc = launch_solve_split(P, fk_dev && s->last_nk_odd && c1 == n, [&](long long r) { return config_solve(s, P, L, r); },
+                                    [&] { return launch_solve(s->dim, P, L.blocks, L.threads, L.smem, st); });
         }
+        if (rc) return rc;
         if (sens_drain) {
             // the previous chunk goes to the host while this one is being computed (its copies were queued on s_out
             // before s_out is told to wait for this chunk's kernel)
@@ -1447,15 +1473,11 @@ int wlsqm_solver_prepare_hoods(wlsqm_solver_t* s, const double* x, int64_t x_s0,
     s->hood_points = npoints;
     rc = s->st_xk.reserve((size_t)n * s->maxnk * dim * 8);
     if (rc) return rc;
-    const long long total = n * s->maxnk * dim;
     if (!s->hood_err) {
         if (dev_alloc((void**)&s->hood_err, 4) != cudaSuccess) { cudaGetLastError(); return fail(WLSQM_E_MEMORY, "device allocation failed"); }
     }
     CU(cudaMemsetAsync(s->hood_err, 0, 4, st));
-    gather_hoods_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)s->sm_count * 32), 256, 0, st>>>(
-        xd, xs0, dim, (const int32_t*)s->hoods_dev.p, s->maxnk, n, s->maxnk, (double*)s->st_xk.p, npoints, s->dmeta,
-        s->uni.nk, s->hood_err);
-    CU(cudaGetLastError());
+    CU(gather_hoods(s, xd, xs0, dim, s->maxnk, (double*)s->st_xk.p, s->hood_err));
     const double* xi_use = xi ? xi : xd;
     const long long xi_use_s0 = xi ? xi_s0 : xs0;
     rc = wlsqm_solver_prepare(s, xi_use, xi_use_s0, (const double*)s->st_xk.p, (long long)s->maxnk * dim, dim);
@@ -1502,12 +1524,8 @@ int wlsqm_solver_solve_hoods(wlsqm_solver_t* s, const double* f, int64_t f_s0, d
     const long long kp = ((long long)s->maxnk + 1) & ~1ll;
     rc = s->hood_fk.reserve((size_t)n * kp * 8);
     if (rc) return rc;
-    const long long total = n * kp;
     // (the indices were validated against [0, hood_points) by prepare_hoods; padding slots are not read)
-    gather_hoods_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)s->sm_count * 32), 256, 0, st>>>(
-        fd, fs0, 1, (const int32_t*)s->hoods_dev.p, s->maxnk, n, (int)kp, (double*)s->hood_fk.p, s->hood_points, s->dmeta,
-        s->uni.nk, nullptr);
-    CU(cudaGetLastError());
+    CU(gather_hoods(s, fd, fs0, 1, (int)kp, (double*)s->hood_fk.p, nullptr));
     return wlsqm_solver_solve(s, (const double*)s->hood_fk.p, kp, 1, fi, fi_s0, sens, sens_s0, sens_s1, iters_out);
 }
 
@@ -1586,16 +1604,8 @@ static int solve_fields_core(wlsqm_solver_t* s, int64_t nf, bool hoods, const do
 
     FieldsParams F{};
     SolveParams& P = F.P;
-    P.meta = s->dmeta; P.uni = s->uni; P.op_stride = s->op_stride; P.ncases = n; P.op = s->op;
-    P.geom_uniform = s->geom_uniform ? 1 : 0;
-    P.algorithm = s->algorithm; P.max_iter = s->max_iter;
-    P.xi = s->xi_dev; P.xi_s0 = s->dim;
-    P.xk = (const double*)s->xk_keep.p; P.xk_s0 = (long long)maxnk * s->dim; P.xk_s1 = s->dim;
-    if (iter) {
-        CU(cudaMemsetAsync(s->iters_dev, 0, ((size_t)n + 1) * 4, st));   // per-case counts: maxima over the passes
-        P.iters_max = s->iters_dev;
-        P.iters_case = s->iters_dev + 1;
-    }
+    solve_params(s, P);
+    if (iter) CU(cudaMemsetAsync(s->iters_dev, 0, ((size_t)n + 1) * 4, st));   // per-case counts: maxima over the passes
     // gathered hood data: (fields of a pass, ncases, kp) with an EVEN row pitch kp, so that every row qualifies for bulk copies
     const long long kp = ((long long)maxnk + 1) & ~1ll;
     auto set_fk = [&](long long p0) {
@@ -1616,40 +1626,20 @@ static int solve_fields_core(wlsqm_solver_t* s, int64_t nf, bool hoods, const do
     }
     for (long long p0 = 0; p0 < nf; p0 += per_pass) {
         const int nfp = (int)std::min(per_pass, nf - p0);
-        if (hoods) {
-            const long long total = n * kp;
-            gather_hoods_kernel<<<(unsigned)std::min<long long>((total + 255) / 256, (long long)s->sm_count * 32), 256, 0, st>>>(
-                hf + p0 * f_sf, f_s0, 1, (const int32_t*)s->hoods_dev.p, maxnk, n, (int)kp, (double*)s->hood_fk.p,
-                s->hood_points, s->dmeta, s->uni.nk, nullptr, nfp, f_sf, n * kp);
-            CU(cudaGetLastError());
-        }
+        if (hoods) CU(gather_hoods(s, hf + p0 * f_sf, f_s0, 1, (int)kp, (double*)s->hood_fk.p, nullptr, nfp, f_sf, n * kp));
         set_fk(p0);
         F.fi = fi_use + p0 * fi_sf_use; F.fi_sf = fi_sf_use; F.fi_s0 = fi_s0_use;
         P.case_lo = 0; P.ncases = n;
         F.nf = nfp;
-        rc = config_solve_fields(s, F, L, n, pack);
+        auto config = [&](long long rows) {
+            const int r = config_solve_fields(s, F, L, rows, pack);
+            if (!r && F.nf != nfp) return fail(WLSQM_E_VALUE, "internal: %d fields per pass do not fit the launch shape", nfp);
+            return r;
+        };
+        // (every field's row of the last case may end its array)
+        if (pack) rc = launch_solve_split(P, false, config, [&] { return launch_solve_pack_fields(F, L.blocks, L.threads, L.smem, st); });
+        else rc = launch_solve_split(P, s->last_nk_odd, config, [&] { return launch_solve_fields(s->dim, F, L.blocks, L.threads, L.smem, st); });
         if (rc) return rc;
-        if (F.nf != nfp) return fail(WLSQM_E_VALUE, "internal: %d fields per pass do not fit the launch shape", nfp);
-        if (pack) {
-            CU(launch_solve_pack_fields(F, L.blocks, L.threads, L.smem, st));
-            continue;
-        }
-        // the last case's fk rows with an odd element count: plain loads, as in wlsqm_solver_solve (every field's row
-        // of that case may end its array)
-        if (P.f_tma && s->last_nk_odd) {
-            if (n > 1) {
-                P.ncases = n - 1;
-                rc = config_solve_fields(s, F, L, n - 1, false);
-                if (rc) return rc;
-                CU(launch_solve_fields(s->dim, F, L.blocks, L.threads, L.smem, st));
-            }
-            P.case_lo = n - 1;
-            P.ncases = n;
-            rc = config_solve_fields(s, F, L, 1, false);
-            if (rc) return rc;
-            P.f_tma = 0;
-        }
-        CU(launch_solve_fields(s->dim, F, L.blocks, L.threads, L.smem, st));
     }
     // the solver's own solution copy is not written: interpolate / get_fi refuse until the next solve()
     s->fi_case_valid = false;
@@ -1727,10 +1717,7 @@ static int opx_stencils(wlsqm_solver_t* s, int nops, const double* coeffs, doubl
     }
     P.stages = S;
     P.bar_off_bytes = P.ring_off * 8 + warps * S * P.stage_doubles * 8;
-    int ctas = (int)(SMEM_PER_SM / (smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, (stage_bytes >= 3072 ? 16 : 32) / warps)));
-    const long long need = (s->ncases + warps - 1) / warps;
-    const int blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    const int blocks = grid_blocks(s, smem, warps, stage_bytes >= 3072 ? 16 : 32, s->ncases);
     CU(launch_stencils(P, blocks, warps * 32, smem, s->stream));
     return WLSQM_OK;
 }
@@ -1953,10 +1940,7 @@ static int opx_interp(wlsqm_solver_t* s, const double* xd, long long xs, const l
     P.stages = S; P.opc = opc; P.cq_doubles = cqd;
     P.cq_off = P.ring_off + warps * S * P.stage_doubles;
     P.bar_off_bytes = (P.cq_off + warps * cqd) * 8;
-    int ctas = (int)(SMEM_PER_SM / (smem + 1024));
-    ctas = std::max(1, std::min(ctas, std::max(1, (stage_bytes >= 3072 ? 16 : 32) / warps)));
-    const long long need = (nx + warps - 1) / warps;      // (there are at most nx runs)
-    const int blocks = (int)std::max<long long>(1, std::min<long long>((long long)s->sm_count * ctas, need));
+    const int blocks = grid_blocks(s, smem, warps, stage_bytes >= 3072 ? 16 : 32, nx);   // (there are at most nx runs)
     CU(launch_interp_stencils(P, blocks, warps * 32, smem, s->stream));
     return WLSQM_OK;
 }

@@ -182,6 +182,57 @@ __device__ __forceinline__ CaseMeta case_meta(const CaseMeta* meta, const CaseMe
 __device__ __forceinline__ uint32_t op_block_bytes(const CaseMeta& m) {
     return ((uint32_t)((m.nk + m.nkn) * (int)m.nr) * 8u + 15u) & ~15u;
 }
+
+// One warp's ring of S shared-memory stages, filled by 1D bulk copies that complete on one mbarrier per stage.  The
+// units [lo, end) are dealt to the warps of the grid in turn; this warp takes first, first + stride, ... (n_my of them).
+// Lane 0 keeps the next S - 1 units in flight while the warp works on the current one.  Per unit i (unit u):
+//   refill(lane, i, u, issue)   lane 0 starts unit u + (S - 1) * stride in the stage that release() freed last (S == 1:
+//                               the current stage, nothing is in flight ahead)
+//   wait()                      before the first read of the stage (cur())
+//   release()                   after the last read: every lane is done with the stage before lane 0 re-arms it
+// issue(stage address, barrier address, unit) is the kernel's: it arms the barrier with the unit's byte count and starts
+// the copies; it is taken by reference (passed by value, it changed solve_pack_fields_kernel<1>'s register allocation and
+// cost it 5 % of its time on a B200).  Every lane must call start() before the loop.
+struct WarpRing {
+    uint32_t base, bars, stage_bytes;
+    int S, stage = 0;
+    uint32_t phase = 0;
+    long long first, stride, n_my;
+
+    __device__ __forceinline__ WarpRing(uint32_t base_, uint32_t bars_, int S_, uint32_t stage_bytes_, long long lo,
+                                        long long end)
+        : base(base_), bars(bars_), stage_bytes(stage_bytes_), S(S_) {
+        const int nwarps = blockDim.x >> 5;
+        first = lo + (long long)blockIdx.x * nwarps + (threadIdx.x >> 5);
+        stride = (long long)gridDim.x * nwarps;
+        n_my = first < end ? (end - first + stride - 1) / stride : 0;
+    }
+    __device__ __forceinline__ uint32_t addr(int s) const { return base + (uint32_t)s * stage_bytes; }
+    __device__ __forceinline__ uint32_t bar(int s) const { return bars + (uint32_t)s * 8u; }
+    __device__ __forceinline__ uint32_t cur() const { return addr(stage); }
+    template <class Issue>
+    __device__ __forceinline__ void start(int lane, const Issue& issue) {
+        if (lane == 0) {
+            for (int s = 0; s < S; ++s) mbar_init_u32(bar(s), 1);
+            fence_mbar_init();
+            for (int s = 0; s < S - 1 && s < n_my; ++s) issue(addr(s), bar(s), first + (long long)s * stride);
+        }
+        __syncwarp();
+    }
+    template <class Issue>
+    __device__ __forceinline__ void refill(int lane, long long i, long long unit, const Issue& issue) {
+        if (lane == 0 && i + S - 1 < n_my) {
+            int sn = stage + S - 1;
+            if (sn >= S) sn -= S;
+            issue(addr(sn), bar(sn), unit + (long long)(S - 1) * stride);
+        }
+    }
+    __device__ __forceinline__ void wait() const { mbar_wait_u32(bar(stage), phase); }
+    __device__ __forceinline__ void release() {
+        __syncwarp();
+        if (++stage == S) { stage = 0; phase ^= 1u; }
+    }
+};
 #endif
 
 struct InterpParams {

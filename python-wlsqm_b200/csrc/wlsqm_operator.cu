@@ -12,8 +12,8 @@
 // CSR row i holds, per distinct neighbour index p, the W[i][k] with hoods[i][k] == p summed in ascending k; with
 // centre folding, the known-F weight K[i][0] is added last to column center + i and reported as 0 in K.
 //
-// stencil_kernel: one warp per case streams its block into a shared-memory ring with the bulk copies of
-// solve_kernel (same CaseMeta addressing, case_meta / op_block_bytes in wlsqm_kernels.h) and produces all nops
+// stencil_kernel: one warp per case streams its block through the shared-memory ring of solve_kernel (WarpRing, same
+// CaseMeta addressing, case_meta / op_block_bytes in wlsqm_kernels.h) and produces all nops
 // operators from that one read; the coefficients live in shared memory.  Bound by the HBM read of the blocks.
 // csr_kernel<false>: distinct columns per row (count); cub exclusive scan; csr_kernel<true>: columns in ascending
 // order, merged values (fill).  A warp per row; the row's used hood indices are staged in shared memory.
@@ -78,63 +78,55 @@ __device__ __forceinline__ void contract_case(const double* op, const CaseMeta& 
     }
 }
 
+// bit s set: coefficient s of the row co (maxno entries) is nonzero (every lane of the warp calls it)
+__device__ __forceinline__ unsigned long long nonzero_slots(const double* co, int maxno, int lane) {
+    const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
+    const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
+    return ((unsigned long long)hi << 32) | lo;
+}
+
+// The CTA's copy of the coefficient rows cs [nops][maxno] and their nonzero slots nzm [nops] (every thread calls it;
+// shared memory the CTA wrote before the call is visible after it)
+__device__ __forceinline__ void stage_coefficients(const double* coef, int nops, int maxno, double* cs, unsigned long long* nzm) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    for (int t = threadIdx.x; t < nops * maxno; t += blockDim.x) cs[t] = coef[t];
+    __syncthreads();
+    for (int o = warp; o < nops; o += nwarps) {
+        const unsigned long long nz = nonzero_slots(cs + o * maxno, maxno, lane);
+        if (lane == 0) nzm[o] = nz;
+    }
+    __syncthreads();
+}
+
 template <bool UNI>
 __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) stencil_kernel(StencilParams P) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
     const int nops = P.nops, maxno = P.maxno;
     double* cs = reinterpret_cast<double*>(smem_raw);                                      // [nops][maxno]
     unsigned long long* nzm = reinterpret_cast<unsigned long long*>(cs + nops * maxno);     // [nops] nonzero slots
-    for (int t = threadIdx.x; t < nops * maxno; t += blockDim.x) cs[t] = P.coef[t];
-    __syncthreads();
-    for (int o = warp; o < nops; o += nwarps) {
-        const double* co = cs + o * maxno;
-        const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
-        const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
-        if (lane == 0) nzm[o] = ((unsigned long long)hi << 32) | lo;
-    }
-    __syncthreads();
+    stage_coefficients(P.coef, nops, maxno, cs, nzm);
 
-    const int S = P.stages;
-    double* ring = reinterpret_cast<double*>(smem_raw) + P.ring_off + (size_t)warp * S * P.stage_doubles;
-    const uint32_t ring_u32 = smem_u32(ring);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
-    const long long gw = (long long)blockIdx.x * nwarps + warp;
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < P.ncases ? (P.ncases - gw + GW - 1) / GW : 0;
-
-    auto issue = [&](int s, long long c) {   // lane 0 only
+    const double* ring = reinterpret_cast<double*>(smem_raw) + P.ring_off + (size_t)warp * P.stages * P.stage_doubles;
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, 0, P.ncases);
+    auto issue = [&](uint32_t st, uint32_t bar, long long c) {   // lane 0 only
         const CaseMeta m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         const uint32_t b = op_block_bytes(m);
         mbar_expect_tx_u32(bar, b);
         if (b) tma_load_1d_u32(st, P.op + m.op_off, b, bar);
     };
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0;
-    uint32_t phase = 0;
-    long long c = gw;
-    for (long long i = 0; i < n_my; ++i, c += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, c + (long long)(S - 1) * GW);
-        }
+    long long c = R.first;
+    for (long long i = 0; i < R.n_my; ++i, c += R.stride) {
+        R.refill(lane, i, c, issue);
         const CaseMeta m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
-        const double* op = ring + (size_t)stage * P.stage_doubles;
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        const double* op = ring + (size_t)R.stage * P.stage_doubles;
+        R.wait();
         contract_case(op, m, cs, nzm, nops, maxno, P.maxnk, P.ncases, c, P.W, P.K, P.kf, lane);
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
     }
 }
 
@@ -180,40 +172,24 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
     const int nops = P.nops, maxno = P.maxno, opc = P.opc, dim = P.dim;
     double* cs = reinterpret_cast<double*>(smem_raw);                                      // [nops][maxno]
     unsigned long long* nzm = reinterpret_cast<unsigned long long*>(cs + nops * maxno);     // [nops] nonzero slots
     unsigned short* ex = reinterpret_cast<unsigned short*>(nzm + nops);                     // [maxno] slot exponents
-    for (int t = threadIdx.x; t < nops * maxno; t += blockDim.x) cs[t] = P.coef[t];
     for (int t = threadIdx.x; t < maxno; t += blockDim.x) ex[t] = c_slot_exp.e[dim - 1][t];
-    __syncthreads();
-    for (int o = warp; o < nops; o += nwarps) {
-        const double* co = cs + o * maxno;
-        const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
-        const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
-        if (lane == 0) nzm[o] = ((unsigned long long)hi << 32) | lo;
-    }
-    __syncthreads();
+    stage_coefficients(P.coef, nops, maxno, cs, nzm);
 
     // the warp's coefficient rows of one query: cq [opc][maxno], their nonzero slots qnz [opc], Taylor terms tt [3][5]
     double* cq = reinterpret_cast<double*>(smem_raw) + P.cq_off + (size_t)warp * P.cq_doubles;
     unsigned long long* qnz = reinterpret_cast<unsigned long long*>(cq + opc * maxno);
     double* tt = reinterpret_cast<double*>(qnz + opc);
 
-    const int S = P.stages;
-    double* ring = reinterpret_cast<double*>(smem_raw) + P.ring_off + (size_t)warp * S * P.stage_doubles;
-    const uint32_t ring_u32 = smem_u32(ring);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
-    const long long nruns = *P.nruns;
-    const long long gw = (long long)blockIdx.x * nwarps + warp;
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < nruns ? (nruns - gw + GW - 1) / GW : 0;
-
-    auto issue = [&](int s, long long r) {   // lane 0 only
+    // units: the runs, whose number the sort left on the device
+    const double* ring = reinterpret_cast<double*>(smem_raw) + P.ring_off + (size_t)warp * P.stages * P.stage_doubles;
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, 0, *P.nruns);
+    auto issue = [&](uint32_t st, uint32_t bar, long long r) {   // lane 0 only
         const long long c = P.run_case[r];
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         uint32_t b = 0;
         CaseMeta m{};
         if (c < P.nmodels) {
@@ -223,26 +199,15 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
         mbar_expect_tx_u32(bar, b);
         if (b) tma_load_1d_u32(st, P.op + m.op_off, b, bar);
     };
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0;
-    uint32_t phase = 0;
-    long long r = gw;
-    for (long long i = 0; i < n_my; ++i, r += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, r + (long long)(S - 1) * GW);
-        }
+    long long r = R.first;
+    for (long long i = 0; i < R.n_my; ++i, r += R.stride) {
+        R.refill(lane, i, r, issue);
         const long long c = P.run_case[r];
         const int q0 = P.run_off[r], nq = P.run_len[r];
-        const double* op = ring + (size_t)stage * P.stage_doubles;
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        const double* op = ring + (size_t)R.stage * P.stage_doubles;
+        R.wait();
         if (c >= P.nmodels) {
             // no model: W row 0, K row NaN (interpolate's NaN for such a query), nothing folded
             for (int t = 0; t < nq; ++t) {
@@ -290,10 +255,8 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
                     }
                     __syncwarp();
                     for (int o = 0; o < oc; ++o) {
-                        const double* co = cq + o * maxno;
-                        const unsigned lo = __ballot_sync(0xffffffffu, lane < maxno && co[lane] != 0.0);
-                        const unsigned hi = __ballot_sync(0xffffffffu, lane + 32 < maxno && co[lane + 32] != 0.0);
-                        if (lane == 0) qnz[o] = ((unsigned long long)hi << 32) | lo;
+                        const unsigned long long nz = nonzero_slots(cq + o * maxno, maxno, lane);
+                        if (lane == 0) qnz[o] = nz;
                     }
                     __syncwarp();
                     contract_case(op, m, cq, qnz, oc, maxno, P.maxnk, P.nx, q, P.W + (long long)o0 * P.nx * P.maxnk,
@@ -303,8 +266,7 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
                 }
             }
         }
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
     }
 }
 

@@ -32,20 +32,14 @@ solve_kernel(SolveParams P) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
-    const int S = P.stages;
     double* wb = reinterpret_cast<double*>(smem_raw) + (size_t)warp * P.warp_doubles;
     double* ring = wb;                      // S stages of [operator block | fext = (fk, known fi) | xk (ITER)]
     double* fis = wb + P.off_fi;            // current solution of the case (no values)
     double* rs = wb + P.off_r;              // ITER: residual at the neighbours
-    const uint32_t ring_u32 = smem_u32(ring);
     const uint32_t rs_u32 = smem_u32(rs);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
-
-    const long long gw = P.case_lo + (long long)blockIdx.x * nwarps + warp;   // first case of this warp
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < P.ncases ? (P.ncases - gw + GW - 1) / GW : 0;
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, P.case_lo, P.ncases);
+    const long long gw = R.first, GW = R.stride, n_my = R.n_my;
 
     auto get_meta = [&](long long c) { return case_meta<UNI>(P.meta, P.uni, P.op_stride, c); };
     // bulk copies need 16 B alignment and sizes: the host says whether the arrays qualify (f_tma, xk_tma: 16 B aligned
@@ -55,9 +49,8 @@ solve_kernel(SolveParams P) {
     // gather instead would put an unprefetched global load on the critical path of every such case.
     auto f_by_tma = [&](const CaseMeta&) { return P.f_tma != 0; };
     auto xk_by_tma = [&](const CaseMeta&) { return ITER && P.xk_tma; };
-    auto issue = [&](int s, long long c) {   // lane 0 only: arm the stage's barrier and start its copies
+    auto issue = [&](uint32_t st, uint32_t bar, long long c) {   // lane 0 only: arm the stage's barrier and start its copies
         const CaseMeta m = get_meta(c);
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         const uint32_t b_op = op_block_bytes(m);
         const uint32_t b_f = f_by_tma(m) ? (((uint32_t)m.nk + 1u) & ~1u) * 8u : 0u;
         const uint32_t b_x = xk_by_tma(m) ? (((uint32_t)(m.nk * DIM) + 1u) & ~1u) * 8u : 0u;
@@ -73,15 +66,9 @@ solve_kernel(SolveParams P) {
         if (lane + 32 < m.no && ((m.knowns >> (lane + 32)) & 1LL)) g1 = P.fi_in[c * P.fi_in_s0 + lane + 32];
     };
 
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0, itmax = 0;
-    uint32_t phase = 0;
+    int itmax = 0;
     double g0 = 0.0, g1 = 0.0;
     CaseMeta mt{};
     if (n_my > 0) {
@@ -90,21 +77,17 @@ solve_kernel(SolveParams P) {
     }
     long long c = gw;
     for (long long i = 0; i < n_my; ++i, c += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, c + (long long)(S - 1) * GW);
-        }
+        R.refill(lane, i, c, issue);
         // per-case records: the one lane 0 needs at the top of the NEXT iteration (to start the copies of the case after
         // next) is requested into L1 now -- fetched cold it held up the whole warp there (17 % of the stall samples of the
         // mixed-size kernel, profiles/r02_solve_kernel_hetero_source_lines.txt)
         // (with a one-stage ring the record in question is the next case's, which every lane fetches below anyway)
-        if (!UNI && S > 1 && lane == 0 && i + S < n_my) asm volatile("prefetch.global.L1 [%0];" ::"l"(P.meta + (c + (long long)S * GW)));
+        if (!UNI && R.S > 1 && lane == 0 && i + R.S < n_my) asm volatile("prefetch.global.L1 [%0];" ::"l"(P.meta + (c + (long long)R.S * GW)));
         const long long knowns = mt.knowns;
         if (UNI) mt = P.uni;   // loop invariant: lets the compiler hoist everything derived from the record
         const int nk = mt.nk, no = mt.no, nr = mt.nr, nkn = mt.nkn, nq = nk + nkn;
-        double* st = ring + (size_t)stage * P.stage_doubles;
-        const uint32_t st_u32 = ring_u32 + (uint32_t)stage * stage_bytes;
+        double* st = ring + (size_t)R.stage * P.stage_doubles;
+        const uint32_t st_u32 = R.cur();
         const double* op = st;
         double* fext = st + P.off_f;
         const double* xks = st + P.off_xk;
@@ -141,7 +124,7 @@ solve_kernel(SolveParams P) {
             if (mt_next.nkn) load_g(c + GW, mt_next, gn0, gn1);
         }
         __syncwarp();
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        R.wait();
         if (nkn && late_knowns) {
             if (in0 && !unk0) fext[nk + below0] = g0;
             if (in1 && !unk1) fext[nk + below1] = g1;
@@ -216,74 +199,9 @@ solve_kernel(SolveParams P) {
         }
 
         // ---- ALGO_ITERATIVE: refinement against the data (impl.pyx:1010-1083) --------------------
-        int it = 0;
         if (ITER) {
-            double xi0 = P.xi[c * P.xi_s0], xi1 = 0.0, xi2 = 0.0;
-            if (DIM >= 2) xi1 = P.xi[c * P.xi_s0 + 1];
-            if (DIM >= 3) xi2 = P.xi[c * P.xi_s0 + 2];
-            double prev = -1.0;
-            bool broke = false;
-            const bool full_model = no == max_no<DIM>();     // (warp-uniform) order 4: no test per coefficient
-            for (it = 0; it < P.max_iter; ++it) {
-                double nrm = 0.0;
-                if (DIM == 3 && nk > 32) {
-                    // more neighbours than lanes: a lane evaluates the model at its two neighbours k and k + 32 together
-                    // (coefficients loaded once, two independent Horner chains).  3D only: the 1D / 2D instantiations run
-                    // 24 warps per SM at 80 registers and have none to spare for the second chain.
-                    for (int k = lane; k < nk; k += 64) {
-                        const int k1 = k + 32;
-                        const bool has1 = k1 < nk;
-                        const int kb = has1 ? k1 : k;
-                        const double dx0 = xks[k * DIM] - xi0, dx1 = xks[kb * DIM] - xi0;
-                        const double dy0 = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                        const double dy1 = DIM >= 2 ? xks[kb * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                        const double dz0 = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                        const double dz1 = DIM >= 3 ? xks[kb * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                        double m0, m1;
-                        if (full_model) eval_taylor_nested2<DIM, true>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
-                        else eval_taylor_nested2<DIM, false>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
-                        const double r0 = fext[k] - m0;
-                        rs[k] = r0;
-                        const double a0 = fabs(r0);
-                        nrm = a0 > nrm ? a0 : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
-                        if (has1) {
-                            const double r1 = fext[k1] - m1;
-                            rs[k1] = r1;
-                            const double a1 = fabs(r1);
-                            nrm = a1 > nrm ? a1 : nrm;
-                        }
-                    }
-                } else {
-                    for (int k = lane; k < nk; k += 32) {
-                        const double dx = xks[k * DIM] - xi0;
-                        const double dy = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                        const double dz = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                        const double r = fext[k] - (full_model ? eval_taylor_nested_full<DIM>(fis, dx, dy, dz)
-                                                               : eval_taylor_nested<DIM>(no, fis, dx, dy, dz));
-                        rs[k] = r;
-                        const double ar = fabs(r);
-                        nrm = ar > nrm ? ar : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
-                    }
-                }
-                nrm = warp_max_nonneg(nrm);
-                if (nrm == prev) { broke = true; break; }
-                prev = nrm;
-                __syncwarp();
-                if (nr > 0) {
-                    double lo, hi;
-                    warp_matvec<ITER>(st_u32, rs_u32, nk, nr, gr, lane, lo, hi);
-                    const double t0 = fetch_reduced(lo, hi, j0);
-                    if (unk0) { v0 += t0; fis[lane] = v0; }
-                    if (no > 32) {
-                        const double t1 = fetch_reduced(lo, hi, j1);
-                        if (unk1) { v1 += t1; fis[lane + 32] = v1; }
-                    }
-                }
-                __syncwarp();
-            }
-            // for/else quirk of impl.pyx:1080-1083: a loop that runs to completion reports max_iter,
-            // except max_iter <= 0, which reports 1.
-            if (!broke) it = P.max_iter > 0 ? P.max_iter : 1;
+            const int it = refine_case<DIM>(P, c, no, nk, nr, gr, lane, fis, xks, fext, rs, rs_u32, st_u32, unk0, unk1, j0, j1,
+                                            v0, v1);
             if (P.iters_case && lane == 0) P.iters_case[c] = it;
             itmax = max(itmax, it);
         }
@@ -311,8 +229,7 @@ solve_kernel(SolveParams P) {
                 if (in1) P.gather[p][g + lane + 32] = v1;
             }
         }
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
         mt = mt_next; g0 = gn0; g1 = gn1;
     }
     if (ITER && lane == 0 && itmax > 0) atomicMax(P.iters_max, itmax);
@@ -330,12 +247,7 @@ __global__ void __launch_bounds__(SOLVE_MAX_THREADS) solve_pack_kernel(SolvePara
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
-    const int S = P.stages;
     double* ring = reinterpret_cast<double*>(smem_raw) + (size_t)warp * P.warp_doubles;
-    const uint32_t ring_u32 = smem_u32(ring);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
 
     const CaseMeta u = P.uni;
     const int nk = u.nk, no = u.no, nr = u.nr, nkn = u.nkn;
@@ -343,17 +255,16 @@ __global__ void __launch_bounds__(SOLVE_MAX_THREADS) solve_pack_kernel(SolvePara
     const int cg = lane >> lw, o = lane & ((1 << lw) - 1);
     const int ops = (int)P.op_stride;                         // doubles per operator block (even)
 
-    const long long npacks = (P.ncases - P.case_lo + CPW - 1) / CPW;
-    const long long gw = (long long)blockIdx.x * nwarps + warp;
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < npacks ? (npacks - gw + GW - 1) / GW : 0;
+    // units are packs, counted from 0: pack pk holds the cases from case_lo + pk * CPW on
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, 0, (P.ncases - P.case_lo + CPW - 1) / CPW);
+    const long long gw = R.first, GW = R.stride, n_my = R.n_my;
 
     auto pack_cases = [&](long long pk) { return (int)min((long long)CPW, P.ncases - (P.case_lo + pk * CPW)); };
     auto f_by_tma = [&](int ncs) { return P.f_tma && !((ncs * nk) & 1); };
-    auto issue = [&](int s, long long pk) {   // lane 0 only
+    auto issue = [&](uint32_t st, uint32_t bar, long long pk) {   // lane 0 only
         const long long c0 = P.case_lo + pk * CPW;
         const int ncs = pack_cases(pk);
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         const uint32_t b_op = (uint32_t)(ncs * ops) * 8u;
         const uint32_t b_f = f_by_tma(ncs) ? (uint32_t)(ncs * nk) * 8u : 0u;
         mbar_expect_tx_u32(bar, b_op + b_f);
@@ -371,30 +282,19 @@ __global__ void __launch_bounds__(SOLVE_MAX_THREADS) solve_pack_kernel(SolvePara
         }
     };
 
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0;
-    uint32_t phase = 0;
     long long knowns = u.knowns;
     double g = 0.0;
     if (n_my > 0 && (nkn || P.meta)) load_slot(gw, knowns, g);
     long long pk = gw;
     for (long long i = 0; i < n_my; ++i, pk += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, pk + (long long)(S - 1) * GW);
-        }
+        R.refill(lane, i, pk, issue);
         const long long c0 = P.case_lo + pk * CPW;
         const int ncs = pack_cases(pk);
         const long long c = c0 + cg;
-        double* st = ring + (size_t)stage * P.stage_doubles;
-        const uint32_t st_u32 = ring_u32 + (uint32_t)stage * stage_bytes;
+        double* st = ring + (size_t)R.stage * P.stage_doubles;
+        const uint32_t st_u32 = R.cur();
         double* fs = st + P.off_f;                 // [CPW][nk]   fk rows of the pack
         double* ks = st + P.off_xk;                // [CPW][nkn]  known values of the pack
         if (!f_by_tma(ncs)) {
@@ -413,7 +313,7 @@ __global__ void __launch_bounds__(SOLVE_MAX_THREADS) solve_pack_kernel(SolvePara
         double g_next = 0.0;
         if (i + 1 < n_my && (nkn || P.meta)) load_slot(pk + GW, kn_next, g_next);
         __syncwarp();
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        R.wait();
 
         // ---- fi[unknown slot] = its operator column . fext ------------------------------------------------
         double v = g;
@@ -470,8 +370,7 @@ __global__ void __launch_bounds__(SOLVE_MAX_THREADS) solve_pack_kernel(SolvePara
                 }
             }
         }
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
         knowns = kn_next;
         g = g_next;
     }

@@ -1,7 +1,9 @@
-// wlsqm_solve_common.cuh -- the warp GEMV of the solve kernels, shared by wlsqm_solve.cu (one field per pass) and
-// wlsqm_solve_fields.cu (several fields per pass, which must reproduce its sums bit for bit).
+// wlsqm_solve_common.cuh -- the warp GEMV and the ALGO_ITERATIVE refinement of the solve kernels, shared by
+// wlsqm_solve.cu (one field per pass) and wlsqm_solve_fields.cu (several fields per pass, which must reproduce its sums
+// bit for bit).
 #pragma once
 #include "wlsqm_common.cuh"
+#include "wlsqm_kernels.h"
 
 namespace wlsqm {
 
@@ -139,6 +141,84 @@ __device__ __forceinline__ double fetch_reduced(double lo, double hi, int j) {
     const double vlo = __shfl_sync(0xffffffffu, lo, j & 31);
     const double vhi = __shfl_sync(0xffffffffu, hi, j & 31);
     return j < 32 ? vlo : vhi;
+}
+
+// ALGO_ITERATIVE refinement of one case against the data (impl.pyx:1010-1083), with the operator block resident at op_s:
+// fis holds the current solution (known slots included), fext the data, rs receives the residuals.  v0 / v1 are this
+// lane's slots lane and lane + 32 (updated in place); returns the reference's iteration count.
+template <int DIM>
+__device__ __forceinline__ int refine_case(const SolveParams& P, long long c, int no, int nk, int nr, const Groups& gr,
+                                           int lane, double* fis, const double* xks, const double* fext, double* rs,
+                                           uint32_t rs_u32, uint32_t op_s, bool unk0, bool unk1, int j0, int j1,
+                                           double& v0, double& v1) {
+    int it;
+    double xi0 = P.xi[c * P.xi_s0], xi1 = 0.0, xi2 = 0.0;
+    if (DIM >= 2) xi1 = P.xi[c * P.xi_s0 + 1];
+    if (DIM >= 3) xi2 = P.xi[c * P.xi_s0 + 2];
+    double prev = -1.0;
+    bool broke = false;
+    const bool full_model = no == max_no<DIM>();     // (warp-uniform) order 4: no test per coefficient
+    for (it = 0; it < P.max_iter; ++it) {
+        double nrm = 0.0;
+        if (DIM == 3 && nk > 32) {
+            // more neighbours than lanes: a lane evaluates the model at its two neighbours k and k + 32 together
+            // (coefficients loaded once, two independent Horner chains).  3D only: the 1D / 2D instantiations run
+            // 24 warps per SM at 80 registers and have none to spare for the second chain.
+            for (int k = lane; k < nk; k += 64) {
+                const int k1 = k + 32;
+                const bool has1 = k1 < nk;
+                const int kb = has1 ? k1 : k;
+                const double dx0 = xks[k * DIM] - xi0, dx1 = xks[kb * DIM] - xi0;
+                const double dy0 = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
+                const double dy1 = DIM >= 2 ? xks[kb * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
+                const double dz0 = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
+                const double dz1 = DIM >= 3 ? xks[kb * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
+                double m0, m1;
+                if (full_model) eval_taylor_nested2<DIM, true>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
+                else eval_taylor_nested2<DIM, false>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
+                const double r0 = fext[k] - m0;
+                rs[k] = r0;
+                const double a0 = fabs(r0);
+                nrm = a0 > nrm ? a0 : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
+                if (has1) {
+                    const double r1 = fext[k1] - m1;
+                    rs[k1] = r1;
+                    const double a1 = fabs(r1);
+                    nrm = a1 > nrm ? a1 : nrm;
+                }
+            }
+        } else {
+            for (int k = lane; k < nk; k += 32) {
+                const double dx = xks[k * DIM] - xi0;
+                const double dy = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
+                const double dz = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
+                const double r = fext[k] - (full_model ? eval_taylor_nested_full<DIM>(fis, dx, dy, dz)
+                                                       : eval_taylor_nested<DIM>(no, fis, dx, dy, dz));
+                rs[k] = r;
+                const double ar = fabs(r);
+                nrm = ar > nrm ? ar : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
+            }
+        }
+        nrm = warp_max_nonneg(nrm);
+        if (nrm == prev) { broke = true; break; }
+        prev = nrm;
+        __syncwarp();
+        if (nr > 0) {
+            double lo, hi;
+            warp_matvec<true>(op_s, rs_u32, nk, nr, gr, lane, lo, hi);
+            const double t0 = fetch_reduced(lo, hi, j0);
+            if (unk0) { v0 += t0; fis[lane] = v0; }
+            if (no > 32) {
+                const double t1 = fetch_reduced(lo, hi, j1);
+                if (unk1) { v1 += t1; fis[lane + 32] = v1; }
+            }
+        }
+        __syncwarp();
+    }
+    // for/else quirk of impl.pyx:1080-1083: a loop that runs to completion reports max_iter,
+    // except max_iter <= 0, which reports 1.
+    if (!broke) it = P.max_iter > 0 ? P.max_iter : 1;
+    return it;
 }
 
 }  // namespace wlsqm

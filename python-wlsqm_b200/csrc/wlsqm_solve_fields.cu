@@ -7,93 +7,14 @@
 //
 // Every field keeps exactly the summation order of the kernel that a single-field solve picks (solve_kernel's grouped
 // warp GEMV, solve_pack_kernel's sequential column chain, the refinement and its exact-equality exit), so each result is
-// bit for bit that solve's; only the reads of the operator elements are shared.  The kernels live in their own
-// translation unit so that the machine code of the single-field kernels (wlsqm_solve.cu) does not change.
+// bit for bit that solve's; only the reads of the operator elements are shared.  The GEMV and the refinement are
+// solve_kernel's own (wlsqm_solve_common.cuh).
 #include <type_traits>
 #include "wlsqm_common.cuh"
 #include "wlsqm_kernels.h"
 #include "wlsqm_solve_common.cuh"
 
 namespace wlsqm {
-
-// ALGO_ITERATIVE refinement of one case against the data (impl.pyx:1010-1083), with the operator block resident at op_s:
-// fis holds the current solution (known slots included), fext the data, rs receives the residuals.  v0 / v1 are this
-// lane's slots lane and lane + 32 (updated in place); returns the reference's iteration count.  The statements of the
-// refinement inside solve_kernel (wlsqm_solve.cu keeps its own copy so that its machine code stays as it is).
-template <int DIM>
-__device__ __forceinline__ int refine_case(const SolveParams& P, long long c, int no, int nk, int nr, const Groups& gr,
-                                           int lane, double* fis, const double* xks, const double* fext, double* rs,
-                                           uint32_t rs_u32, uint32_t op_s, bool unk0, bool unk1, int j0, int j1,
-                                           double& v0, double& v1) {
-    int it;
-    double xi0 = P.xi[c * P.xi_s0], xi1 = 0.0, xi2 = 0.0;
-    if (DIM >= 2) xi1 = P.xi[c * P.xi_s0 + 1];
-    if (DIM >= 3) xi2 = P.xi[c * P.xi_s0 + 2];
-    double prev = -1.0;
-    bool broke = false;
-    const bool full_model = no == max_no<DIM>();     // (warp-uniform) order 4: no test per coefficient
-    for (it = 0; it < P.max_iter; ++it) {
-        double nrm = 0.0;
-        if (DIM == 3 && nk > 32) {
-            // more neighbours than lanes: a lane evaluates the model at its two neighbours k and k + 32 together
-            // (coefficients loaded once, two independent Horner chains).  3D only: the 1D / 2D instantiations run
-            // 24 warps per SM at 80 registers and have none to spare for the second chain.
-            for (int k = lane; k < nk; k += 64) {
-                const int k1 = k + 32;
-                const bool has1 = k1 < nk;
-                const int kb = has1 ? k1 : k;
-                const double dx0 = xks[k * DIM] - xi0, dx1 = xks[kb * DIM] - xi0;
-                const double dy0 = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                const double dy1 = DIM >= 2 ? xks[kb * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                const double dz0 = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                const double dz1 = DIM >= 3 ? xks[kb * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                double m0, m1;
-                if (full_model) eval_taylor_nested2<DIM, true>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
-                else eval_taylor_nested2<DIM, false>(no, fis, dx0, dy0, dz0, dx1, dy1, dz1, m0, m1);
-                const double r0 = fext[k] - m0;
-                rs[k] = r0;
-                const double a0 = fabs(r0);
-                nrm = a0 > nrm ? a0 : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
-                if (has1) {
-                    const double r1 = fext[k1] - m1;
-                    rs[k1] = r1;
-                    const double a1 = fabs(r1);
-                    nrm = a1 > nrm ? a1 : nrm;
-                }
-            }
-        } else {
-            for (int k = lane; k < nk; k += 32) {
-                const double dx = xks[k * DIM] - xi0;
-                const double dy = DIM >= 2 ? xks[k * DIM + (DIM >= 2 ? 1 : 0)] - xi1 : 0.0;
-                const double dz = DIM >= 3 ? xks[k * DIM + (DIM >= 3 ? 2 : 0)] - xi2 : 0.0;
-                const double r = fext[k] - (full_model ? eval_taylor_nested_full<DIM>(fis, dx, dy, dz)
-                                                       : eval_taylor_nested<DIM>(no, fis, dx, dy, dz));
-                rs[k] = r;
-                const double ar = fabs(r);
-                nrm = ar > nrm ? ar : nrm;          // `if tmp > norm` (impl.pyx:1037-1041)
-            }
-        }
-        nrm = warp_max_nonneg(nrm);
-        if (nrm == prev) { broke = true; break; }
-        prev = nrm;
-        __syncwarp();
-        if (nr > 0) {
-            double lo, hi;
-            warp_matvec<true>(op_s, rs_u32, nk, nr, gr, lane, lo, hi);
-            const double t0 = fetch_reduced(lo, hi, j0);
-            if (unk0) { v0 += t0; fis[lane] = v0; }
-            if (no > 32) {
-                const double t1 = fetch_reduced(lo, hi, j1);
-                if (unk1) { v1 += t1; fis[lane + 32] = v1; }
-            }
-        }
-        __syncwarp();
-    }
-    // for/else quirk of impl.pyx:1080-1083: a loop that runs to completion reports max_iter,
-    // except max_iter <= 0, which reports 1.
-    if (!broke) it = P.max_iter > 0 ? P.max_iter : 1;
-    return it;
-}
 
 // warp_matvec_t<LW, false> for FB fields at once: each operator element read from shared memory feeds the four FMA
 // chains of every field (fields f < nfb; the vector of field f at v_s + f * vstride), so that issue per field and row
@@ -201,36 +122,30 @@ __device__ __forceinline__ void warp_matvec_fields(uint32_t op_s, uint32_t v_s, 
 }
 
 // solve_kernel for F.nf fields (ALGO_BASIC: FB fields per block of accumulators; ALGO_ITERATIVE: the fields one after
-// another, each refined against the resident block with its own exit and count).  Ring, records and bulk copies as in
-// solve_kernel; each field's fk row is one more bulk copy into its fext slot of the stage.
+// another, each refined against the resident block with its own exit and count).  Ring and records as in solve_kernel;
+// each field's fk row is one more bulk copy into its fext slot of the stage.
 template <int DIM, bool ITER, bool UNI, int FB>
 __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS, 1) solve_fields_kernel(FieldsParams F) {
     const SolveParams& P = F.P;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
-    const int S = P.stages, nf = F.nf;
+    const int nf = F.nf;
     double* wb = reinterpret_cast<double*>(smem_raw) + (size_t)warp * P.warp_doubles;
     double* ring = wb;
     double* fis = wb + P.off_fi;
     double* rs = wb + P.off_r;
-    const uint32_t ring_u32 = smem_u32(ring);
     const uint32_t rs_u32 = smem_u32(rs);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
     const uint32_t fstride = (uint32_t)F.f_doubles * 8u;
-
-    const long long gw = P.case_lo + (long long)blockIdx.x * nwarps + warp;
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < P.ncases ? (P.ncases - gw + GW - 1) / GW : 0;
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, P.case_lo, P.ncases);
+    const long long gw = R.first, GW = R.stride, n_my = R.n_my;
 
     auto get_meta = [&](long long c) { return case_meta<UNI>(P.meta, P.uni, P.op_stride, c); };
     const bool f_tma = P.f_tma != 0;
     const bool xk_tma = ITER && P.xk_tma;
-    auto issue = [&](int s, long long c) {   // lane 0 only
+    auto issue = [&](uint32_t st, uint32_t bar, long long c) {   // lane 0 only
         const CaseMeta m = get_meta(c);
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         const uint32_t b_op = op_block_bytes(m);
         const uint32_t b_f = f_tma ? (((uint32_t)m.nk + 1u) & ~1u) * 8u : 0u;
         const uint32_t b_x = xk_tma ? (((uint32_t)(m.nk * DIM) + 1u) & ~1u) * 8u : 0u;
@@ -242,30 +157,20 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS, 1) solve_fields_kernel(F
         if (b_x) tma_load_1d_u32(st + (uint32_t)P.off_xk * 8u, P.xk + c * P.xk_s0, b_x, bar);
     };
 
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0, itmax = 0;
-    uint32_t phase = 0;
+    int itmax = 0;
     CaseMeta mt{};
     if (n_my > 0) mt = get_meta(gw);
     long long c = gw;
     for (long long i = 0; i < n_my; ++i, c += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, c + (long long)(S - 1) * GW);
-        }
-        if (!UNI && S > 1 && lane == 0 && i + S < n_my) asm volatile("prefetch.global.L1 [%0];" ::"l"(P.meta + (c + (long long)S * GW)));
+        R.refill(lane, i, c, issue);
+        if (!UNI && R.S > 1 && lane == 0 && i + R.S < n_my) asm volatile("prefetch.global.L1 [%0];" ::"l"(P.meta + (c + (long long)R.S * GW)));
         const long long knowns = mt.knowns;
         if (UNI) mt = P.uni;
         const int nk = mt.nk, no = mt.no, nr = mt.nr, nkn = mt.nkn, nq = nk + nkn;
-        double* st = ring + (size_t)stage * P.stage_doubles;
-        const uint32_t st_u32 = ring_u32 + (uint32_t)stage * stage_bytes;
+        double* st = ring + (size_t)R.stage * P.stage_doubles;
+        const uint32_t st_u32 = R.cur();
         double* fext0 = st + P.off_f;
         const double* xks = st + P.off_xk;
         const Groups gr = make_groups(nr, lane);
@@ -292,7 +197,7 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS, 1) solve_fields_kernel(F
         CaseMeta mt_next = mt;
         if (i + 1 < n_my && (!UNI || P.meta)) mt_next = get_meta(c + GW);
         __syncwarp();
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        R.wait();
         // known values of every field (after the copies have landed: a copy of an odd-length row also writes fext[nk])
         if (nkn) {
             for (int f = 0; f < nf; ++f) {
@@ -358,8 +263,7 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS, 1) solve_fields_kernel(F
             if (P.iters_case && lane == 0) P.iters_case[c] = max(P.iters_case[c], itc);
             itmax = max(itmax, itc);
         }
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
         mt = mt_next;
     }
     if (ITER && lane == 0 && itmax > 0) atomicMax(P.iters_max, itmax);
@@ -373,12 +277,8 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS) solve_pack_fields_kernel
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
-    const int nwarps = blockDim.x >> 5;
-    const int S = P.stages, nf = F.nf;
+    const int nf = F.nf;
     double* ring = reinterpret_cast<double*>(smem_raw) + (size_t)warp * P.warp_doubles;
-    const uint32_t ring_u32 = smem_u32(ring);
-    const uint32_t bars_u32 = smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * S) * 8u;
-    const uint32_t stage_bytes = (uint32_t)P.stage_doubles * 8u;
     const uint32_t fstride = (uint32_t)F.f_doubles * 8u, kstride = (uint32_t)F.k_doubles * 8u;
 
     const CaseMeta u = P.uni;
@@ -387,17 +287,14 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS) solve_pack_fields_kernel
     const int cg = lane >> lw, o = lane & ((1 << lw) - 1);
     const int ops = (int)P.op_stride;
 
-    const long long npacks = (P.ncases - P.case_lo + CPW - 1) / CPW;
-    const long long gw = (long long)blockIdx.x * nwarps + warp;
-    const long long GW = (long long)gridDim.x * nwarps;
-    const long long n_my = gw < npacks ? (npacks - gw + GW - 1) / GW : 0;
+    WarpRing R(smem_u32(ring), smem_u32(smem_raw + P.bar_off_bytes) + (uint32_t)(warp * P.stages) * 8u, P.stages,
+               (uint32_t)P.stage_doubles * 8u, 0, (P.ncases - P.case_lo + CPW - 1) / CPW);   // packs, as in solve_pack_kernel
 
     auto pack_cases = [&](long long pk) { return (int)min((long long)CPW, P.ncases - (P.case_lo + pk * CPW)); };
     auto f_by_tma = [&](int ncs) { return P.f_tma && !((ncs * nk) & 1); };
-    auto issue = [&](int s, long long pk) {   // lane 0 only
+    auto issue = [&](uint32_t st, uint32_t bar, long long pk) {   // lane 0 only
         const long long c0 = P.case_lo + pk * CPW;
         const int ncs = pack_cases(pk);
-        const uint32_t st = ring_u32 + (uint32_t)s * stage_bytes, bar = bars_u32 + (uint32_t)s * 8u;
         const uint32_t b_op = (uint32_t)(ncs * ops) * 8u;
         const uint32_t b_f = f_by_tma(ncs) ? (uint32_t)(ncs * nk) * 8u : 0u;
         mbar_expect_tx_u32(bar, b_op + (uint32_t)nf * b_f);
@@ -407,27 +304,16 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS) solve_pack_fields_kernel
                 tma_load_1d_u32(st + (uint32_t)P.off_f * 8u + (uint32_t)f * fstride, P.fk + f * F.fk_sf + c0 * P.fk_s0, b_f, bar);
     };
 
-    if (lane == 0) {
-        for (int s = 0; s < S; ++s) mbar_init_u32(bars_u32 + (uint32_t)s * 8u, 1);
-        fence_mbar_init();
-        for (int s = 0; s < S - 1 && s < n_my; ++s) issue(s, gw + (long long)s * GW);
-    }
-    __syncwarp();
+    R.start(lane, issue);
 
-    int stage = 0;
-    uint32_t phase = 0;
-    long long pk = gw;
-    for (long long i = 0; i < n_my; ++i, pk += GW) {
-        if (lane == 0 && i + S - 1 < n_my) {
-            int sn = stage + S - 1;
-            if (sn >= S) sn -= S;
-            issue(sn, pk + (long long)(S - 1) * GW);
-        }
+    long long pk = R.first;
+    for (long long i = 0; i < R.n_my; ++i, pk += R.stride) {
+        R.refill(lane, i, pk, issue);
         const long long c0 = P.case_lo + pk * CPW;
         const int ncs = pack_cases(pk);
         const long long c = c0 + cg;
-        double* st = ring + (size_t)stage * P.stage_doubles;
-        const uint32_t st_u32 = ring_u32 + (uint32_t)stage * stage_bytes;
+        double* st = ring + (size_t)R.stage * P.stage_doubles;
+        const uint32_t st_u32 = R.cur();
         if (!f_by_tma(ncs)) {
             for (int f = 0; f < nf; ++f) {
                 double* fs = st + P.off_f + f * F.f_doubles;
@@ -446,7 +332,7 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS) solve_pack_fields_kernel
         if (nkn && valid && isk)
             for (int f = 0; f < nf; ++f) st[P.off_xk + f * F.k_doubles + cg * nkn + below] = F.fi[f * F.fi_sf + c * F.fi_s0 + o];
         __syncwarp();
-        mbar_wait_u32(bars_u32 + (uint32_t)stage * 8u, phase);
+        R.wait();
 
         if (valid && !isk) {
             for (int f0 = 0; f0 < nf; f0 += FB) {
@@ -499,8 +385,7 @@ __global__ void __launch_bounds__(SOLVE_FIELDS_THREADS) solve_pack_fields_kernel
                 }
             }
         }
-        __syncwarp();   // every lane is done with this stage before lane 0 re-arms it
-        if (++stage == S) { stage = 0; phase ^= 1u; }
+        R.release();
     }
 }
 

@@ -179,6 +179,37 @@ WLSQM_API int wlsqm_grid_info(wlsqm_grid_t* g, int64_t* ncells, double* cell_siz
 WLSQM_API int wlsqm_grid_knn(wlsqm_grid_t* g, const double* xq, int64_t xq_s0, int64_t nq, int k, int exclude_self,
                    int32_t* idx32, int64_t* idx64, double* d2);
 
+/* Fixed-radius neighbourhoods -- cKDTree.query_ball_point(xq, r) (the callers' other neighbourhood search,
+ * examples/wlsqm_example.py:100-132), as CSR lists: row q holds the grid points p with
+ *     d2(p, q) <= r_q * r_q,   d2 = sum over the axes in axis order of (x_p[d] - q[d])^2,
+ * every difference, square, sum and r_q * r_q rounded on its own (no fused multiply-add), identically in every kernel
+ * that decides membership.  A point at exactly r is a member (as in cKDTree).
+ *   - Points with a NaN or infinite coordinate are never members.  A query with a NaN or infinite coordinate gets an
+ *     empty row (cKDTree raises for NaN queries).
+ *   - xq == NULL: the queries are the grid's own points (nq is ignored, row i is point i); exclude_self drops only the
+ *     point's own index, coincident points stay.  With xq, exclude_self is ignored.
+ *   - r: one radius (r_s0 == 0) or one per query (row stride r_s0; for the grid's own points r[i] belongs to point i).
+ *     Every radius must be >= 0 and not NaN, else WLSQM_E_VALUE; +inf means every finite point.
+ *   - order WLSQM_BALL_BY_INDEX: each row ascending by index (query_ball_point's order for several queries);
+ *     WLSQM_BALL_BY_DISTANCE: ascending by (d2, index), the order of wlsqm_grid_knn.
+ *   - max_k (0: no cap, else 1..128): a row keeps its max_k members nearest by (d2, index), then arranged by order.
+ *     With r = inf, a capped self-query row is the row of wlsqm_grid_knn(k = max_k) as a set, and in the same order
+ *     under WLSQM_BALL_BY_DISTANCE, wherever the distances of the row and of the (k+1)-th neighbour are distinct beyond
+ *     rounding: wlsqm_grid_knn may fuse the squares and sums of d2 into FMAs, so at near-ties the two can rank
+ *     differently.
+ * Two calls with the same arguments: the count call gives rowptr int64 [nq + 1] (may be NULL), counts int32 [nq] (may be
+ * NULL) and *nnz = rowptr[nq]; the csr call fills col int32 [nnz] for that rowptr (at most 2^31 - 1 entries per call).
+ * Any array may be in host or device memory (host ones are staged); the work is ordered after the caller's stream
+ * and both calls return when their outputs are written. */
+#define WLSQM_BALL_BY_INDEX 0
+#define WLSQM_BALL_BY_DISTANCE 1
+WLSQM_API int wlsqm_grid_ball_count(wlsqm_grid_t* g, const double* xq, int64_t xq_s0, int64_t nq, const double* r,
+                                    int64_t r_s0, int exclude_self, int max_k, int64_t* rowptr, int32_t* counts,
+                                    int64_t* nnz);
+WLSQM_API int wlsqm_grid_ball_csr(wlsqm_grid_t* g, const double* xq, int64_t xq_s0, int64_t nq, const double* r,
+                                  int64_t r_s0, int exclude_self, int max_k, int order, const int64_t* rowptr,
+                                  int32_t* col);
+
 /* x[hoods] / f[hoods]: dst[i][k][0..w) = src[idx[i][k]][0..w)  (the caller-side gathers of the examples).
  * src [nsrc][w] (row stride src_s0), idx int32 [n][k] (row stride idx_s0), dst [n][k][w] dense.  Asynchronous on
  * cuda_stream; an index outside [0, nsrc) -- where numpy raises IndexError -- yields NaN, nothing is read out of bounds. */

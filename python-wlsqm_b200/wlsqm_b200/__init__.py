@@ -13,7 +13,7 @@ from .fitter.simple import *    # noqa: F401,F403
 from .fitter.interp import *    # noqa: F401,F403
 from .fitter.expert import *    # noqa: F401,F403
 from ._lib import pinned_empty, pinned_free, pool_stats, pool_trim, LIB_PATH  # noqa: F401
-from .neighbors import PointGrid, knn_hoods, gather  # noqa: F401  (extension: device-side neighbour search)
+from .neighbors import PointGrid, knn_hoods, ball_hoods, gather  # noqa: F401  (extension: device-side neighbour search)
 from . import fitter, utils     # noqa: F401  (the reference exposes its subpackages as attributes)
 from .fitter import impl, infra, polyeval  # noqa: F401  (module layout of the reference; see their docstrings)
 from .utils import ptrwrap      # noqa: F401

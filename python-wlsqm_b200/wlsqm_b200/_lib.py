@@ -60,6 +60,8 @@ SIGNATURES = {
     "wlsqm_grid_destroy": (_int, [_vp]),
     "wlsqm_grid_info": (_int, [_vp, _i64p, C.POINTER(C.c_double), _i64p]),
     "wlsqm_grid_knn": (_int, [_vp, _vp, _i64, _i64, _int, _int, _vp, _vp, _vp]),
+    "wlsqm_grid_ball_count": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _int, _int, _vp, _vp, _i64p]),
+    "wlsqm_grid_ball_csr": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _int, _int, _int, _vp, _vp]),
     "wlsqm_gather_hoods": (_int, [_vp, _i64, _int, _i64, _vp, _i64, _i64, _int, _vp, _int, _vp]),
     "wlsqm_solver_prepare_hoods": (_int, [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _i64]),
     "wlsqm_solver_solve_hoods": (_int, [_vp, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32p]),

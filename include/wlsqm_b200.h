@@ -318,6 +318,33 @@ WLSQM_API int wlsqm_solver_nearest_models(wlsqm_solver_t* s, const double* x, in
 WLSQM_API int wlsqm_solver_interpolate_continuous(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
                                         int diff, double* out);
 
+/* Several fields on one geometry (extension): evaluate caller-held solutions, e.g. the fi written by
+ * wlsqm_solver_solve_fields, at query points.  Field j of out is BIT FOR BIT what wlsqm_solver_interpolate (or
+ * _interpolate_continuous) writes for the same x, I, diff (and r) when the solver's solution copy holds fi[j][i][0..no_i)
+ * for every case i -- what a guest solver answers after its last solve() produced fi[j].  Each query loads its index,
+ * coordinates and origin, and in continuous mode walks the model grid, once per pass of up to 8 fields.
+ *   - fi [nf][ncases][>= max no], element strides fi_sf, fi_s0 (any non-negative values: it is only read; fields-outer,
+ *     fields-inner and fi_sf = 0 all work), contiguous last axis.  Slots >= no_i are never read.
+ *   - wlsqm_solver_interpolate_fields (nearest mode): I int64 [nx].  One slot: out[j*out_sf + q*out_sq].
+ *     diff == WLSQM_DIFF_ALL: out[j*out_sf + q*out_sq + s] for s < max no, slots >= no_{I[q]} written as 0.0.
+ *     I[q] outside [0, ncases) gives NaN, as in wlsqm_solver_interpolate.
+ *   - wlsqm_solver_interpolate_continuous_fields: one slot; r > 0 (else WLSQM_E_VALUE); needs wlsqm_solver_index_models
+ *     (else WLSQM_E_NOTREADY).  A query with no model within r gives NaN (0/0).
+ *   - out: out_sf, out_sq >= 0 in a layout whose (field, query, slot) map is injective, with width 1 or max no:
+ *     fields-outer (out_sf >= (nx-1)*out_sq + width, out_sq >= width) or fields-inner (out_sf >= width,
+ *     out_sq >= (nf-1)*out_sf + width); else WLSQM_E_VALUE.  A device out overlapping a device fi, x or I: WLSQM_E_VALUE.
+ *   - Solver not prepared, or without cases: WLSQM_E_NOTREADY.  Invalid diff: WLSQM_E_VALUE.  nf = 0 or nx = 0: no-op.
+ *   - The solver's solution copy is neither read nor written: the calls work after solve_fields and keep_solution(0).
+ *   - Any array may be in host or device memory.  Device arrays are used in place, asynchronously on the solver's
+ *     stream; host ones are staged, and the call returns when host outputs are written.  A guest answers with its host's
+ *     origins. */
+WLSQM_API int wlsqm_solver_interpolate_fields(wlsqm_solver_t* s, int64_t nf, const double* fi, int64_t fi_sf, int64_t fi_s0,
+                                              const double* x, int64_t x_s0, const int64_t* I, int64_t nx, int diff,
+                                              double* out, int64_t out_sf, int64_t out_sq);
+WLSQM_API int wlsqm_solver_interpolate_continuous_fields(wlsqm_solver_t* s, int64_t nf, const double* fi, int64_t fi_sf,
+                                                         int64_t fi_s0, const double* x, int64_t x_s0, int64_t nx, double r,
+                                                         int diff, double* out, int64_t out_sf, int64_t out_sq);
+
 /* The reference keeps the solution twice: in the caller's fi and in each Case (Case_set_fi, infra.pyx:780-786), which is
  * what interpolate() evaluates (expert.pyx:571-699).  A caller that never interpolates can drop the second copy:
  * keep = 0 makes solve() with a device-resident fi write the caller's array only (8 * no bytes per case less traffic);

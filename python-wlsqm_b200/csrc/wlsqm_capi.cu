@@ -215,6 +215,7 @@ struct wlsqm_solver {
     double* fi_case = nullptr;
     // wlsqm_solver_keep_solution(s, 0): solve() with a device fi writes the caller's array only; interpolate() needs the copy
     bool keep_solution = true, fi_case_valid = true;
+    int l2_bytes = 0;                            // L2 size of the device (interpolate_fields' pass plan)
     double* xi_dev = nullptr;
     double* As = nullptr;
     int as_stride = 0;
@@ -611,6 +612,15 @@ bool ranges_overlap(const void* a, long long abytes, const void* b, long long bb
     const char* a0 = (const char*)a;
     const char* b0 = (const char*)b;
     return a0 < b0 + bbytes && b0 < a0 + abytes;
+}
+
+// whether the (field, row, slot) -> element map of an [nf][rows][width] array with element strides sf, s0 and a
+// contiguous last axis is injective in one of the two accepted layouts: fields-outer (sf >= (rows-1)*s0 + width,
+// s0 >= width) or fields-inner (sf >= width, s0 >= (nf-1)*sf + width).  fitter/fields.py states the same rule.
+bool fields_layout_ok(long long nf, long long rows, long long width, long long sf, long long s0) {
+    const bool outer = (nf == 1 || sf >= (rows - 1) * s0 + width) && (rows == 1 || s0 >= width);
+    const bool inner = (nf == 1 || sf >= width) && (rows == 1 || s0 >= (nf - 1) * sf + width);
+    return sf >= 0 && s0 >= 0 && (outer || inner);
 }
 
 }  // namespace
@@ -1545,9 +1555,7 @@ static int solve_fields_core(wlsqm_solver_t* s, int64_t nf, bool hoods, const do
     if ((hoods ? !hf : !fk) || !fi) return fail(WLSQM_E_VALUE, "fk (f) and fi must not be NULL");
     const int maxno = s->maxno, maxnk = s->maxnk;
     // the (field, case, slot) -> element map of fi must be injective: fields-outer or fields-inner rows
-    const bool fi_outer = (nf == 1 || fi_sf >= (n - 1) * fi_s0 + maxno) && (n == 1 || fi_s0 >= maxno);
-    const bool fi_inner = (nf == 1 || fi_sf >= maxno) && (n == 1 || fi_s0 >= (nf - 1) * fi_sf + maxno);
-    if (fi_sf < 0 || fi_s0 < 0 || !(fi_outer || fi_inner))
+    if (!fields_layout_ok(nf, n, maxno, fi_sf, fi_s0))
         return fail(WLSQM_E_VALUE, "fi layout (field stride %lld, row stride %lld) maps two (field, case, slot) entries to one "
                     "element; use fields-outer (fi_sf >= (ncases-1)*fi_s0 + max no) or fields-inner (fi_sf >= max no, "
                     "fi_s0 >= (nf-1)*fi_sf + max no) rows", (long long)fi_sf, (long long)fi_s0);
@@ -2116,6 +2124,156 @@ int wlsqm_solver_interpolate_continuous(wlsqm_solver_t* s, const double* x, int6
     if (!out_dev) CU(cudaMemcpyAsync(out, s->st_out.p, (size_t)nx * 8, cudaMemcpyDeviceToHost, st));
     if (!x_dev || !out_dev) CU(cudaStreamSynchronize(st));
     return WLSQM_OK;
+}
+
+// Several caller-held solutions at once (wlsqm_interp_fields.cu): wlsqm_solver_interpolate (I given) or
+// wlsqm_solver_interpolate_continuous (I == NULL, continuous) per field j of fi [nf][ncases][>= max no].
+static int interp_fields_core(wlsqm_solver_t* s, int64_t nf, const double* fi, int64_t fi_sf, int64_t fi_s0, const double* x,
+                              int64_t x_s0, const int64_t* I, int64_t nx, bool continuous, double r, int diff, double* out,
+                              int64_t out_sf, int64_t out_sq) {
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    if (!s->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called first");
+    if (continuous && !s->models_grid)
+        return fail(WLSQM_E_NOTREADY, "Points xi have not been indexed; prep_interpolate() must be called before interpolate()");
+    if (nf < 0 || nx < 0) return fail(WLSQM_E_VALUE, "nf and nx must be >= 0");
+    if (nf == 0 || nx == 0) return WLSQM_OK;
+    if (!fi || !x || (!continuous && !I) || !out) return fail(WLSQM_E_VALUE, "fi, x, I and out must not be NULL");
+    if (continuous && !(r > 0.0)) return fail(WLSQM_E_VALUE, "r must be positive");
+    const int size = number_of_dofs(s->dim, 4);
+    const bool all = !continuous && diff == WLSQM_DIFF_ALL;
+    if (!all && (diff < 0 || diff >= size)) return fail(WLSQM_E_VALUE, "invalid diff %d", diff);
+    const long long n = s->ncases, dim = s->dim, maxno = s->maxno, width = all ? maxno : 1;
+    if (n == 0) return fail(WLSQM_E_NOTREADY, "the solver has no models to evaluate");
+    if (fi_sf < 0 || fi_s0 < 0 || x_s0 < 0) return fail(WLSQM_E_VALUE, "fi and x strides must be >= 0");
+    if (!fields_layout_ok(nf, nx, width, out_sf, out_sq))
+        return fail(WLSQM_E_VALUE, "out layout (field stride %lld, query stride %lld) maps two (field, query, slot) entries to "
+                    "one element; use fields-outer (out_sf >= (nx-1)*out_sq + width, out_sq >= width) or fields-inner "
+                    "(out_sf >= width, out_sq >= (nf-1)*out_sf + width) rows, width %lld", (long long)out_sf,
+                    (long long)out_sq, width);
+    int rc = use_device(s);
+    if (rc) return rc;
+    cudaStream_t st = s->stream;
+    const bool fi_dev = is_device_ptr(fi), x_dev = is_device_ptr(x), I_dev = !continuous && is_device_ptr(I);
+    const bool out_dev = is_device_ptr(out);
+    // elements spanned by each strided array (all strides are non-negative)
+    const long long fi_span = (nf - 1) * fi_sf + (n - 1) * fi_s0 + maxno;
+    const long long out_span = (nf - 1) * out_sf + (nx - 1) * out_sq + width;
+    if (out_dev) {
+        if ((fi_dev && ranges_overlap(out, out_span * 8, fi, fi_span * 8)) ||
+            (x_dev && ranges_overlap(out, out_span * 8, x, ((nx - 1) * x_s0 + dim) * 8)) ||
+            (I_dev && ranges_overlap(out, out_span * 8, I, nx * 8)))
+            return fail(WLSQM_E_VALUE, "device out overlaps device fi, x or I");
+    }
+
+    InterpFieldsParams F{};
+    InterpParams& P = F.P;
+    P.dim = s->dim; P.nx = nx; P.diff = all ? -1 : diff; P.nmodels = n;
+    P.xi = s->xi_dev; P.xi_s0 = s->dim;
+    P.order = s->dorder; P.order_uniform = s->uni.order;
+    F.width = (int)width;
+    // fi rows that are not dense (fields-inner, pitched) are copied to dense rows, one pass at a time right before the
+    // pass: the rows of one field then share L2 lines with no other field's, and the rows just written are still largely
+    // in L2 when the pass reads them.  Read in place, fields-inner rows at 1M models and 16M queries took 2.7 to 3.4 times
+    // the time of dense ones (profiles/r08_interp_fields_plans.txt).  Host fi is staged the same way, per pass; host rows
+    // that overlap (fi_s0 < max no) are staged whole as one span, strides kept.
+    const double* fi_use = fi;
+    const bool compact = fi_s0 >= maxno && (!fi_dev || (fi_s0 != maxno && n > 1));
+    if (!compact && !fi_dev) {
+        rc = s->st_fi.reserve((size_t)fi_span * 8);
+        if (rc) return rc;
+        rc = to_dense((double*)s->st_fi.p, fi, 1, fi_span, fi_span, st);
+        if (rc) return rc;
+        fi_use = (const double*)s->st_fi.p;
+    }
+    if (x_dev) { P.x = x; P.x_s0 = x_s0; }
+    else {
+        rc = s->st_x.reserve((size_t)nx * dim * 8);
+        if (rc) return rc;
+        rc = stage_in(s->device, (double*)s->st_x.p, x, nx, dim, x_s0, st);
+        if (rc) return rc;
+        P.x = (const double*)s->st_x.p; P.x_s0 = dim;
+    }
+    if (!continuous) {
+        if (I_dev) P.I = (const long long*)I;
+        else {
+            rc = s->st_I.reserve((size_t)nx * 8);
+            if (rc) return rc;
+            rc = stage_in(s->device, (double*)s->st_I.p, reinterpret_cast<const double*>(I), nx, 1, 1, st);   // (8-byte items)
+            if (rc) return rc;
+            P.I = (const long long*)s->st_I.p;
+        }
+    }
+    double* out_use = out;
+    long long out_sf_use = out_sf;
+    if (out_dev) P.out_s0 = out_sq;
+    else {
+        rc = s->st_out.reserve((size_t)nf * nx * width * 8);
+        if (rc) return rc;
+        out_use = (double*)s->st_out.p; out_sf_use = nx * width; P.out_s0 = width;
+    }
+    P.stage_no = (all && s->uniform_no && P.out_s0 == s->uni.no) ? s->uni.no : 0;
+
+    // fields per pass from the byte model of wlsqm_interp_fields.cu
+    if (!s->l2_bytes) CU(cudaDeviceGetAttribute(&s->l2_bytes, cudaDevAttrL2CacheSize, s->device));
+    double rows_per_query = 1.0, query_bytes = 8.0 * dim + 8.0;
+    GridView g{};
+    if (continuous) {
+        // models in a ball of radius r and candidates in its cell box, for a uniform density over the grid's box
+        g = grid_view(s->models_grid);
+        double box = 1.0, ball = 1.0, cells = 1.0;
+        for (int d = 0; d < dim; ++d) { box *= g.dims[d] * g.h; ball *= r; cells *= 2.0 * r + g.h; }
+        ball *= dim == 1 ? 2.0 : (dim == 2 ? 3.141592653589793 : 4.0 / 3.0 * 3.141592653589793);
+        rows_per_query = std::min((double)n, std::max(1.0, n * ball / box));
+        query_bytes = 8.0 * dim + std::min((double)n, n * cells / box) * (8.0 * dim + 4.0);
+    }
+    const int fb = interp_fields_per_pass(nf, n, s->maxno, nx, rows_per_query, query_bytes, 8.0 * width, s->l2_bytes);
+    if (compact) {
+        rc = s->st_fi.reserve((size_t)std::min<long long>(fb, nf) * n * maxno * 8);
+        if (rc) return rc;
+    }
+    for (long long p0 = 0; p0 < nf; p0 += fb) {
+        F.nf = (int)std::min<long long>(fb, nf - p0);
+        if (compact) {
+            double* dense = (double*)s->st_fi.p;
+            if (fi_dev) CU(launch_compact_rows(fi + p0 * fi_sf, fi_sf, fi_s0, F.nf, n, (int)maxno, dense, st));
+            else {
+                for (int j = 0; j < F.nf; ++j) {
+                    rc = to_dense(dense + j * n * maxno, fi + (p0 + j) * fi_sf, n, maxno, fi_s0, st);
+                    if (rc) return rc;
+                }
+            }
+            P.fi = dense; P.fi_s0 = maxno; F.fi_sf = n * maxno;
+        } else {
+            P.fi = fi_use + p0 * fi_sf; P.fi_s0 = fi_s0; F.fi_sf = fi_sf;
+        }
+        P.out = out_use + p0 * out_sf_use; F.out_sf = out_sf_use;
+        if (F.nf == 1 && !all && P.out_s0 == 1) {
+            // one field in this pass, dense one-slot output: the single-field kernel and its launch shape serve it
+            CU(continuous ? launch_interpolate_continuous(P, g, r, st) : launch_interpolate(P, st));
+        } else {
+            CU(continuous ? launch_interpolate_continuous_fields(F, g, r, st) : launch_interpolate_fields(F, st));
+        }
+    }
+    if (!out_dev) {
+        for (long long j = 0; j < nf; ++j) {
+            rc = stage_out(s->device, out + j * out_sf, out_sq, (const double*)s->st_out.p + j * nx * width, width, nx, width, st);
+            if (rc) return rc;
+        }
+    }
+    if (!fi_dev || !x_dev || (!continuous && !I_dev) || !out_dev) CU(cudaStreamSynchronize(st));
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_interpolate_fields(wlsqm_solver_t* s, int64_t nf, const double* fi, int64_t fi_sf, int64_t fi_s0,
+                                    const double* x, int64_t x_s0, const int64_t* I, int64_t nx, int diff, double* out,
+                                    int64_t out_sf, int64_t out_sq) {
+    return interp_fields_core(s, nf, fi, fi_sf, fi_s0, x, x_s0, I, nx, false, 0.0, diff, out, out_sf, out_sq);
+}
+
+int wlsqm_solver_interpolate_continuous_fields(wlsqm_solver_t* s, int64_t nf, const double* fi, int64_t fi_sf,
+                                               int64_t fi_s0, const double* x, int64_t x_s0, int64_t nx, double r, int diff,
+                                               double* out, int64_t out_sf, int64_t out_sq) {
+    return interp_fields_core(s, nf, fi, fi_sf, fi_s0, x, x_s0, nullptr, nx, true, r, diff, out, out_sf, out_sq);
 }
 
 // One-shot fits without sensitivities on a uniform batch: one launch of the fused kernel (assemble, equilibrate,

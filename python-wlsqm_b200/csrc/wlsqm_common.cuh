@@ -186,6 +186,35 @@ __device__ __forceinline__ double eval_diff(const double* __restrict__ fg, int n
     return eval_diff_from<DIM, D>([&](int S) { return __ldg(fg + S); }, no, hx, hy, hz);
 }
 
+// In-place Taylor shift of the coefficient array along one axis: afterwards u[(a, b, c)] holds the a-th partial
+// derivative along AXIS, at offset h (st = steps_of(h)), of the line of coefficients with the other two exponents fixed.
+// The interpolation kernels (wlsqm_interp.cu, wlsqm_interp_fields.cu) share it, so their slots agree bit for bit.
+template <int DIM, int AXIS>
+__device__ __forceinline__ void taylor_shift(double (&u)[max_no<DIM>()], const Steps& st) {
+    static_for<0, 5>([&](auto Bc) {
+        static_for<0, 5>([&](auto Cc) {
+            constexpr int b = decltype(Bc)::value, c = decltype(Cc)::value;   // the other two exponents, in axis order
+            constexpr int A = 4 - b - c;
+            constexpr bool line = A >= 1 && (DIM >= 3 || c == 0) && (DIM >= 2 || b == 0);
+            if constexpr (line) {
+                static_for<0, A>([&](auto Jc) {
+                    constexpr int j = decltype(Jc)::value;
+                    static_rfor<A - 1, j>([&](auto Ic) {
+                        constexpr int i = decltype(Ic)::value;
+                        constexpr int S0 = AXIS == 0 ? slot_of<DIM>(i, b, c) : (AXIS == 1 ? slot_of<DIM>(b, i, c) : slot_of<DIM>(b, c, i));
+                        constexpr int S1 = AXIS == 0 ? slot_of<DIM>(i + 1, b, c) : (AXIS == 1 ? slot_of<DIM>(b, i + 1, c) : slot_of<DIM>(b, c, i + 1));
+                        u[S0] = fma(st.s[i], u[S1], u[S0]);
+                    });
+                });
+            }
+        });
+    });
+}
+template <int DIM, int AXIS>
+__device__ __forceinline__ void taylor_shift(double (&u)[max_no<DIM>()], double h) {
+    taylor_shift<DIM, AXIS>(u, steps_of(h));
+}
+
 // Model value at offset (dx,dy,dz) from the origin, coefficients anywhere (shared memory in the solve kernel's
 // refinement loop): one broadcast load and one FMA per coefficient.
 template <int DIM>

@@ -33,31 +33,6 @@ namespace wlsqm {
 constexpr int INTERP_THREADS = 256;
 constexpr int INTERP_Q = 4;        // queries per thread (all slots); the one-slot kernels in 1D / 2D take 2, see launch_interp_m
 
-// In-place Taylor shift of the coefficient array along one axis: afterwards u[(a, b, c)] holds the a-th partial
-// derivative along AXIS, at offset h, of the line of coefficients with the other two exponents fixed.
-template <int DIM, int AXIS>
-__device__ __forceinline__ void taylor_shift(double (&u)[max_no<DIM>()], double h) {
-    const Steps st = steps_of(h);
-    static_for<0, 5>([&](auto Bc) {
-        static_for<0, 5>([&](auto Cc) {
-            constexpr int b = decltype(Bc)::value, c = decltype(Cc)::value;   // the other two exponents, in axis order
-            constexpr int A = 4 - b - c;
-            constexpr bool line = A >= 1 && (DIM >= 3 || c == 0) && (DIM >= 2 || b == 0);
-            if constexpr (line) {
-                static_for<0, A>([&](auto Jc) {
-                    constexpr int j = decltype(Jc)::value;
-                    static_rfor<A - 1, j>([&](auto Ic) {
-                        constexpr int i = decltype(Ic)::value;
-                        constexpr int S0 = AXIS == 0 ? slot_of<DIM>(i, b, c) : (AXIS == 1 ? slot_of<DIM>(b, i, c) : slot_of<DIM>(b, c, i));
-                        constexpr int S1 = AXIS == 0 ? slot_of<DIM>(i + 1, b, c) : (AXIS == 1 ? slot_of<DIM>(b, i + 1, c) : slot_of<DIM>(b, c, i + 1));
-                        u[S0] = fma(st.s[i], u[S1], u[S0]);
-                    });
-                });
-            }
-        });
-    });
-}
-
 // ALL = every derivative slot (WLSQM_DIFF_ALL); STAGE = transpose the warp's results through shared memory.
 // Each thread owns INTERP_Q queries, blockDim apart (coalesced), and issues their index and coordinate loads
 // together before the dependent model-row loads: the kernel is bound by load latency, not by arithmetic.

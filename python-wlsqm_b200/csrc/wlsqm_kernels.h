@@ -250,6 +250,15 @@ struct InterpParams {
                                                      // results are transposed through shared memory (else 0)
 };
 
+// Several fields per launch (wlsqm_interp_fields.cu): P.fi / P.out point at the first field of the pass, field j at
+// + j * fi_sf / + j * out_sf; P.out_s0 is the query stride of out in both modes.
+struct InterpFieldsParams {
+    InterpParams P;
+    long long fi_sf, out_sf;
+    int nf;                                          // fields of this pass (<= 8)
+    int width;                                       // all slots: slots written per query (max no), zeros beyond no_i
+};
+
 // thread-local message behind wlsqm_last_error() (wlsqm_capi.cu)
 void set_last_error(const char* msg);
 
@@ -278,6 +287,12 @@ cudaError_t interp_runs(const long long* I, long long nx, long long nmodels, con
 cudaError_t launch_interp_stencils(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
 struct GridView;
 cudaError_t launch_interpolate_continuous(const InterpParams& P, const GridView& g, double r, cudaStream_t st);
+int interp_fields_per_pass(long long nf, long long ncases, int maxno, long long nx, double rows_per_query,
+                           double query_bytes, double out_bytes, long long l2_bytes);
+cudaError_t launch_interpolate_fields(const InterpFieldsParams& F, cudaStream_t st);
+cudaError_t launch_compact_rows(const double* src, long long sf, long long s0, int nfp, long long n, int maxno, double* dst,
+                                cudaStream_t st);
+cudaError_t launch_interpolate_continuous_fields(const InterpFieldsParams& F, const GridView& g, double r, cudaStream_t st);
 cudaError_t launch_getrf(int n, long long nlhs, double* A, int* ipiv, cudaStream_t st);
 cudaError_t launch_getrs(int n, long long nlhs, const double* LU, const int* ipiv, double* b, cudaStream_t st);
 cudaError_t launch_gesv(int n, long long nlhs, double* A, int* ipiv, double* b, cudaStream_t st);

@@ -76,6 +76,9 @@ SIGNATURES = {
     "wlsqm_solver_index_models": (_int, [_vp]),
     "wlsqm_solver_nearest_models": (_int, [_vp, _vp, _i64, _i64, _vp]),
     "wlsqm_solver_interpolate_continuous": (_int, [_vp, _vp, _i64, _i64, C.c_double, _int, _vp]),
+    "wlsqm_solver_interpolate_fields": (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _i64, _vp, _i64, _int, _vp, _i64, _i64]),
+    "wlsqm_solver_interpolate_continuous_fields": (_int, [_vp, _i64, _vp, _i64, _i64, _vp, _i64, _i64, C.c_double, _int,
+                                                          _vp, _i64, _i64]),
     "wlsqm_peer_alloc": (_int, [_int, _i64, C.POINTER(_vp), _vp]),
     "wlsqm_peer_open": (_int, [_int, _vp, C.POINTER(_vp)]),
     "wlsqm_peer_close": (_int, [_vp]),

@@ -858,6 +858,14 @@ class ExpertSolver:
         _check(rc)
         return out, (I_out if ax.cuda and _is_tensor(I_out) else np.asanyarray(I_out))
 
+    def interpolate_fields(self, x, fi, mode='nearest', r=None, diff=0, I=None):
+        """interpolate() for nf caller-held solutions at once (extension): fi (nf, >= ncases, >= max no), e.g. the fi of
+        solve_fields (fi[None] for one field).  Returns (out, I_out) with out (nf, nx), or (nf, nx, max no) for
+        diff='all'; out[j] is bit for bit what interpolate() returns on a solver whose last solve() produced fi[j].  The
+        solver's own solution copy is not used, so this works after solve_fields and keep_solution(False).  See
+        wlsqm_b200.fitter.fields.interpolate_fields."""
+        return _fields.interpolate_fields(self, x, fi, mode, r, diff, I)
+
     def _interpolate_continuous(self, x, uintptr_t xp, int64_t x_s0, Py_ssize_t nx, bint cuda, double r, int cdiff):
         """mode='continuous' (``expert_interpolate_continuous``, ``expert.pyx:898-985``): weighted average
         over every local model whose origin lies within r; weights (1 - sqrt(d2/r2))^2.  One kernel: each query

@@ -471,6 +471,14 @@ class ExpertSolver:
         _lib.check(_lib.lib().wlsqm_solver_interpolate(self._handle, x_a.ptr, x_s0, I_a.ptr, nx, cdiff, out_p, width))
         return out, (I_out if x_a.is_cuda and _lib._is_torch_tensor(I_out) else np.asanyarray(I_out))
 
+    def interpolate_fields(self, x, fi, mode='nearest', r=None, diff=0, I=None):
+        """interpolate() for nf caller-held solutions at once (extension): fi (nf, >= ncases, >= max no), e.g. the fi of
+        solve_fields (fi[None] for one field).  Returns (out, I_out) with out (nf, nx), or (nf, nx, max no) for
+        diff='all'; out[j] is bit for bit what interpolate() returns on a solver whose last solve() produced fi[j].  The
+        solver's own solution copy is not used, so this works after solve_fields and keep_solution(False).  See
+        wlsqm_b200.fitter.fields.interpolate_fields."""
+        return fields.interpolate_fields(self, x, fi, mode, r, diff, I)
+
     def _interpolate_continuous(self, x_a, x_s0, r, cdiff):
         """mode='continuous' (``expert_interpolate_continuous``, ``expert.pyx:898-985``): weighted average
         over every local model whose origin lies within r; weights (1 - sqrt(d2/r2))^2.  One kernel: each query

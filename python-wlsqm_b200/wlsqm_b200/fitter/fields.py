@@ -17,6 +17,7 @@ import ctypes as C
 import numpy as np
 
 from .. import _lib
+from . import opexport
 
 
 def fi_layout_ok(nf, ncases, maxno, fi_sf, fi_s0):
@@ -107,3 +108,69 @@ def solve_hoods_fields(solver, f, fi):
     _lib.check(_lib.lib().wlsqm_solver_solve_hoods_fields(solver._handle, nf, f_a.ptr, f_sf, f_s0, fi_a.ptr, fi_sf, fi_s0,
                                                           C.byref(it)))
     return int(it.value)
+
+
+def resolve_fi_read(fi, ncases, maxno):
+    """fi (nf, >= ncases, >= max no) float64, read only, contiguous last axis -> (Arr, nf, fi_sf, fi_s0); any
+    non-negative strides"""
+    if _no_fields(fi, 3):
+        return None, 0, 0, 0
+    a = _lib.as_arr(fi, np.float64, 3, "fi")
+    nf = a.shape[0]
+    if nf and (a.shape[1] < ncases or a.shape[2] < maxno):
+        raise ValueError("fi must have shape (nf, >= ncases = %d, >= max no = %d), got %s" % (ncases, maxno, a.shape))
+    return a, nf, a.strides[0], a.strides[1]
+
+
+def interpolate_fields(solver, x, fi, mode='nearest', r=None, diff=0, I=None):
+    """interpolate() for nf caller-held solutions fi (nf, >= ncases, >= max no) -- the fi of solve_fields, say -- in one
+    pass over the queries.  Returns (out, I_out): out (nf, nx), or (nf, nx, max no) for diff='all', a CUDA tensor when x
+    is one, else numpy; out[j] is bit for bit interpolate(x, mode, r, diff, I)[0] of a solver whose last solve() produced
+    fi[j].  Models and I_out are found as interpolate() finds them; the solver's own solution copy is not used."""
+    if mode not in ['nearest', 'continuous']:
+        raise ValueError("mode must be one of 'nearest', 'continuous'; got '%s'" % mode)
+    if mode == 'continuous' and r is None:
+        raise ValueError("r must be specified in mode='continuous'")
+    if diff is None:
+        raise ValueError("diff cannot be None")
+    if solver.tree is None:
+        raise RuntimeError("Points xi have not been indexed; prep_interpolate() must be called before interpolate()")
+    if I is not None and len(I) != len(x):
+        raise ValueError("When 'I' is specified, 'I' must have the same length as x; got len(I) = %d, len(x) = %d."
+                         % (len(I), len(x)))
+    all_diffs = isinstance(diff, str) and diff == 'all'
+    if mode == 'continuous' and all_diffs:
+        raise ValueError("diff='all' is not available in mode='continuous'")
+    cdiff = _lib.DIFF_ALL if all_diffs else int(diff)
+    fi_a, nf, fi_sf, fi_s0 = resolve_fi_read(fi, solver.ncases, solver._maxno)
+    fi_p = fi_a.ptr if nf else None
+    if mode == 'continuous':
+        x_a, x_s0, nx = opexport._points(solver, x)
+        I_c, I_out = None, np.asanyarray(None)
+    else:
+        x_a, x_s0, nx, I_c, I_out = opexport._queries(solver, x, I)
+    width = solver._maxno if all_diffs else 1
+    shape = (nf, nx, width) if all_diffs else (nf, nx)
+    if x_a.is_cuda:
+        import torch
+        out = torch.empty(shape, dtype=torch.float64, device=x_a.keep.device)
+        out_p = int(out.data_ptr())
+    else:
+        out = np.empty(shape, dtype=np.float64)
+        out_p = out.ctypes.data
+    out_sf, out_sq = nx * width, width
+    if mode == 'continuous':
+        solver._use_stream()                      # (opexport._queries sets it in nearest mode)
+        _lib.check(_lib.lib().wlsqm_solver_interpolate_continuous_fields(solver._handle, nf, fi_p, fi_sf, fi_s0,
+                                                                         x_a.ptr, x_s0, nx, float(r), cdiff, out_p,
+                                                                         out_sf, out_sq))
+        return out, I_out
+    # a query that found no neighbour (NaN coordinates) poisons the whole output (expert.pyx:862-870)
+    I_cuda = _lib._is_torch_tensor(I_c) and I_c.is_cuda
+    if not I_cuda and nx and (I_c == solver.ncases).any():
+        out[...] = np.nan
+        return out, I_out
+    I_p = int(I_c.data_ptr()) if I_cuda else I_c.ctypes.data
+    _lib.check(_lib.lib().wlsqm_solver_interpolate_fields(solver._handle, nf, fi_p, fi_sf, fi_s0, x_a.ptr, x_s0, I_p,
+                                                          nx, cdiff, out_p, out_sf, out_sq))
+    return out, I_out

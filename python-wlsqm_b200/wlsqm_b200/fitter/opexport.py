@@ -127,9 +127,8 @@ def operator(solver, coeffs, center=None):
     return (mats[0], K[0]) if squeeze else (mats, K)
 
 
-def _queries(solver, x, I):
-    """-> (x Arr, row stride, nx, int64 index array for the C ABI, I_out): the query points and their models, resolved
-    as ``interpolate(x, mode='nearest', I=I)`` resolves them (``solver._nearest_models``)."""
+def _points(solver, x):
+    """-> (x Arr, row stride, nx): the query points for the C ABI"""
     dim = solver.dimension
     x_a = _lib.as_arr(x, np.float64, 2 if dim >= 2 else 1, "x", last_contig=dim >= 2)
     nx = x_a.shape[0]
@@ -139,6 +138,13 @@ def _queries(solver, x, I):
     if not x_a.is_cuda and dim == 1 and nx > 1 and x_s0 != 1:
         x_a = _lib.as_arr(np.ascontiguousarray(x_a.np), np.float64, 1, "x", last_contig=False)
         x_s0 = 1
+    return x_a, x_s0, nx
+
+
+def _queries(solver, x, I):
+    """-> (x Arr, row stride, nx, int64 index array for the C ABI, I_out): the query points and their models, resolved
+    as ``interpolate(x, mode='nearest', I=I)`` resolves them (``solver._nearest_models``)."""
+    x_a, x_s0, nx = _points(solver, x)
     if I is None and solver.tree is None:
         raise RuntimeError("Points xi have not been indexed; prep_interpolate() must be called before the nearest models "
                            "can be found (or pass I)")

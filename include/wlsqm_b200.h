@@ -318,6 +318,61 @@ WLSQM_API int wlsqm_solver_nearest_models(wlsqm_solver_t* s, const double* x, in
 WLSQM_API int wlsqm_solver_interpolate_continuous(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
                                         int diff, double* out);
 
+/* Continuous-mode interpolation operators (extension): the linear map from the data to interpolate(x, mode='continuous',
+ * r, diff), the weighted average of every local model within r (expert.pyx:898-985), as rows per (query, model) pair and
+ * as a CSR matrix.  For query q with coordinates x[q]:
+ *   - Pairs.  The models of q are the origins xi[m] with d2(xi[m], x[q]) <= r*r under the ball rule of wlsqm_grid_ball_*
+ *     (every difference, square and sum rounded on its own, in axis order; the search runs over the solver's model grid
+ *     of wlsqm_solver_index_models).  Non-finite origins are never members; a query with a non-finite coordinate has no
+ *     models.  The pairs of a query are listed in ascending m -- the rows of cKDTree(xi).query_ball_point(x, r), sorted
+ *     -- and numbered query-major: pair_ptr int64 [nx + 1], J int64 [npairs] (the model of each pair).
+ *   - Weights.  Per pair, w = tmp * tmp with tmp = 1 - sqrt(d2 / (r*r)), the same rounded d2, every operation rounded on its
+ *     own (__ddiv_rn, __dsqrt_rn, __dsub_rn, __dmul_rn); per query S = the sum of w over its pairs in ascending m from +0,
+ *     separately rounded adds; alpha = w / S, one rounded division.
+ *   - Coefficient rows.  c_q^(m) is the nearest-mode row of wlsqm_solver_interp_stencils at offset h = x[q] - xi[m] (what
+ *     it forms for I[q] = m); the pair's row is c_qm[o][s] = alpha * c_q^(m)[o][s], one rounded multiply per entry.  The
+ *     pair's W [nops][npairs][max nk] and K [nops][npairs][max no] rows are EXACTLY the definitions of
+ *     wlsqm_solver_stencils for case m with c_qm in place of coeffs (ascending-slot FMA chain from 0, zero coefficients
+ *     skipped, c_qm[m] added last for known slots).
+ *   - CSR row q of E (nx x npoints, columns = points of prepare_hoods) holds, per column p, a sequential sum from +0 in the
+ *     order of the row's candidate list: the pairs of q in ascending m; within a pair the neighbours hoods[m][k] in
+ *     ascending k, then, with center (as for wlsqm_solver_operator_csr), the pair's known-F weight at column center + m,
+ *     which is then reported as 0 in K.  Columns strictly ascending, explicit zeros stored; the pattern depends on x, r,
+ *     hoods, knowns and center only and is shared by the nops operators; rowptr / col int32 (index_bits = 32,
+ *     nnz < 2^31) or int64, values [nops][nnz].  A row of at most 2048 candidate slots (pairs x (max nk + 1)) is merged
+ *     by one warp in shared memory; longer rows are sorted stably by column on the device, over chunks of queries of
+ *     bounded scratch, so rows of any length work and the call's total size is not limited.
+ * Then  sum_D coeffs[D] d^D f(x[q]) = (E f)[q] + sum over the pairs p of q of K[p] . fi[J[p]]  for an ALGO_BASIC solve, up
+ * to rounding against interpolate(x, mode='continuous', r, diff) after the solve.
+ *   - A query without a pair has an empty pair range and an empty E row (interpolate returns NaN there).  A query whose
+ *     only members lie at exactly r has S = 0 and NaN alpha: its W, K and E entries are NaN (interpolate's 0/0).
+ *   - Known difference: wlsqm_solver_interpolate_continuous may contract the sum of d2 into FMAs, so near |x - xi| = r it
+ *     can include or exclude a model that the ball rule decides the other way; such a model's weight is below about
+ *     2^-100 of a full weight.
+ *   - r > 0 (else WLSQM_E_VALUE); the solver must have been indexed (wlsqm_solver_index_models, else WLSQM_E_NOTREADY).
+ *   - The map is the ALGO_BASIC one for every solver and does not read the solution copy.  A guest answers with its host's
+ *     operators and neighbour lists and with its own model grid, as interpolate does.
+ *   - x [nx][dim] (row pitch x_s0) and every output may be host or device memory; host inputs are staged, and the calls
+ *     return when their outputs are written.  nx = 0 works (pair_ptr / rowptr = [0]).  One call handles up to 2^31 - 2
+ *     pairs (the limit of the ball search); for the CSR one query may hold up to 2^31 - 2 candidate slots and the columns
+ *     up to 2^32 - 2 points.
+ * wlsqm_solver_interp_continuous_count: pair_ptr (may be NULL), *npairs, and *nnz (may be NULL; counting it needs
+ *   prepare_hoods as the last prepare, else WLSQM_E_NOTREADY) for center.
+ * wlsqm_solver_interp_continuous_stencils: valid after any prepare; pair_ptr is the count call's for the same x and r
+ *   (a different one fails with WLSQM_E_VALUE, so nothing is written past pair_ptr[q + 1]); J [npairs] (may be NULL),
+ *   W, K (K may be NULL).
+ * wlsqm_solver_interp_continuous_operator_csr: as the stencils call for pair_ptr and J; recounts its pattern (like
+ *   wlsqm_solver_operator_csr) and returns rowptr [nx + 1], col, values and K per pair (may be NULL). */
+WLSQM_API int wlsqm_solver_interp_continuous_count(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
+                                                   int64_t center, int64_t* pair_ptr, int64_t* npairs, int64_t* nnz);
+WLSQM_API int wlsqm_solver_interp_continuous_stencils(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
+                                                      int nops, const double* coeffs, const int64_t* pair_ptr, int64_t* J,
+                                                      double* W, double* K);
+WLSQM_API int wlsqm_solver_interp_continuous_operator_csr(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx,
+                                                          double r, int nops, const double* coeffs, int64_t center,
+                                                          int index_bits, const int64_t* pair_ptr, int64_t* J, void* rowptr,
+                                                          void* col, double* values, double* K);
+
 /* Several fields on one geometry (extension): evaluate caller-held solutions, e.g. the fi written by
  * wlsqm_solver_solve_fields, at query points.  Field j of out is BIT FOR BIT what wlsqm_solver_interpolate (or
  * _interpolate_continuous) writes for the same x, I, diff (and r) when the solver's solution copy holds fi[j][i][0..no_i)

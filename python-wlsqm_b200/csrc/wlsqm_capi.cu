@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <new>
 #include <string>
@@ -1901,9 +1902,11 @@ static int opx_points(wlsqm_solver_t* s, const double* x, int64_t x_s0, long lon
     return WLSQM_OK;
 }
 
-// W [nops][nx][maxnk], K [nops][nx][maxno] (or NULL), kf [nops][nx] (or NULL) of the queries: device pointers
+// W [nops][nx][maxnk], K [nops][nx][maxno] (or NULL), kf [nops][nx] (or NULL) of the queries: device pointers.
+// Continuous mode: the nx rows are pairs, row p at query row_query[p] with its coefficient rows scaled by row_scale[p].
 static int opx_interp(wlsqm_solver_t* s, const double* xd, long long xs, const long long* Id, long long nx, int nops,
-                      const double* coeffs, double* W, double* K, double* kf) {
+                      const double* coeffs, double* W, double* K, double* kf, const int* row_query = nullptr,
+                      const double* row_scale = nullptr) {
     const wlsqm_solver* r = s->lender ? s->lender : s;
     if (s->lender) CU(order_streams(r->stream, s->stream));   // the host's prepare may still be in flight
     const int maxno = s->maxno;
@@ -1926,7 +1929,7 @@ static int opx_interp(wlsqm_solver_t* s, const double* xd, long long xs, const l
     P.nmodels = s->ncases; P.op = r->op; P.xi = r->xi_dev; P.x = xd; P.x_s0 = xs; P.dim = s->dim; P.nx = nx;
     P.run_case = R.run_case; P.run_len = R.run_len; P.run_off = R.run_off; P.nruns = R.nruns; P.perm = R.perm;
     P.coef = (const double*)s->opx_coef.p; P.nops = nops; P.maxnk = s->maxnk; P.maxno = maxno;
-    P.W = W; P.K = K; P.kf = kf;
+    P.W = W; P.K = K; P.kf = kf; P.row_query = row_query; P.row_scale = row_scale;
     // the ring of stencil_kernel, plus per warp the coefficient rows of one query (all nops operators, or fewer per pass
     // when shared memory is short) and its Taylor terms
     P.stage_doubles = std::max(2, even(s->maxnq * s->maxnr));
@@ -2123,6 +2126,369 @@ int wlsqm_solver_interpolate_continuous(wlsqm_solver_t* s, const double* x, int6
     CU(launch_interpolate_continuous(P, grid_view(s->models_grid), r, st));
     if (!out_dev) CU(cudaMemcpyAsync(out, s->st_out.p, (size_t)nx * 8, cudaMemcpyDeviceToHost, st));
     if (!x_dev || !out_dev) CU(cudaStreamSynchronize(st));
+    return WLSQM_OK;
+}
+
+// ---- continuous-mode interpolation operators (wlsqm_operator.cu) --------------------------------------------------
+// The pairs (q, m) of the models within r come from the ball search over the solver's own model grid (the grid of
+// interpolate(mode='continuous')); operators and neighbour lists are the lender's.
+static int cont_check(wlsqm_solver_t* s, long long nx, double r) {
+    if (!s) return fail(WLSQM_E_VALUE, "NULL solver");
+    const wlsqm_solver* rt = s->lender ? s->lender : s;
+    if (!rt->ready) return fail(WLSQM_E_NOTREADY, "Solver is not in the ready state; prepare() must be called first");
+    if (!s->models_grid) return fail(WLSQM_E_NOTREADY, "Points xi have not been indexed; prep_interpolate() must be called before interpolate()");
+    if (!(r > 0.0)) return fail(WLSQM_E_VALUE, "r must be positive");
+    if (nx < 0) return fail(WLSQM_E_VALUE, "nx must be >= 0, got %lld", nx);
+    if (nx >= (1LL << 31) - 1) return fail(WLSQM_E_VALUE, "the interpolation operators support up to 2^31 - 2 queries");
+    return WLSQM_OK;
+}
+
+// pp: pair_ptr [nx + 1] (device); models: J [npairs] (int64, device), the query pq and the weight alpha of each pair
+struct ContPairs {
+    DevBuf pp, j32, pq, alpha;
+    long long npairs = 0;
+};
+
+// pair_ptr of the queries xd (device, row pitch xs); the ball search returns when its outputs are written
+static int cont_count(wlsqm_solver_t* s, const double* xd, long long xs, long long nx, double r, ContPairs& C) {
+    int rc = C.pp.reserve((size_t)(nx + 1) * 8);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(s->stream));     // staged queries, earlier work on the solver's stream
+    int64_t np = 0;
+    rc = wlsqm_grid_ball_count(s->models_grid, xd, xs, nx, &r, 0, 0, 0, (int64_t*)C.pp.p, nullptr, &np);
+    if (rc) return rc;
+    C.npairs = np;
+    return WLSQM_OK;
+}
+
+// the models of the pairs (ascending per query) -> Jd [npairs], and their queries and weights
+static int cont_models(wlsqm_solver_t* s, const double* xd, long long xs, long long nx, double r, ContPairs& C, long long* Jd) {
+    const long long np = C.npairs;
+    if (np >= (1LL << 31) - 1) return fail(WLSQM_E_VALUE, "%lld pairs in one call exceed 2^31 - 2: split the queries", np);
+    int rc = C.j32.reserve((size_t)std::max(np, 1LL) * 4);
+    if (!rc) rc = C.pq.reserve((size_t)std::max(np, 1LL) * 4);
+    if (!rc) rc = C.alpha.reserve((size_t)std::max(np, 1LL) * 8);
+    if (rc) return rc;
+    rc = wlsqm_grid_ball_csr(s->models_grid, xd, xs, nx, &r, 0, 0, 0, WLSQM_BALL_BY_INDEX, (const int64_t*)C.pp.p,
+                             (int32_t*)C.j32.p);
+    if (rc) return rc;
+    CU(launch_cont_weights(xd, xs, s->dim, s->xi_dev, nx, r, (const long long*)C.pp.p, (const int32_t*)C.j32.p, Jd,
+                           (int*)C.pq.p, (double*)C.alpha.p, s->stream));
+    return WLSQM_OK;
+}
+
+// the caller's pair_ptr must be the one of wlsqm_solver_interp_continuous_count for the same x and r
+static int cont_same_ptr(wlsqm_solver_t* s, const int64_t* pair_ptr, const ContPairs& C, long long nx) {
+    DevBuf staged, flag;
+    const long long* pd = (const long long*)pair_ptr;
+    int rc = flag.reserve(4);
+    if (!rc && !is_device_ptr(pair_ptr)) {
+        rc = staged.reserve((size_t)(nx + 1) * 8);
+        if (!rc) pd = (const long long*)staged.p;
+    }
+    if (rc) return rc;
+    int bad = 0;
+    cudaError_t e = cudaSuccess;
+    if (pd != (const long long*)pair_ptr) e = cudaMemcpyAsync(staged.p, pair_ptr, (size_t)(nx + 1) * 8, cudaMemcpyHostToDevice, s->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(flag.p, 0, 4, s->stream);
+    if (e == cudaSuccess) e = launch_ptr_mismatch(pd, (const long long*)C.pp.p, nx + 1, (int*)flag.p, s->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&bad, flag.p, 4, cudaMemcpyDeviceToHost, s->stream);
+    const cudaError_t e2 = cudaStreamSynchronize(s->stream);
+    staged.release(); flag.release();
+    if (e == cudaSuccess) e = e2;
+    if (e != cudaSuccess) return fail(WLSQM_E_CUDA, "pair_ptr: %s", cudaGetErrorString(e));
+    if (bad) return fail(WLSQM_E_VALUE, "pair_ptr does not match the pairs of x and r (wlsqm_solver_interp_continuous_count)");
+    return WLSQM_OK;
+}
+
+// The CSR pattern over the pairs and its fill.  Rows of at most row_cap candidate slots (max nk + 1 per pair) are merged
+// by one warp in shared memory; longer rows by the sort route, over chunks of consecutive queries of at most
+// WLSQM_CONT_CHUNK_SLOTS slots (default 2^26; a single longer row is one chunk), so that the scratch stays bounded and no
+// call is refused for its total size.  WLSQM_CONT_ROW_CAP (default 2048, rounded up to a power of two; 0: every row
+// takes the sort route) sets row_cap.
+struct ContPattern {
+    DevBuf cnt, rp, seg, keys, cand, keys_s, cand_s, head, hpos, tmp;
+    std::vector<long long> hp;      // pair_ptr on the host
+    long long chunk_slots = 0;
+};
+
+// the chunks of the sort route: each [q0, q1) starts at a long row; fn(q0, q1) runs one
+static int cont_chunks(const ContCsrParams& P, const ContPattern& B, const std::function<int(long long, long long)>& fn) {
+    const long long nx = P.nx, L = P.L;
+    long long q0 = 0;
+    for (;;) {
+        while (q0 < nx && (B.hp[q0 + 1] - B.hp[q0]) * L <= P.row_cap) ++q0;
+        if (q0 >= nx) return WLSQM_OK;
+        long long q1 = q0 + 1;
+        while (q1 < nx && (B.hp[q1 + 1] - B.hp[q0]) * L <= B.chunk_slots) ++q1;
+        const int rc = fn(q0, q1);
+        if (rc) return rc;
+        q0 = q1;
+    }
+}
+
+static int cont_chunk_run(wlsqm_solver_t* s, ContCsrParams& P, ContPattern& B, long long q0, long long q1, bool fill,
+                          int index_bits) {
+    P.q0 = q0; P.q1 = q1; P.slot0 = B.hp[q0] * P.L; P.nslots = (B.hp[q1] - B.hp[q0]) * P.L;
+    CU(cont_long_rows(P, fill, index_bits, B.tmp.p, &B.tmp.cap, s->stream));
+    return WLSQM_OK;
+}
+
+// count pass: the row counts and their scan (B.rp, nnz on the host); P is ready for the fill afterwards
+static int cont_pattern(wlsqm_solver_t* s, const ContPairs& C, long long nx, int64_t center, const long long* Jd,
+                        ContPattern& B, ContCsrParams& P, long long* nnz) {
+    const wlsqm_solver* r = s->lender ? s->lender : s;
+    if (s->lender) CU(order_streams(r->stream, s->stream));
+    if (r->hood_points > (long long)CONT_NO_COLUMN - 1)
+        return fail(WLSQM_E_VALUE, "the continuous-mode operator supports up to 2^32 - 2 points, got %lld", r->hood_points);
+    const long long L = r->maxnk + 1;
+    B.hp.assign(nx + 1, 0);
+    CU(cudaMemcpyAsync(B.hp.data(), C.pp.p, (size_t)(nx + 1) * 8, cudaMemcpyDeviceToHost, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    long long maxrow = 0;
+    for (long long q = 0; q < nx; ++q) maxrow = std::max(maxrow, (B.hp[q + 1] - B.hp[q]) * L);
+    if (maxrow >= (1LL << 31) - 1)
+        return fail(WLSQM_E_VALUE, "one query has %lld candidate slots (pairs x (max nk + 1)); at most 2^31 - 2 are supported", maxrow);
+    const int cap_env = env_int("WLSQM_CONT_ROW_CAP", 2048);
+    int row_cap = 0;
+    if (cap_env > 0) {
+        row_cap = 32;
+        while (row_cap < cap_env && row_cap < maxrow) row_cap <<= 1;
+    }
+    B.chunk_slots = std::max<long long>(std::max(env_int("WLSQM_CONT_CHUNK_SLOTS", 1 << 26), 1), maxrow);
+    int rc = B.cnt.reserve((size_t)(nx + 1) * 8);
+    if (!rc) rc = B.rp.reserve((size_t)(nx + 1) * 8);
+    if (rc) return rc;
+    P.meta = r->dmeta; P.uni = r->uni; P.nx = nx; P.npairs = C.npairs; P.pair_ptr = (const long long*)C.pp.p; P.J = Jd;
+    P.pair_query = (const int*)C.pq.p; P.hoods = (const int32_t*)r->hoods_dev.p; P.hoods_s0 = r->maxnk; P.center = center;
+    P.L = (int)L; P.maxnk = r->maxnk; P.row_cap = row_cap; P.cnt = (long long*)B.cnt.p; P.rp = (const long long*)B.rp.p;
+    CU(cudaMemsetAsync(B.cnt.p, 0, (size_t)(nx + 1) * 8, s->stream));
+    CU(launch_cont_rows(P, false, 32, s->stream));
+    if (maxrow > row_cap) {
+        // scratch for the largest chunk
+        long long slots = 0, nseg = 0;
+        cont_chunks(P, B, [&](long long q0, long long q1) {
+            slots = std::max(slots, (B.hp[q1] - B.hp[q0]) * L);
+            nseg = std::max(nseg, q1 - q0);
+            return WLSQM_OK;
+        });
+        rc = B.seg.reserve((size_t)(nseg + 1) * 4);
+        if (!rc) rc = B.keys.reserve((size_t)slots * 4);
+        if (!rc) rc = B.keys_s.reserve((size_t)slots * 4);
+        if (!rc) rc = B.cand.reserve((size_t)slots * 4);
+        if (!rc) rc = B.cand_s.reserve((size_t)slots * 4);
+        if (!rc) rc = B.head.reserve((size_t)(slots + 1) * 4);
+        if (!rc) rc = B.hpos.reserve((size_t)(slots + 1) * 4);
+        if (rc) return rc;
+        P.seg = (int*)B.seg.p; P.keys = (unsigned*)B.keys.p; P.cand = (int*)B.cand.p;
+        P.keys_sorted = (const unsigned*)B.keys_s.p; P.cand_sorted = (const int*)B.cand_s.p;
+        P.head = (int*)B.head.p; P.hpos = (const int*)B.hpos.p;
+        P.q0 = 0; P.q1 = nseg; P.nslots = slots;
+        size_t tb = 0;
+        CU(cont_long_rows(P, false, 32, nullptr, &tb, s->stream));
+        rc = B.tmp.reserve(tb + 16);
+        if (!rc) rc = cont_chunks(P, B, [&](long long q0, long long q1) { return cont_chunk_run(s, P, B, q0, q1, false, 32); });
+        if (rc) return rc;
+    }
+    size_t tb = 0;
+    CU(csr_scan((long long*)B.cnt.p, (long long*)B.rp.p, nx + 1, nullptr, &tb, s->stream));
+    DevBuf tmp;
+    rc = tmp.reserve(tb + 16);
+    if (rc) return rc;
+    tb += 16;
+    long long total = 0;
+    cudaError_t e = csr_scan((long long*)B.cnt.p, (long long*)B.rp.p, nx + 1, tmp.p, &tb, s->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(&total, (const long long*)B.rp.p + nx, 8, cudaMemcpyDeviceToHost, s->stream);
+    const cudaError_t e2 = cudaStreamSynchronize(s->stream);
+    tmp.release();
+    if (e == cudaSuccess) e = e2;
+    if (e != cudaSuccess) return fail(WLSQM_E_CUDA, "continuous operator pattern: %s", cudaGetErrorString(e));
+    P.nnz = total;
+    *nnz = total;
+    return WLSQM_OK;
+}
+
+// fill pass after cont_pattern: rowptr, the short rows, then the chunks of the sort route
+static int cont_fill(wlsqm_solver_t* s, ContCsrParams& P, ContPattern& B, int index_bits) {
+    CU(launch_cont_rows(P, true, index_bits, s->stream));
+    if (!B.tmp.p) return WLSQM_OK;
+    return cont_chunks(P, B, [&](long long q0, long long q1) { return cont_chunk_run(s, P, B, q0, q1, true, index_bits); });
+}
+
+// rowptr = [0] for nx = 0
+static int cont_empty_rowptr(void* rowptr, size_t ib) {
+    const long long z = 0;
+    if (is_device_ptr(rowptr)) CU(cudaMemcpy(rowptr, &z, ib, cudaMemcpyHostToDevice));
+    else memcpy(rowptr, &z, ib);
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_interp_continuous_count(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
+                                         int64_t center, int64_t* pair_ptr, int64_t* npairs, int64_t* nnz) {
+    if (!npairs) return fail(WLSQM_E_VALUE, "npairs must not be NULL");
+    *npairs = 0;
+    if (nnz) *nnz = 0;
+    int rc = cont_check(s, nx, r);
+    if (rc) return rc;
+    if (nnz) {
+        const wlsqm_solver* rt = s->lender ? s->lender : s;
+        if (!rt->hoods_current)
+            return fail(WLSQM_E_NOTREADY, "the global operator needs the neighbour lists of prepare_hoods() as the last prepare");
+        rc = opx_center(s, center);
+        if (rc) return rc;
+    }
+    if (nx == 0) return pair_ptr ? cont_empty_rowptr(pair_ptr, 8) : WLSQM_OK;
+    rc = use_device(s);
+    if (rc) return rc;
+    const double* xd;
+    long long xs;
+    rc = opx_points(s, x, x_s0, nx, &xd, &xs);
+    if (rc) return rc;
+    ContPairs C;
+    ContPattern B;
+    DevBuf Jd;
+    struct Release {
+        wlsqm_solver_t* s; DevBuf* b[12];
+        ~Release() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release{s, {&C.pp, &C.j32, &C.pq, &C.alpha, &B.seg, &B.keys, &B.cand, &B.keys_s, &B.cand_s, &B.head, &B.hpos, &Jd}};
+    struct ReleaseMore {
+        wlsqm_solver_t* s; DevBuf* b[3];
+        ~ReleaseMore() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release_more{s, {&B.cnt, &B.rp, &B.tmp}};
+    rc = cont_count(s, xd, xs, nx, r, C);
+    if (rc) return rc;
+    long long total = 0;
+    if (nnz) {
+        rc = Jd.reserve((size_t)std::max(C.npairs, 1LL) * 8);
+        if (!rc) rc = cont_models(s, xd, xs, nx, r, C, (long long*)Jd.p);
+        ContCsrParams P{};
+        if (!rc) rc = cont_pattern(s, C, nx, center, (const long long*)Jd.p, B, P, &total);
+        if (rc) return rc;
+    }
+    if (pair_ptr) CU(cudaMemcpyAsync(pair_ptr, C.pp.p, (size_t)(nx + 1) * 8, cudaMemcpyDefault, s->stream));
+    CU(cudaStreamSynchronize(s->stream));
+    *npairs = C.npairs;
+    if (nnz) *nnz = total;
+    return WLSQM_OK;
+}
+
+// the pairs of x and r after the caller's pair_ptr has been checked, W / K / kf of the pairs, and J in Jd
+static int cont_rows(wlsqm_solver_t* s, const double* xd, long long xs, long long nx, double r, const int64_t* pair_ptr,
+                     int nops, const double* coeffs, ContPairs& C, DevBuf& sj, int64_t* J, void** Jd, double* W, double* K,
+                     double* kf) {
+    int rc = cont_same_ptr(s, pair_ptr, C, nx);
+    if (rc) return rc;
+    rc = opx_out(J, (size_t)C.npairs * 8, sj, Jd);
+    if (!rc && !*Jd) {
+        rc = sj.reserve((size_t)std::max(C.npairs, 1LL) * 8);
+        *Jd = sj.p;
+    }
+    if (!rc) rc = cont_models(s, xd, xs, nx, r, C, (long long*)*Jd);
+    if (!rc && C.npairs)
+        rc = opx_interp(s, xd, xs, (const long long*)*Jd, C.npairs, nops, coeffs, W, K, kf, (const int*)C.pq.p,
+                        (const double*)C.alpha.p);
+    return rc;
+}
+
+int wlsqm_solver_interp_continuous_stencils(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r, int nops,
+                                            const double* coeffs, const int64_t* pair_ptr, int64_t* J, double* W, double* K) {
+    int rc = opx_check(s, nops, coeffs, false);
+    if (!rc) rc = cont_check(s, nx, r);
+    if (rc) return rc;
+    if (!pair_ptr) return fail(WLSQM_E_VALUE, "pair_ptr must not be NULL");
+    if (nx == 0) return WLSQM_OK;
+    const double* xd;
+    long long xs;
+    rc = opx_points(s, x, x_s0, nx, &xd, &xs);
+    if (rc) return rc;
+    ContPairs C;
+    DevBuf sj, sw, sk;
+    struct Release {
+        wlsqm_solver_t* s; DevBuf* b[7];
+        ~Release() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release{s, {&C.pp, &C.j32, &C.pq, &C.alpha, &sj, &sw, &sk}};
+    rc = cont_count(s, xd, xs, nx, r, C);
+    if (rc) return rc;
+    const long long np = C.npairs;
+    if (np > 0 && !W) return fail(WLSQM_E_VALUE, "W must not be NULL");
+    const size_t wb = (size_t)nops * np * s->maxnk * 8, kb = (size_t)nops * np * s->maxno * 8;
+    void *Jd, *Wd, *Kd;
+    rc = opx_out(np ? W : nullptr, wb, sw, &Wd);
+    if (!rc) rc = opx_out(np ? K : nullptr, kb, sk, &Kd);
+    if (!rc) rc = cont_rows(s, xd, xs, nx, r, pair_ptr, nops, coeffs, C, sj, J, &Jd, (double*)Wd, (double*)Kd, nullptr);
+    if (!rc && np) rc = opx_copy_out(W, Wd, wb, s->stream);
+    if (!rc && np && K) rc = opx_copy_out(K, Kd, kb, s->stream);
+    if (!rc && np && J) rc = opx_copy_out(J, Jd, (size_t)np * 8, s->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(s->stream));
+    return WLSQM_OK;
+}
+
+int wlsqm_solver_interp_continuous_operator_csr(wlsqm_solver_t* s, const double* x, int64_t x_s0, int64_t nx, double r,
+                                                int nops, const double* coeffs, int64_t center, int index_bits,
+                                                const int64_t* pair_ptr, int64_t* J, void* rowptr, void* col, double* values,
+                                                double* K) {
+    int rc = opx_check(s, nops, coeffs, true);
+    if (!rc) rc = opx_center(s, center);
+    if (!rc) rc = cont_check(s, nx, r);
+    if (rc) return rc;
+    if (index_bits != 32 && index_bits != 64) return fail(WLSQM_E_VALUE, "index_bits must be 32 or 64, got %d", index_bits);
+    if (!rowptr) return fail(WLSQM_E_VALUE, "rowptr must not be NULL");
+    if (!pair_ptr) return fail(WLSQM_E_VALUE, "pair_ptr must not be NULL");
+    const size_t ib = index_bits / 8;
+    if (nx == 0) return cont_empty_rowptr(rowptr, ib);
+    const double* xd;
+    long long xs;
+    rc = opx_points(s, x, x_s0, nx, &xd, &xs);
+    if (rc) return rc;
+    ContPairs C;
+    ContPattern B;
+    DevBuf sj, wtmp, kf, s_rp, s_col, s_val, s_k;
+    struct Release {
+        wlsqm_solver_t* s; DevBuf* b[18];
+        ~Release() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release{s, {&C.pp, &C.j32, &C.pq, &C.alpha, &B.seg, &B.keys, &B.cand, &B.keys_s, &B.cand_s, &B.head, &B.hpos, &sj,
+                  &wtmp, &kf, &s_rp, &s_col, &s_val, &s_k}};
+    struct ReleaseMore {
+        wlsqm_solver_t* s; DevBuf* b[3];
+        ~ReleaseMore() { cudaStreamSynchronize(s->stream); for (DevBuf* d : b) d->release(); }
+    } release_more{s, {&B.cnt, &B.rp, &B.tmp}};
+    rc = cont_count(s, xd, xs, nx, r, C);
+    if (rc) return rc;
+    const long long np = C.npairs;
+    rc = wtmp.reserve((size_t)nops * std::max(np, 1LL) * std::max(s->maxnk, 1) * 8);
+    if (!rc && center >= 0) rc = kf.reserve((size_t)nops * std::max(np, 1LL) * 8);
+    if (rc) return rc;
+    const size_t kb = (size_t)nops * np * s->maxno * 8;
+    void *Jd, *kd;
+    rc = opx_out(np ? K : nullptr, kb, s_k, &kd);
+    if (!rc) rc = cont_rows(s, xd, xs, nx, r, pair_ptr, nops, coeffs, C, sj, J, &Jd, (double*)wtmp.p, (double*)kd,
+                            center >= 0 ? (double*)kf.p : nullptr);
+    if (rc) return rc;
+    ContCsrParams P{};
+    long long nnz = 0;
+    rc = cont_pattern(s, C, nx, center, (const long long*)Jd, B, P, &nnz);
+    if (rc) return rc;
+    if (index_bits == 32 && nnz >= (1LL << 31))
+        return fail(WLSQM_E_VALUE, "nnz = %lld does not fit 32-bit indices; use index_bits = 64", nnz);
+    if (nnz > 0 && (!col || !values)) return fail(WLSQM_E_VALUE, "col and values must not be NULL");
+    const size_t rb = (size_t)(nx + 1) * ib, cb = (size_t)nnz * ib, vb = (size_t)nops * nnz * 8;
+    void *rpd, *cd, *vd;
+    rc = opx_out(rowptr, rb, s_rp, &rpd);
+    if (!rc) rc = opx_out(nnz ? col : nullptr, cb, s_col, &cd);
+    if (!rc) rc = opx_out(nnz ? values : nullptr, vb, s_val, &vd);
+    if (rc) return rc;
+    P.W = (const double*)wtmp.p; P.kf = (const double*)kf.p; P.nops = nops;
+    P.rowptr = rpd; P.col = cd; P.values = (double*)vd;
+    rc = cont_fill(s, P, B, index_bits);
+    if (rc) return rc;
+    rc = opx_copy_out(rowptr, rpd, rb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(col, cd, cb, s->stream);
+    if (!rc && nnz) rc = opx_copy_out(values, vd, vb, s->stream);
+    if (!rc && np && K) rc = opx_copy_out(K, kd, kb, s->stream);
+    if (!rc && np && J) rc = opx_copy_out(J, Jd, (size_t)np * 8, s->stream);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(s->stream));
     return WLSQM_OK;
 }
 

@@ -161,6 +161,42 @@ struct InterpStencilParams {
     double* K;                                       // [nops][nx][maxno] or nullptr
     double* kf;                                      // [nops][nx] known-F weight for centre folding, or nullptr
     int stages, stage_doubles, ring_off, cq_off, cq_doubles, bar_off_bytes;
+    // continuous mode: the rows are the (query, model) pairs (nx of them, I = J), row p is evaluated at query
+    // row_query[p] and its coefficient rows are scaled by row_scale[p]; nullptr in nearest mode
+    const int* row_query;
+    const double* row_scale;
+};
+
+// continuous-mode interpolation operators (wlsqm_operator.cu): per query the pairs (q, m) of the models within r, in
+// ascending m (pair_ptr [nx + 1], J [npairs] from the ball search over the model grid); per pair the normalised weight
+// alpha and its query.  The CSR rows merge the candidates of each query's pairs: L = maxnk + 1 slots per pair
+// (neighbours k < nk_m, then the folded known F), slot order = candidate order.  Rows of at most row_cap slots are
+// sorted by one warp in shared memory (cont_row_kernel); longer rows by cub's segmented sort over chunks of queries.
+constexpr int CONT_ROW_WARPS = 8;
+constexpr unsigned CONT_NO_COLUMN = 0xffffffffu;
+struct ContCsrParams {
+    const CaseMeta* meta;
+    CaseMeta uni;
+    long long nx, npairs;
+    const long long* pair_ptr;                       // [nx + 1]
+    const long long* J;                              // [npairs]
+    const int* pair_query;                           // [npairs]
+    const int32_t* hoods; int hoods_s0;
+    long long center;
+    int L;                                           // maxnk + 1 candidate slots per pair
+    int row_cap;                                     // rows of at most row_cap slots: cont_row_kernel (a power of two, or 0)
+    long long* cnt;                                  // count: distinct columns of each row [nx + 1]
+    const long long* rp;                             // fill: exclusive scan of cnt
+    // sort route, one chunk: queries [q0, q1), slots [slot0, slot0 + nslots)
+    long long q0, q1, slot0, nslots;
+    int* seg;                                        // [q1 - q0 + 1] first chunk slot of each query
+    unsigned* keys; int* cand;                       // [nslots] column (or CONT_NO_COLUMN), chunk slot
+    const unsigned* keys_sorted; const int* cand_sorted;
+    int* head;                                       // [nslots + 1]: 1 at the first slot of each (query, column) run
+    const int* hpos;                                 // exclusive scan of head
+    const double* W; const double* kf; int nops, maxnk;
+    void* rowptr; void* col; double* values;
+    long long nnz;
 };
 
 #ifdef __CUDACC__
@@ -285,6 +321,12 @@ cudaError_t launch_csr_fill(const CsrParams& P, int index_bits, cudaStream_t st)
 cudaError_t interp_runs(const long long* I, long long nx, long long nmodels, const InterpRuns& R, void* tmp, size_t* tmp_bytes,
                         cudaStream_t st);
 cudaError_t launch_interp_stencils(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st);
+cudaError_t launch_cont_weights(const double* x, long long x_s0, int dim, const double* xi, long long nx, double r,
+                                const long long* pair_ptr, const int32_t* J32, long long* J, int* pair_query, double* alpha,
+                                cudaStream_t st);
+cudaError_t launch_ptr_mismatch(const long long* a, const long long* b, long long n, int* flag, cudaStream_t st);
+cudaError_t launch_cont_rows(const ContCsrParams& P, bool fill, int index_bits, cudaStream_t st);
+cudaError_t cont_long_rows(const ContCsrParams& P, bool fill, int index_bits, void* tmp, size_t* tmp_bytes, cudaStream_t st);
 struct GridView;
 cudaError_t launch_interpolate_continuous(const InterpParams& P, const GridView& g, double r, cudaStream_t st);
 int interp_fields_per_pass(long long nf, long long ncases, int maxno, long long nx, double rows_per_query,

@@ -23,6 +23,11 @@
 // queries are sorted stably by I (cub radix sort of 32-bit keys, run-length encoding, scan); interp_stencil_kernel
 // takes one run per warp, streams the model's block once through the ring of stencil_kernel and writes each query's
 // rows at the query's own position through the same contract_case.  csr_kernel<., ., true> maps row q to case I[q].
+//
+// Continuous mode (DESIGN.md §4 K6c): the rows are the (query, model) pairs of the models within r (the ball search over
+// the model grid), each the nearest-mode row scaled by the pair's normalised weight (cont_weights_kernel,
+// interp_stencil_kernel<., true>).  A query's CSR row merges its pairs' candidates: one warp sorts a short row in shared
+// memory (cont_row_kernel); longer rows take a stable segmented sort over chunks of queries.
 #include <cub/cub.cuh>
 #include "wlsqm_common.cuh"
 #include "wlsqm_kernels.h"
@@ -167,7 +172,10 @@ __constant__ SlotExpTable c_slot_exp = make_slot_exp_table();
 // the Taylor terms of the offset h = x[q] - xi[m] per axis (st = steps_of(h)), and contract them with the block
 // (contract_case) into row q.  A term with T_D(s) = 0 is not added: the sum starts at +0 and never becomes -0, so
 // adding +-0 changes nothing.  Runs of the index nmodels (I outside [0, nmodels)): W row 0, K row NaN.
-template <bool UNI>
+// PAIRS (continuous mode): the rows are (query, model) pairs; row p takes its offset from query row_query[p] and its
+// coefficient rows are c_qm = alpha * c_q with alpha = row_scale[p] (one rounded multiply per entry).  A separate
+// instantiation, so that the nearest-mode kernels are unchanged.
+template <bool UNI, bool PAIRS>
 __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(InterpStencilParams P) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
@@ -224,8 +232,9 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
             const CaseMeta m = case_meta<UNI>(P.meta, P.uni, P.op_stride, c);
             for (int t = 0; t < nq; ++t) {
                 const long long q = P.perm[q0 + t];
+                const long long xq = PAIRS ? (long long)P.row_query[q] : q;
                 if (lane < 3) {     // Taylor terms of axis `lane` (h = 0 beyond the dimension: 1, 0, 0, 0, 0)
-                    const double h = lane < dim ? P.x[q * P.x_s0 + lane] - P.xi[c * dim + lane] : 0.0;
+                    const double h = lane < dim ? P.x[xq * P.x_s0 + lane] - P.xi[c * dim + lane] : 0.0;
                     const Steps st = steps_of(h);
                     double tv = 1.0;
                     tt[lane * 5] = tv;
@@ -251,7 +260,7 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
                                 acc = __dadd_rn(acc, __dmul_rn(co[D], T));
                             }
                         }
-                        cq[idx] = acc;
+                        cq[idx] = PAIRS ? __dmul_rn(P.row_scale[q], acc) : acc;
                     }
                     __syncwarp();
                     for (int o = 0; o < oc; ++o) {
@@ -270,19 +279,286 @@ __global__ void __launch_bounds__(OPX_MAX_THREADS, 1) interp_stencil_kernel(Inte
     }
 }
 
+template <bool UNI, bool PAIRS>
+static cudaError_t launch_interp_stencils_t(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st) {
+    const cudaError_t e = cudaFuncSetAttribute(interp_stencil_kernel<UNI, PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    interp_stencil_kernel<UNI, PAIRS><<<blocks, threads, smem, st>>>(P);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_interp_stencils(const InterpStencilParams& P, int blocks, int threads, size_t smem, cudaStream_t st) {
     const bool uni = P.meta == nullptr || P.geom_uniform;
-    cudaError_t e;
-    if (uni) {
-        e = cudaFuncSetAttribute(interp_stencil_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        interp_stencil_kernel<true><<<blocks, threads, smem, st>>>(P);
-    } else {
-        e = cudaFuncSetAttribute(interp_stencil_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        interp_stencil_kernel<false><<<blocks, threads, smem, st>>>(P);
+    if (P.row_query)
+        return uni ? launch_interp_stencils_t<true, true>(P, blocks, threads, smem, st)
+                   : launch_interp_stencils_t<false, true>(P, blocks, threads, smem, st);
+    return uni ? launch_interp_stencils_t<true, false>(P, blocks, threads, smem, st)
+               : launch_interp_stencils_t<false, false>(P, blocks, threads, smem, st);
+}
+
+// ---- continuous-mode interpolation operators --------------------------------------------------------------------
+// Per query q (one thread): its pairs p in [pair_ptr[q], pair_ptr[q+1]) (models J32[p], ascending), d2 recomputed by the
+// ball rule of wlsqm_grid_ball_* (xi - x per axis, square, sum in axis order, each rounded on its own), the weight
+// w = (1 - sqrt(d2 / r2))^2 with every operation rounded on its own, S = the sum of w in pair order from +0, and
+// alpha[p] = w / S (NaN when S = 0: every member at exactly r).  Also widens J and records each pair's query.
+template <int DIM>
+__global__ void cont_weights_kernel(const double* __restrict__ x, long long x_s0, const double* __restrict__ xi,
+                                    long long nx, double r, const long long* __restrict__ pair_ptr,
+                                    const int32_t* __restrict__ J32, long long* __restrict__ J, int* __restrict__ pair_query,
+                                    double* __restrict__ alpha) {
+    const double r2 = __dmul_rn(r, r);
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < nx; q += (long long)gridDim.x * blockDim.x) {
+        const long long p0 = pair_ptr[q], p1 = pair_ptr[q + 1];
+        double xq[DIM];
+#pragma unroll
+        for (int d = 0; d < DIM; ++d) xq[d] = x[q * x_s0 + d];
+        double S = 0.0;
+        for (long long p = p0; p < p1; ++p) {
+            const long long m = J32[p];
+            double d2 = 0.0;
+#pragma unroll
+            for (int d = 0; d < DIM; ++d) {
+                const double dd = __dsub_rn(xi[m * DIM + d], xq[d]);
+                d2 = __dadd_rn(d2, __dmul_rn(dd, dd));
+            }
+            const double tmp = __dsub_rn(1.0, __dsqrt_rn(__ddiv_rn(d2, r2)));
+            const double w = __dmul_rn(tmp, tmp);
+            S = __dadd_rn(S, w);
+            alpha[p] = w;
+            J[p] = m;
+            pair_query[p] = (int)q;
+        }
+        for (long long p = p0; p < p1; ++p) alpha[p] = __ddiv_rn(alpha[p], S);
     }
+}
+
+static unsigned grid_for(long long n, int threads) {
+    return (unsigned)std::max<long long>(1, std::min<long long>((n + threads - 1) / threads, 148LL * 32));
+}
+
+cudaError_t launch_cont_weights(const double* x, long long x_s0, int dim, const double* xi, long long nx, double r,
+                                const long long* pair_ptr, const int32_t* J32, long long* J, int* pair_query, double* alpha,
+                                cudaStream_t st) {
+    const unsigned b = grid_for(nx, 128);
+    if (dim == 1) cont_weights_kernel<1><<<b, 128, 0, st>>>(x, x_s0, xi, nx, r, pair_ptr, J32, J, pair_query, alpha);
+    else if (dim == 2) cont_weights_kernel<2><<<b, 128, 0, st>>>(x, x_s0, xi, nx, r, pair_ptr, J32, J, pair_query, alpha);
+    else cont_weights_kernel<3><<<b, 128, 0, st>>>(x, x_s0, xi, nx, r, pair_ptr, J32, J, pair_query, alpha);
     return cudaGetLastError();
+}
+
+// *flag := 1 where a[i] != b[i], i < n
+__global__ void ptr_mismatch_kernel(const long long* __restrict__ a, const long long* __restrict__ b, long long n, int* flag) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        if (a[i] != b[i]) *flag = 1;
+}
+
+cudaError_t launch_ptr_mismatch(const long long* a, const long long* b, long long n, int* flag, cudaStream_t st) {
+    ptr_mismatch_kernel<<<grid_for(n, 256), 256, 0, st>>>(a, b, n, flag);
+    return cudaGetLastError();
+}
+
+// Candidate slot (p, k) of pair p (model m = J[p]), k < L = max nk + 1: k < nk_m the neighbour hoods[m][k], k = L - 1
+// the folded known F (column center + m) when centre folding applies to m, else no column.
+__device__ __forceinline__ unsigned cont_slot_column(const ContCsrParams& P, long long p, int k) {
+    const long long m = P.J[p];
+    const CaseMeta cm = P.meta ? P.meta[m] : P.uni;
+    if (k < cm.nk) return (unsigned)P.hoods[m * P.hoods_s0 + k];
+    if (k == P.L - 1 && P.center >= 0 && (cm.knowns & 1LL)) return (unsigned)(P.center + m);
+    return CONT_NO_COLUMN;
+}
+__device__ __forceinline__ double cont_slot_value(const ContCsrParams& P, int o, long long p, int k) {
+    return k < P.maxnk ? P.W[((long long)o * P.npairs + p) * P.maxnk + k] : P.kf[(long long)o * P.npairs + p];
+}
+__device__ __forceinline__ long long cont_row_slots(const ContCsrParams& P, long long q) {
+    return (P.pair_ptr[q + 1] - P.pair_ptr[q]) * P.L;
+}
+
+// Short rows (at most row_cap candidate slots): one warp per query stages the keys (column << 32 | slot) of its slots in
+// shared memory and sorts them (bitonic, padded to a power of two with ~0).  Keys are unique, so equal columns end up
+// adjacent in slot order -- the candidate order.  FILL = false: the number of distinct columns -> cnt[q]; FILL = true:
+// column and per operator the run's values summed from +0 in candidate order at rp[q] + (the run's rank).  Longer rows
+// are left to the sort route below.
+template <bool FILL, typename IDX>
+__global__ void __launch_bounds__(CONT_ROW_WARPS * 32) cont_row_kernel(ContCsrParams P) {
+    extern __shared__ unsigned long long cont_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    unsigned long long* buf = cont_smem + (size_t)warp * P.row_cap;
+    const long long GW = (long long)gridDim.x * nwarps;
+    for (long long q = (long long)blockIdx.x * nwarps + warp; q < P.nx; q += GW) {
+        const long long nl = cont_row_slots(P, q);
+        if (nl > P.row_cap) continue;
+        const long long p0 = P.pair_ptr[q];
+        const int n = (int)nl;
+        int N = 32;
+        while (N < n) N <<= 1;
+        for (int i = lane; i < N; i += 32) {
+            unsigned long long key = ~0ull;
+            if (i < n) {
+                const int pp = i / P.L;
+                const unsigned c = cont_slot_column(P, p0 + pp, i - pp * P.L);
+                if (c != CONT_NO_COLUMN) key = ((unsigned long long)c << 32) | (unsigned)i;
+            }
+            buf[i] = key;
+        }
+        __syncwarp();
+        for (int size = 2; size <= N; size <<= 1)
+            for (int stride = size >> 1; stride > 0; stride >>= 1) {
+                for (int t = lane; t < (N >> 1); t += 32) {
+                    const int a = ((t & ~(stride - 1)) << 1) | (t & (stride - 1)), b = a + stride;
+                    const unsigned long long ka = buf[a], kb = buf[b];
+                    if ((ka > kb) == ((a & size) == 0)) { buf[a] = kb; buf[b] = ka; }
+                }
+                __syncwarp();
+            }
+        long long cnt = 0;
+        const long long base = FILL ? P.rp[q] : 0;
+        for (int i0 = 0; i0 < n; i0 += 32) {
+            const int i = i0 + lane;
+            unsigned long long key = ~0ull;
+            bool head = false;
+            if (i < n) {
+                key = buf[i];
+                head = key != ~0ull && (i == 0 || (key >> 32) != (buf[i - 1] >> 32));
+            }
+            const unsigned bal = __ballot_sync(0xffffffffu, head);
+            if (FILL && head) {
+                const long long pos = base + cnt + __popc(bal & ((1u << lane) - 1u));
+                const unsigned c = (unsigned)(key >> 32);
+                static_cast<IDX*>(P.col)[pos] = (IDX)c;
+                for (int o = 0; o < P.nops; ++o) {
+                    double v = 0.0;
+                    for (int j = i; j < n && (unsigned)(buf[j] >> 32) == c; ++j) {
+                        const int sl = (int)(unsigned)buf[j], pp = sl / P.L;
+                        v = __dadd_rn(v, cont_slot_value(P, o, p0 + pp, sl - pp * P.L));
+                    }
+                    P.values[(long long)o * P.nnz + pos] = v;
+                }
+            }
+            cnt += __popc(bal);
+        }
+        if (!FILL && lane == 0) P.cnt[q] = cnt;
+        __syncwarp();   // buf is rewritten for the next row
+    }
+}
+
+// ---- sort route for rows longer than row_cap: chunk [q0, q1) of the queries, slots [slot0, slot0 + nslots) -------
+// chunk slot i (global slot g = slot0 + i, pair g / L): its column when its row is long, else none (sorted last)
+__global__ void cont_keys_kernel(ContCsrParams P) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < P.nslots; i += (long long)gridDim.x * blockDim.x) {
+        const long long g = P.slot0 + i, p = g / P.L;
+        const bool lng = cont_row_slots(P, P.pair_query[p]) > P.row_cap;
+        P.keys[i] = lng ? cont_slot_column(P, p, (int)(g - p * P.L)) : CONT_NO_COLUMN;
+        P.cand[i] = (int)i;
+    }
+}
+
+// seg[j] = the first chunk slot of query q0 + j, j <= q1 - q0
+__global__ void cont_seg_kernel(ContCsrParams P) {
+    for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j <= P.q1 - P.q0; j += (long long)gridDim.x * blockDim.x)
+        P.seg[j] = (int)(P.pair_ptr[P.q0 + j] * P.L - P.slot0);
+}
+
+// head[i] = 1 where sorted chunk slot i starts a (query, column) run; head[nslots] = 0 (the scan's total)
+__global__ void cont_heads_kernel(ContCsrParams P) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i <= P.nslots; i += (long long)gridDim.x * blockDim.x) {
+        int h = 0;
+        if (i < P.nslots) {
+            const unsigned key = P.keys_sorted[i];
+            const bool first = i == 0 || P.pair_query[(P.slot0 + i) / P.L] != P.pair_query[(P.slot0 + i - 1) / P.L];
+            h = key != CONT_NO_COLUMN && (first || key != P.keys_sorted[i - 1]);
+        }
+        P.head[i] = h;
+    }
+}
+
+// count: cnt[q] of the chunk's long rows
+__global__ void cont_long_count_kernel(ContCsrParams P) {
+    for (long long q = P.q0 + (long long)blockIdx.x * blockDim.x + threadIdx.x; q < P.q1; q += (long long)gridDim.x * blockDim.x)
+        if (cont_row_slots(P, q) > P.row_cap) P.cnt[q] = P.hpos[P.seg[q - P.q0 + 1]] - P.hpos[P.seg[q - P.q0]];
+}
+
+// fill: one thread per run head, the run's values summed in candidate order from +0 (the sort is stable)
+template <typename IDX>
+__global__ void cont_long_fill_kernel(ContCsrParams P) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < P.nslots; i += (long long)gridDim.x * blockDim.x) {
+        if (!P.head[i]) continue;
+        const unsigned key = P.keys_sorted[i];
+        const long long q = P.pair_query[(P.slot0 + i) / P.L];
+        const long long s0 = P.seg[q - P.q0], end = P.seg[q - P.q0 + 1];
+        const long long pos = P.rp[q] + P.hpos[i] - P.hpos[s0];
+        static_cast<IDX*>(P.col)[pos] = (IDX)key;
+        for (int o = 0; o < P.nops; ++o) {
+            double v = 0.0;
+            for (long long j = i; j < end && P.keys_sorted[j] == key; ++j) {
+                const long long g = P.slot0 + P.cand_sorted[j], p = g / P.L;
+                v = __dadd_rn(v, cont_slot_value(P, o, p, (int)(g - p * P.L)));
+            }
+            P.values[(long long)o * P.nnz + pos] = v;
+        }
+    }
+}
+
+// One chunk of the sort route: keys, stable sort per query, heads, scan, then the count or the fill of its long rows.
+// tmp == nullptr: *tmp_bytes := the scratch needed for a chunk of P.nslots slots and P.q1 - P.q0 queries.
+cudaError_t cont_long_rows(const ContCsrParams& P, bool fill, int index_bits, void* tmp, size_t* tmp_bytes, cudaStream_t st) {
+    const int n = (int)P.nslots, nseg = (int)(P.q1 - P.q0);
+    if (!tmp) {
+        size_t a = 0, b = 0;
+        cudaError_t e = cub::DeviceSegmentedSort::StableSortPairs(nullptr, a, P.keys, const_cast<unsigned*>(P.keys_sorted),
+                                                                  P.cand, const_cast<int*>(P.cand_sorted), n, nseg, P.seg,
+                                                                  P.seg + 1, st);
+        if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(nullptr, b, P.head, const_cast<int*>(P.hpos), n + 1, st);
+        *tmp_bytes = std::max(a, b);
+        return e;
+    }
+    cont_seg_kernel<<<grid_for(nseg + 1, 256), 256, 0, st>>>(P);
+    cont_keys_kernel<<<grid_for(n, 256), 256, 0, st>>>(P);
+    cudaError_t e = cudaGetLastError();
+    size_t tb = *tmp_bytes;
+    if (e == cudaSuccess)
+        e = cub::DeviceSegmentedSort::StableSortPairs(tmp, tb, P.keys, const_cast<unsigned*>(P.keys_sorted), P.cand,
+                                                      const_cast<int*>(P.cand_sorted), n, nseg, P.seg, P.seg + 1, st);
+    if (e == cudaSuccess) {
+        cont_heads_kernel<<<grid_for(n + 1, 256), 256, 0, st>>>(P);
+        e = cudaGetLastError();
+    }
+    tb = *tmp_bytes;
+    if (e == cudaSuccess) e = cub::DeviceScan::ExclusiveSum(tmp, tb, P.head, const_cast<int*>(P.hpos), n + 1, st);
+    if (e != cudaSuccess) return e;
+    if (!fill) cont_long_count_kernel<<<grid_for(nseg, 256), 256, 0, st>>>(P);
+    else if (index_bits == 32) cont_long_fill_kernel<int32_t><<<grid_for(n, 256), 256, 0, st>>>(P);
+    else cont_long_fill_kernel<long long><<<grid_for(n, 256), 256, 0, st>>>(P);
+    return cudaGetLastError();
+}
+
+template <bool FILL, typename IDX>
+static cudaError_t launch_cont_row_t(const ContCsrParams& P, cudaStream_t st) {
+    const size_t smem = (size_t)CONT_ROW_WARPS * P.row_cap * 8;
+    const cudaError_t e = cudaFuncSetAttribute(cont_row_kernel<FILL, IDX>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const unsigned blocks = (unsigned)std::max<long long>(1, std::min<long long>((P.nx + CONT_ROW_WARPS - 1) / CONT_ROW_WARPS, 148LL * 64));
+    cont_row_kernel<FILL, IDX><<<blocks, CONT_ROW_WARPS * 32, smem, st>>>(P);
+    return cudaGetLastError();
+}
+
+// rowptr[q] = rp[q], q <= nx
+template <typename IDX>
+__global__ void cont_rowptr_kernel(ContCsrParams P) {
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q <= P.nx; q += (long long)gridDim.x * blockDim.x)
+        static_cast<IDX*>(P.rowptr)[q] = (IDX)P.rp[q];
+}
+
+// the short rows: count (fill = false) or rowptr and fill
+cudaError_t launch_cont_rows(const ContCsrParams& P, bool fill, int index_bits, cudaStream_t st) {
+    if (fill) {
+        if (index_bits == 32) cont_rowptr_kernel<int32_t><<<grid_for(P.nx + 1, 256), 256, 0, st>>>(P);
+        else cont_rowptr_kernel<long long><<<grid_for(P.nx + 1, 256), 256, 0, st>>>(P);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    if (P.row_cap == 0) return cudaSuccess;
+    if (!fill) return launch_cont_row_t<false, int32_t>(P, st);
+    return index_bits == 32 ? launch_cont_row_t<true, int32_t>(P, st) : launch_cont_row_t<true, long long>(P, st);
 }
 
 // keys[q] = I[q] when it is a case index, else nmodels; qidx[q] = q

@@ -73,6 +73,10 @@ SIGNATURES = {
     "wlsqm_solver_interp_stencils": (_int, [_vp, _vp, _i64, _vp, _i64, _int, _vp, _vp, _vp]),
     "wlsqm_solver_interp_operator_nnz": (_int, [_vp, _vp, _i64, _i64, _vp]),
     "wlsqm_solver_interp_operator_csr": (_int, [_vp, _vp, _i64, _vp, _i64, _int, _vp, _i64, _int, _vp, _vp, _vp, _vp]),
+    "wlsqm_solver_interp_continuous_count": (_int, [_vp, _vp, _i64, _i64, C.c_double, _i64, _vp, _i64p, _i64p]),
+    "wlsqm_solver_interp_continuous_stencils": (_int, [_vp, _vp, _i64, _i64, C.c_double, _int, _vp, _vp, _vp, _vp, _vp]),
+    "wlsqm_solver_interp_continuous_operator_csr": (_int, [_vp, _vp, _i64, _i64, C.c_double, _int, _vp, _i64, _int, _vp,
+                                                           _vp, _vp, _vp, _vp, _vp]),
     "wlsqm_solver_index_models": (_int, [_vp]),
     "wlsqm_solver_nearest_models": (_int, [_vp, _vp, _i64, _i64, _vp]),
     "wlsqm_solver_interpolate_continuous": (_int, [_vp, _vp, _i64, _i64, C.c_double, _int, _vp]),

@@ -781,17 +781,18 @@ class ExpertSolver:
         return I_out, I_out
 
     # -- interpolation operators (extension; wlsqm_b200/fitter/opexport.py) -------------------------------------------
-    def interp_stencils(self, x, coeffs=0, I=None):
+    def interp_stencils(self, x, coeffs=0, I=None, mode='nearest', r=None):
         """(W, K, I_out): the map from the data to interpolate(x, mode='nearest') as per-query weights -- W (nops, nx,
         max nk) on fk[I[q]], K (nops, nx, max no) on the known values of model I[q], for the coefficient rows coeffs over
         the derivative slots (an int slot, a (max no,) row or a (nops, max no) array).  I=None: the nearest models, found
-        as interpolate() finds them.  See wlsqm_b200.fitter.opexport.interp_stencils."""
-        return _opexport.interp_stencils(self, x, coeffs, I)
+        as interpolate() finds them.  mode='continuous' (needs r, refuses I): one row per (query, model) pair of the
+        models within r, returned as (W, K, (pair_ptr, J)).  See wlsqm_b200.fitter.opexport.interp_stencils."""
+        return _opexport.interp_stencils(self, x, coeffs, I, mode, r)
 
-    def interp_operator(self, x, coeffs=0, I=None, center=None):
+    def interp_operator(self, x, coeffs=0, I=None, center=None, mode='nearest', r=None):
         """(E, K, I_out): the same map as a sparse matrix (nx, npoints) over the points of prepare_hoods, like operator().
-        See wlsqm_b200.fitter.opexport.interp_operator."""
-        return _opexport.interp_operator(self, x, coeffs, I, center)
+        mode='continuous': (E, K, (pair_ptr, J)) with K per pair.  See wlsqm_b200.fitter.opexport.interp_operator."""
+        return _opexport.interp_operator(self, x, coeffs, I, center, mode, r)
 
     def interpolate(self, x, mode='nearest', r=None, diff=0, I=None):
         """Interpolate the global patched model or one derivative of it (``expert.pyx:687-781``).

@@ -11,6 +11,10 @@ The interpolation operators do the same at arbitrary query points: the map from 
 I[q] contracted with the Taylor terms of the offset x[q] - xi[I[q]] (``wlsqm_solver_interp_stencils`` /
 ``wlsqm_solver_interp_operator_csr``).  For fixed queries one CSR product replaces a solve followed by an interpolate;
 mesh-to-mesh transfer, boundary conditions at points that are not fit origins and observation operators are such maps.
+With ``mode='continuous'`` they export the map to ``interpolate(x, mode='continuous', r, diff)``, the weighted average of
+every model within r: one row per (query, model) pair, each the nearest-mode row of that model scaled by the pair's
+normalised weight, and a CSR row per query that merges its pairs (``wlsqm_solver_interp_continuous_*``).  The transpose
+of either matrix is the adjoint of the fit-and-interpolate map.
 
 Both bindings of ``ExpertSolver`` (the Cython shim and the ctypes twin) call these functions.
 """
@@ -73,6 +77,14 @@ def _ptr(a):
     return a.data_ptr() if _lib._is_torch_tensor(a) else a.ctypes.data
 
 
+def _csr_matrices(rowptr, col, values, shape, cuda):
+    if cuda:
+        import torch
+        return [torch.sparse_csr_tensor(rowptr, col, values[o], size=shape) for o in range(values.shape[0])]
+    import scipy.sparse as sp
+    return [sp.csr_array((values[o], col, rowptr), shape=shape) for o in range(values.shape[0])]
+
+
 def stencils(solver, coeffs):
     """(W, K): W (nops, ncases, max nk) stencil weights on fk, K (nops, ncases, max no) weights on the known values;
     the nops axis is dropped for an int slot or a 1-D coefficient row.  CUDA tensors when the solver was prepared
@@ -118,12 +130,7 @@ def operator(solver, coeffs, center=None):
     K = _empty((nops, n, solver._maxno), np.float64, cuda, solver.device)
     _lib.check(L.wlsqm_solver_operator_csr(solver._handle, nops, c.ctypes.data, center, bits, _ptr(rowptr), _ptr(col),
                                            _ptr(values), _ptr(K)))
-    if cuda:
-        import torch
-        mats = [torch.sparse_csr_tensor(rowptr, col, values[o], size=(n, npoints)) for o in range(nops)]
-    else:
-        import scipy.sparse as sp
-        mats = [sp.csr_array((values[o], col, rowptr), shape=(n, npoints)) for o in range(nops)]
+    mats = _csr_matrices(rowptr, col, values, (n, npoints), cuda)
     return (mats[0], K[0]) if squeeze else (mats, K)
 
 
@@ -169,15 +176,64 @@ def _queries(solver, x, I):
     return x_a, x_s0, nx, I_c, I_out
 
 
-def interp_stencils(solver, x, coeffs=0, I=None):
+def _mode_args(solver, mode, r, I):
+    """-> float r in mode='continuous' (None in nearest mode), after interpolate()'s argument checks"""
+    if mode not in ['nearest', 'continuous']:
+        raise ValueError("mode must be one of 'nearest', 'continuous'; got '%s'" % mode)
+    if mode == 'nearest':
+        return None
+    if r is None:
+        raise ValueError("r must be specified in mode='continuous'")
+    if I is not None:
+        raise ValueError("I cannot be given in mode='continuous': the models of a query are every origin within r")
+    r = float(r)
+    if not r > 0.0:
+        raise ValueError("r must be positive, got %r" % r)
+    if solver.tree is None:
+        raise RuntimeError("Points xi have not been indexed; prep_interpolate() must be called before interpolate()")
+    return r
+
+
+def _pairs(solver, x_a, x_s0, nx, r, cuda, center=None):
+    """-> (pair_ptr (nx + 1,) int64, npairs, nnz): the count call of the continuous-mode operators; nnz of the CSR
+    with that center (-1: no folding) is counted when center is given, else it is None"""
+    pair_ptr = _empty((nx + 1,), np.int64, cuda, solver.device)
+    npairs, nnz = C.c_int64(0), C.c_int64(0)
+    solver._use_stream()
+    _lib.check(_lib.lib().wlsqm_solver_interp_continuous_count(solver._handle, x_a.ptr, x_s0, nx, r,
+                                                               -1 if center is None else center, _ptr(pair_ptr),
+                                                               C.byref(npairs), None if center is None else C.byref(nnz)))
+    return pair_ptr, int(npairs.value), (None if center is None else int(nnz.value))
+
+
+def _center_arg(center):
+    if center is None:
+        return -1
+    center = int(center)
+    if center < 0:
+        raise ValueError("center must be >= 0, got %d" % center)
+    return center
+
+
+def interp_stencils(solver, x, coeffs=0, I=None, mode='nearest', r=None):
     """(W, K, I_out): the interpolation operators at the query points x as per-query weights.
 
     W (nops, nx, max nk) weights on the data of model I[q]'s neighbours, K (nops, nx, max no) on its known values, so
     that for an ALGO_BASIC solve  sum_D coeffs[D] d^D f(x[q]) = W[q] . fk[I[q]] + K[q] . fi[I[q]]  with d^D f the value
     interpolate(x, mode='nearest', diff=D) returns.  The nops axis is dropped for an int slot or a 1-D row.  I=None: the
     nearest models, found as interpolate() finds them (I_out returns them); a query without a model (I outside
-    [0, ncases)) has W row 0 and K row NaN.  CUDA tensors when the solver was prepared from CUDA tensors."""
+    [0, ncases)) has W row 0 and K row NaN.  CUDA tensors when the solver was prepared from CUDA tensors.
+
+    mode='continuous' (r required, I refused): the map to interpolate(x, mode='continuous', r), returned as
+    (W, K, (pair_ptr, J)).  The pairs (q, J[p]) for p in [pair_ptr[q], pair_ptr[q+1]) are the models within r of x[q] in
+    ascending order; W (nops, npairs, max nk) and K (nops, npairs, max no) are their rows, the nearest-mode rows of
+    model J[p] at x[q] scaled by the normalised weight of the pair, so that
+    sum_D coeffs[D] d^D f(x[q]) = sum over the pairs p of q of W[p] . fk[J[p]] + K[p] . fi[J[p]].  A query without a
+    model has an empty pair range."""
+    r = _mode_args(solver, mode, r, I)
     c, squeeze = coefficient_rows(coeffs, solver._maxno)
+    if r is not None:
+        return _continuous_stencils(solver, x, c, squeeze, r)
     x_a, x_s0, nx, I_c, I_out = _queries(solver, x, I)
     root = _root(solver)
     cuda = getattr(root, "_cuda_out", False)
@@ -189,21 +245,37 @@ def interp_stencils(solver, x, coeffs=0, I=None):
     return (W[0], K[0], I_out) if squeeze else (W, K, I_out)
 
 
-def interp_operator(solver, x, coeffs=0, I=None, center=None):
+def _continuous_stencils(solver, x, c, squeeze, r):
+    x_a, x_s0, nx = _points(solver, x)
+    cuda = getattr(_root(solver), "_cuda_out", False)
+    pair_ptr, npairs, _ = _pairs(solver, x_a, x_s0, nx, r, cuda)
+    nops = c.shape[0]
+    J = _empty((npairs,), np.int64, cuda, solver.device)
+    W = _empty((nops, npairs, solver._maxnk), np.float64, cuda, solver.device)
+    K = _empty((nops, npairs, solver._maxno), np.float64, cuda, solver.device)
+    _lib.check(_lib.lib().wlsqm_solver_interp_continuous_stencils(solver._handle, x_a.ptr, x_s0, nx, r, nops, c.ctypes.data,
+                                                                  _ptr(pair_ptr), _ptr(J), _ptr(W), _ptr(K)))
+    return (W[0], K[0], (pair_ptr, J)) if squeeze else (W, K, (pair_ptr, J))
+
+
+def interp_operator(solver, x, coeffs=0, I=None, center=None, mode='nearest', r=None):
     """(E, K, I_out): the interpolation operators as a sparse matrix over the points of ``prepare_hoods``.
 
     E (nx, npoints), rows in the order of x: a ``torch.sparse_csr_tensor`` or a ``scipy.sparse.csr_array`` by the rule
     of ``operator()`` (a list of nops matrices sharing one index pair for 2-D coeffs), so that
     sum_D coeffs[D] d^D f(x[q]) = (E @ f)[q] + K[q] . fi[I[q]].  ``center``: index in x of case 0's own point; the weight
     on a known F of model I[q] then moves into column center + I[q] and is 0 in K.  A query without a model has an
-    empty row and a NaN K row."""
+    empty row and a NaN K row.
+
+    mode='continuous' (r required, I refused): (E, K, (pair_ptr, J)) for interpolate(x, mode='continuous', r), with K per
+    pair as in interp_stencils, so that sum_D coeffs[D] d^D f(x[q]) = (E @ f)[q] + sum over the pairs p of q of
+    K[p] . fi[J[p]]; with ``center`` the known-F weight of each pair moves into column center + J[p].  A query without a
+    model has an empty row."""
+    r = _mode_args(solver, mode, r, I)
     c, squeeze = coefficient_rows(coeffs, solver._maxno)
-    if center is None:
-        center = -1
-    else:
-        center = int(center)
-        if center < 0:
-            raise ValueError("center must be >= 0, got %d" % center)
+    center = _center_arg(center)
+    if r is not None:
+        return _continuous_operator(solver, x, c, squeeze, r, center)
     x_a, x_s0, nx, I_c, I_out = _queries(solver, x, I)
     root = _root(solver)
     L = _lib.lib()
@@ -220,10 +292,25 @@ def interp_operator(solver, x, coeffs=0, I=None, center=None):
     K = _empty((nops, nx, solver._maxno), np.float64, cuda, solver.device)
     _lib.check(L.wlsqm_solver_interp_operator_csr(solver._handle, x_a.ptr, x_s0, _ptr(I_c), nx, nops, c.ctypes.data,
                                                   center, bits, _ptr(rowptr), _ptr(col), _ptr(values), _ptr(K)))
-    if cuda:
-        import torch
-        mats = [torch.sparse_csr_tensor(rowptr, col, values[o], size=(nx, npoints)) for o in range(nops)]
-    else:
-        import scipy.sparse as sp
-        mats = [sp.csr_array((values[o], col, rowptr), shape=(nx, npoints)) for o in range(nops)]
+    mats = _csr_matrices(rowptr, col, values, (nx, npoints), cuda)
     return (mats[0], K[0], I_out) if squeeze else (mats, K, I_out)
+
+
+def _continuous_operator(solver, x, c, squeeze, r, center):
+    x_a, x_s0, nx = _points(solver, x)
+    root = _root(solver)
+    cuda = getattr(root, "_cuda_out", False)
+    pair_ptr, npairs, nnz = _pairs(solver, x_a, x_s0, nx, r, cuda, center=center)
+    nops, npoints = c.shape[0], int(getattr(root, "_hood_points", 0))
+    bits = 32 if nnz < 2 ** 31 else 64
+    it = np.int32 if bits == 32 else np.int64
+    J = _empty((npairs,), np.int64, cuda, solver.device)
+    rowptr = _empty((nx + 1,), it, cuda, solver.device)
+    col = _empty((nnz,), it, cuda, solver.device)
+    values = _empty((nops, nnz), np.float64, cuda, solver.device)
+    K = _empty((nops, npairs, solver._maxno), np.float64, cuda, solver.device)
+    _lib.check(_lib.lib().wlsqm_solver_interp_continuous_operator_csr(
+        solver._handle, x_a.ptr, x_s0, nx, r, nops, c.ctypes.data, center, bits, _ptr(pair_ptr), _ptr(J), _ptr(rowptr),
+        _ptr(col), _ptr(values), _ptr(K)))
+    mats = _csr_matrices(rowptr, col, values, (nx, npoints), cuda)
+    return (mats[0], K[0], (pair_ptr, J)) if squeeze else (mats, K, (pair_ptr, J))
